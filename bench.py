@@ -2,6 +2,7 @@
 """Benchmark of the DPoser hot path: poses/sec for reverse-SDE sampling + SMPL LBS.
 
     python bench.py --gpus N --steps K --warmup W [--workload sample_lbs|lbs|sample|completion] [--impl reference]
+                    [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one batch of synthetic input resident in HBM:
   sample_lbs (default): x_T[B,63] -> 1000-step reverse SDE (EM predictor, subVP, config default) ->
@@ -9,7 +10,9 @@ One "step" = one pass of the hot path over one batch of synthetic input resident
                         (BASELINE.json configs[1] batch; the metric "reverse-SDE sampling + SMPL LBS").
   lbs:     configs[1] alone (SMPL LBS forward, B = 65536).
   sample:  the sampler alone.     completion: configs[2] (imputation sampler, 40960 rows).
-Prints ONE JSON line (rank 0).  Multi-GPU: rows are independent, every rank processes its own B rows
+Prints ONE JSON line (rank 0).  `--dump-outputs DIR` also writes what the last timed step returned (rank 0) as
+float32 DIR/<name>.npy; all inputs are seeded, so two builds run with the same arguments compare output for output.
+Multi-GPU: rows are independent, every rank processes its own B rows
 (weak scaling, no data-path collective in `value`); timing is barrier + CUDA events, max over ranks.  The end-to-end
 leg (`e2e`) at N > 1 also runs the collectives the reference's evaluation uses (run/completion.py:300-305,
 lib/utils/metric.py:8-37): all-gather of the generated poses and the rank-sharded APD with its all-reduce.
@@ -28,6 +31,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -569,6 +573,26 @@ def cpu_task_loops(budget_s=12.0):
     return res
 
 
+DUMP_BYTES = 63 * 10 ** 6             # array data of one --dump-outputs; with the .npy headers under 64 MB
+
+
+def dump_outputs(res, out_dir, budget=DUMP_BYTES):
+    """Write each array of `res` as float32 `out_dir/<name>.npy`, smallest first, each within an even share of what is
+    left of `budget`.  An array larger than its share keeps a fixed sample of rows (first-dimension entries chosen by
+    a seed-0 permutation, in ascending order): the same rows in every run with the same batch size."""
+    os.makedirs(out_dir, exist_ok=True)
+    items = sorted(res.items(), key=lambda kv: kv[1].numel())
+    for i, (name, t) in enumerate(items):
+        t = t.detach().float()
+        share = budget // (len(items) - i)
+        if t.numel() * 4 > share:
+            keep = share // (t[0].numel() * 4)
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows.to(t.device)]
+        budget -= t.numel() * 4
+        np.save(os.path.join(out_dir, f'{name}.npy'), t.cpu().numpy())
+
+
 def run_gpu_arm(args):
     from dposer_b200 import _lib as L
     from dposer_b200 import dist as D
@@ -678,17 +702,19 @@ def run_gpu_arm(args):
         torch.cuda.synchronize()
 
     def timed(e2e, n_steps):
+        """mean step time (ms) and the outputs of the last step"""
         total = 0.0
         for _ in range(n_steps):
+            res = None                  # free the previous step's outputs first: one set alive, as in the warm-up
             flush.fill_(1)
             barrier()
             e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             e0.record()
-            step(e2e)
+            res = step(e2e)
             e1.record()
             torch.cuda.synchronize()
             total += D.max_over_ranks(e0.elapsed_time(e1), dev)
-        return total / n_steps
+        return total / n_steps, res
 
     # the LBS stage is timed ALONE, before the sampler brings the GPU to its power cap (the roofline of a kernel
     # timed alone; inside the pipeline it runs at the capped clock and shows up in `value`)
@@ -702,10 +728,13 @@ def run_gpu_arm(args):
     clocks = ClockSampler(local)
     if rank == 0:
         clocks.start()
-    ms = timed(False, args.steps)
+    ms, last = timed(False, args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(last, args.dump_outputs)
+    del last
     step(True)                      # untimed: allocates the pinned result buffers the end-to-end steps copy into
     torch.cuda.synchronize()
-    ms_e2e = timed(True, max(1, min(args.steps, 3)))
+    ms_e2e = timed(True, max(1, min(args.steps, 3)))[0]
     clk = clocks.stop() if rank == 0 else None
 
     # per-kernel timing of the two stages for the roofline (same stream, CUDA events, inputs resident)
@@ -818,7 +847,13 @@ def main():
     ap.add_argument('--c4-sequences', type=int, default=256, help='sequences per batch of the motion-denoising config')
     ap.add_argument('--c4-batches', type=int, default=0, help='batches to time (0 = the whole config: 8192 sequences)')
     ap.add_argument('--c5-images', type=int, default=131072, help='images on this GPU for the SMPLify config')
+    ap.add_argument('--dump-outputs', metavar='DIR', help='write the outputs of the last timed step (rank 0) as '
+                    'float32 DIR/<name>.npy, under 64 MB in all (a fixed sample of rows where an output is larger)')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs needs --impl ours (the reference arm returns no arrays)')
     if args.impl == 'reference':
         run_reference_arm(args)
     else:

@@ -8,6 +8,7 @@ dposer_b200/data/.  While generating, it also asserts that oracle/ reproduces th
 reference (so a fixture is only ever written from a state where oracle == reference).
 Import shims follow SURVEY.md Appendix C (test-only scaffolding around the untouched reference).
 """
+import math
 import os
 import sys
 import types
@@ -94,7 +95,9 @@ def main():
         if k.startswith('pre_dense_cond'):
             continue
         assert torch.equal(v, sd[k]), f'weight recipe mismatch at {k}'
-        fingerprint[k] = np.float64(v.double().abs().sum().item())
+        # exactly rounded sum: torch's CPU sum() splits the reduction by thread count, so it can differ in the last
+        # bit from one host to another
+        fingerprint[k] = np.float64(math.fsum(v.double().abs().flatten().tolist()))
     print('weights: oracle recipe == reference recipe (bit-exact), params',
           sum(v.numel() for k, v in ref_sd.items() if k != 'sigmas'))
     np.savez(os.path.join(HERE, 'weights_fingerprint.npz'), **fingerprint)

@@ -1,5 +1,6 @@
 """CPU: the oracle must reproduce every golden vector produced by the REAL reference
 (tests/golden/make_golden.py).  This is what pins the oracle (prompt section 3)."""
+import math
 import os
 
 import numpy as np
@@ -32,7 +33,7 @@ def test_known_answers_appendix_d():
 def test_weight_recipe_fingerprint(oracle_sd):
     fp = golden('weights_fingerprint.npz')
     for k in fp.files:
-        assert oracle_sd[k].double().abs().sum().item() == float(fp[k]), k
+        assert math.fsum(oracle_sd[k].double().abs().flatten().tolist()) == float(fp[k]), k
 
 
 def test_score_net_matches_reference(oracle_sd):
