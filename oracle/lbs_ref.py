@@ -15,6 +15,8 @@ from the reference: 22-joint parents (lib/body_model/utils.py:180-205), 49-entry
 Second opinion: oracle/lbs_np64.py is an independent float64 formulation (no homogeneous matrices); the CPU suite
 checks that the two agree to fp32 round-off and that both satisfy the zero-pose / rigid-root / translation /
 single-joint invariants (tests/test_oracle_golden.py).
+Device-generic: every constant is created on its input's device, so a float64 model dict on CUDA runs there (the
+GPU suite's full-batch float64 reference, tests/test_gpu_lbs_scale.py).
 """
 import torch
 
@@ -37,9 +39,9 @@ def batch_rodrigues(rot_vecs):
     cos = torch.cos(angle)[:, None]
     sin = torch.sin(angle)[:, None]
     rx, ry, rz = torch.split(rot_dir, 1, dim=1)
-    zeros = torch.zeros((n, 1), dtype=rot_vecs.dtype)
+    zeros = torch.zeros((n, 1), dtype=rot_vecs.dtype, device=rot_vecs.device)
     K = torch.cat([zeros, -rz, ry, rz, zeros, -rx, -ry, rx, zeros], dim=1).view(n, 3, 3)
-    ident = torch.eye(3, dtype=rot_vecs.dtype)[None]
+    ident = torch.eye(3, dtype=rot_vecs.dtype, device=rot_vecs.device)[None]
     return ident + sin * K + (1 - cos) * torch.bmm(K, K)
 
 
@@ -48,17 +50,17 @@ def batch_rigid_transform(rot_mats, joints, parents):
     B, J = joints.shape[:2]
     joints = joints.unsqueeze(-1)
     rel = joints.clone()
-    par = torch.as_tensor(parents[1:], dtype=torch.long)
+    par = torch.as_tensor(parents[1:], dtype=torch.long, device=joints.device)
     rel[:, 1:] = rel[:, 1:] - joints[:, par]
     top = torch.cat([rot_mats, rel], dim=-1)                              # [B,J,3,4]
-    bottom = torch.tensor([0, 0, 0, 1], dtype=joints.dtype).view(1, 1, 1, 4).expand(B, J, 1, 4)
+    bottom = torch.tensor([0, 0, 0, 1], dtype=joints.dtype, device=joints.device).view(1, 1, 1, 4).expand(B, J, 1, 4)
     M = torch.cat([top, bottom], dim=-2)                                  # [B,J,4,4]
     chain = [M[:, 0]]
     for i in range(1, J):
         chain.append(torch.matmul(chain[parents[i]], M[:, i]))
     G = torch.stack(chain, dim=1)
     posed = G[:, :, :3, 3]
-    jh = torch.cat([joints, torch.zeros(B, J, 1, 1, dtype=joints.dtype)], dim=2)   # [B,J,4,1]
+    jh = torch.cat([joints, torch.zeros(B, J, 1, 1, dtype=joints.dtype, device=joints.device)], dim=2)   # [B,J,4,1]
     corr = torch.matmul(G, jh)                                            # [B,J,4,1]
     A = G - torch.nn.functional.pad(corr, [3, 0])
     return posed, A
@@ -71,12 +73,12 @@ def lbs(betas, pose, v_template, shapedirs, posedirs, J_regressor, parents, lbs_
     v_shaped = v_template[None] + torch.einsum('bl,mkl->bmk', betas, shapedirs)
     Jrest = torch.einsum('bik,ji->bjk', v_shaped, J_regressor)
     R = batch_rodrigues(pose.reshape(-1, 3)).view(B, J, 3, 3)
-    feat = (R[:, 1:] - torch.eye(3, dtype=betas.dtype)).reshape(B, -1)
+    feat = (R[:, 1:] - torch.eye(3, dtype=betas.dtype, device=betas.device)).reshape(B, -1)
     v_posed = v_shaped + torch.matmul(feat, posedirs).view(B, -1, 3)
     Jposed, A = batch_rigid_transform(R, Jrest, parents)
     W = lbs_weights[None].expand(B, -1, -1)
     T = torch.matmul(W, A.view(B, J, 16)).view(B, -1, 4, 4)
-    vh = torch.cat([v_posed, torch.ones(B, v_posed.shape[1], 1, dtype=betas.dtype)], dim=2)
+    vh = torch.cat([v_posed, torch.ones(B, v_posed.shape[1], 1, dtype=betas.dtype, device=betas.device)], dim=2)
     verts = torch.matmul(T, vh.unsqueeze(-1))[:, :, :3, 0]
     return verts, Jposed
 
@@ -96,7 +98,7 @@ def body_forward(model, betas, full_pose, transl=None, chunk=1024):
         e = s + chunk
         v, j = lbs(betas[s:e], full_pose[s:e], model['v_template'], model['shapedirs'], model['posedirs'],
                    model['J_regressor'], model['parents'], model['lbs_weights'])
-        extra = v[:, torch.as_tensor(model['extra_vids'], dtype=torch.long)]
+        extra = v[:, torch.as_tensor(model['extra_vids'], dtype=torch.long, device=v.device)]
         parts = [j, extra]
         if model.get('lmk_faces') is not None:
             tri = v[:, model['lmk_faces'].reshape(-1)].view(v.shape[0], -1, 3, 3)
