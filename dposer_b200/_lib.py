@@ -15,6 +15,8 @@ SAMPLER_IMPUTE, SAMPLER_NOISE_GIVEN = 1 << 4, 1 << 5
 LBS_CONST_TAIL, LBS_NO_SAVE = 1 << 4, 1 << 5
 COEF_STRIDE = 8
 POSE_DIM, HIDDEN, EMBED, NUM_DENSE = 63, 1024, 512, 5
+POSE_DIM_ROT6D = 126
+POSE_DIMS = (POSE_DIM, POSE_DIM_ROT6D)      # pose widths a score handle can be built for (axis-angle, rot6d)
 
 _f32p = C.POINTER(C.c_float)
 _i32p = C.POINTER(C.c_int32)
@@ -39,7 +41,8 @@ class BodyTensors(C.Structure):
                 ('n_lmk', C.c_int), ('lmk_faces', _i32p), ('lmk_bary', _f32p)]
 
 
-EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create', 'dpb_score_destroy',
+EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create', 'dpb_score_create_dim',
+           'dpb_score_pose_dim', 'dpb_normal_fill_dim', 'dpb_langevin_norms_dim', 'dpb_langevin_update_dim', 'dpb_score_destroy',
            'dpb_score_time_table', 'dpb_score_workspace_bytes', 'dpb_score_forward', 'dpb_score_jvp',
            'dpb_score_jvp_workspace_bytes', 'dpb_sampler_run_pc', 'dpb_sampler_pc_workspace_bytes', 'dpb_sampler_run',
            'dpb_langevin_norms', 'dpb_langevin_update', 'dpb_normal_fill', 'dpb_prior_loss', 'dpb_lbs_create',
@@ -73,6 +76,8 @@ def load():
     lib.dpb_last_error.restype = C.c_char_p
     lib.dpb_device_info.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
     lib.dpb_score_create.argtypes = [C.POINTER(vp), C.POINTER(ScoreWeights), C.c_int]
+    lib.dpb_score_create_dim.argtypes = [C.POINTER(vp), C.POINTER(ScoreWeights), C.c_int, C.c_int]
+    lib.dpb_score_pose_dim.argtypes = [vp]
     lib.dpb_score_destroy.argtypes = [vp]
     lib.dpb_score_time_table.argtypes = [vp, vp, C.c_int, vp, vp]
     lib.dpb_score_workspace_bytes.argtypes = [vp, i64, C.c_int]
@@ -83,6 +88,9 @@ def load():
     lib.dpb_langevin_norms.argtypes = [vp, vp, vp, i64, vp]
     lib.dpb_langevin_update.argtypes = [vp, vp, vp, vp, vp, f32, f32, i64, vp]
     lib.dpb_normal_fill.argtypes = [vp, i64, u64, u64, C.c_int, vp]
+    lib.dpb_langevin_norms_dim.argtypes = [vp, vp, vp, i64, C.c_int, vp]
+    lib.dpb_langevin_update_dim.argtypes = [vp, vp, vp, vp, vp, f32, f32, i64, C.c_int, vp]
+    lib.dpb_normal_fill_dim.argtypes = [vp, i64, u64, u64, C.c_int, C.c_int, vp]
     lib.dpb_prior_loss.argtypes = [vp, vp, vp, f32, f32, f32, C.c_int, f32, vp, u64, u64, vp, vp, vp, i64, C.c_int,
                                    vp, sz, vp]
     lib.dpb_sampler_pc_workspace_bytes.argtypes = [vp, i64]

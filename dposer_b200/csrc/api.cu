@@ -17,14 +17,15 @@ int fail(int code, const std::string& msg) {
 }
 
 // sampler.cu launchers
+// sampler.cu launchers; `dp` = the handle's padded pose width (64 or 128)
 int launch_em_update(float*, const float*, const float*, const float*, const float*, const float*, int, uint64_t,
-                     uint32_t, float*, float*, int64_t, int, cudaStream_t);
-int launch_impute(float*, const float*, const float*, const float*, const float*, uint64_t, uint32_t, int64_t,
+                     uint32_t, float*, float*, int64_t, int, int dp, cudaStream_t);
+int launch_impute(float*, const float*, const float*, const float*, const float*, uint64_t, uint32_t, int64_t, int dp,
                   cudaStream_t);
-int launch_scale_out(const float*, const float*, float, float*, int64_t, cudaStream_t);
-int launch_perturb(const float*, const float*, uint64_t, uint32_t, float, float, float*, int64_t, cudaStream_t);
+int launch_scale_out(const float*, const float*, float, float*, int64_t, int dp, cudaStream_t);
+int launch_perturb(const float*, const float*, uint64_t, uint32_t, float, float, float*, int64_t, int dp, cudaStream_t);
 int launch_prior_loss(const float*, const float*, const float*, float, float, float, float, float, float*, float*,
-                      float*, int64_t, cudaStream_t);
+                      float*, int64_t, int dp, cudaStream_t);
 
 static int pick_engine(const dpb_score* h, int flags, int64_t B, bool uniform_t) {
   int e = flags & DPB_ENGINE_MASK;
@@ -59,7 +60,9 @@ static int up_f32(float** dst, const float* src, size_t n) {
   return DPB_OK;
 }
 
-extern "C" int dpb_score_create(dpb_score_t** out, const dpb_score_weights* w, int device) {
+extern "C" int dpb_score_create_dim(dpb_score_t** out, const dpb_score_weights* w, int pose_dim, int device) {
+  if (pose_dim != DPB_POSE_DIM && pose_dim != DPB_POSE_DIM_ROT6D)
+    return fail(DPB_EUNSUPPORTED, "dpb_score_create_dim: pose_dim must be 63 (axis-angle) or 126 (rot6d)");
   if (!out || !w) return fail(DPB_EINVAL, "dpb_score_create: null argument");
   const void* req[] = {w->pre_w, w->pre_b, w->pre_t_w, w->pre_t_b, w->pre_gn_w, w->pre_gn_b, w->temb_w, w->temb_b,
                        w->post_w, w->post_b, w->emb_freqs};
@@ -75,11 +78,14 @@ extern "C" int dpb_score_create(dpb_score_t** out, const dpb_score_weights* w, i
   dpb_score* h = new dpb_score();
   h->device = device;
   h->sm_count = sm;
+  h->pose_dim = pose_dim;
+  h->pose_dp = pose_dim == D126 ? DP128 : DP;
+  const int hd = h->pose_dim, hdp = h->pose_dp;
   // padded fp32 copies
-  std::vector<float> prew((size_t)H * DP, 0.f), postw((size_t)DP * H, 0.f), postb(DP, 0.f);
-  for (int o = 0; o < H; ++o) std::memcpy(&prew[(size_t)o * DP], w->pre_w + (size_t)o * D, D * sizeof(float));
-  std::memcpy(postw.data(), w->post_w, (size_t)D * H * sizeof(float));
-  std::memcpy(postb.data(), w->post_b, D * sizeof(float));
+  std::vector<float> prew((size_t)H * hdp, 0.f), postw((size_t)hdp * H, 0.f), postb(hdp, 0.f);
+  for (int o = 0; o < H; ++o) std::memcpy(&prew[(size_t)o * hdp], w->pre_w + (size_t)o * hd, hd * sizeof(float));
+  std::memcpy(postw.data(), w->post_w, (size_t)hd * H * sizeof(float));
+  std::memcpy(postb.data(), w->post_b, hd * sizeof(float));
   const float* lin_b[5] = {w->pre_b, w->blk_b[0], w->blk_b[1], w->blk_b[2], w->blk_b[3]};
   const float* t_w[5] = {w->pre_t_w, w->blk_t_w[0], w->blk_t_w[1], w->blk_t_w[2], w->blk_t_w[3]};
   const float* t_b[5] = {w->pre_t_b, w->blk_t_b[0], w->blk_t_b[1], w->blk_t_b[2], w->blk_t_b[3]};
@@ -112,6 +118,15 @@ extern "C" int dpb_score_create(dpb_score_t** out, const dpb_score_weights* w, i
   return DPB_OK;
 }
 
+extern "C" int dpb_score_create(dpb_score_t** out, const dpb_score_weights* w, int device) {
+  return dpb_score_create_dim(out, w, DPB_POSE_DIM, device);
+}
+
+extern "C" int dpb_score_pose_dim(dpb_score_t* h) {
+  if (!h) return fail(DPB_EINVAL, "dpb_score_pose_dim: null handle");
+  return h->pose_dim;
+}
+
 extern "C" int dpb_score_destroy(dpb_score_t* h) {
   if (!h) return DPB_OK;
   DeviceGuard guard(h->device);
@@ -137,8 +152,9 @@ extern "C" int dpb_score_time_table(dpb_score_t* h, const float* labels, int n, 
 extern "C" size_t dpb_score_workspace_bytes(dpb_score_t* h, int64_t B, int flags) {
   (void)flags;
   if (!h || B <= 0) return 0;
-  // fp32 engine buffers + raw [B,64] + perturbed x [B,63]; the tcgen05 engine owns its scratch
-  return simt_forward_ws_bytes(B) + align_up((size_t)B * DP * 4, 256) + align_up((size_t)B * D * 4, 256) + 1024;
+  // fp32 engine buffers + raw [B,DP] + perturbed x [B,D]; the tcgen05 engine owns its scratch
+  return simt_forward_ws_bytes(B, h->pose_dp) + align_up((size_t)B * h->pose_dp * 4, 256) + align_up((size_t)B * h->pose_dim * 4, 256) +
+         1024;
 }
 
 namespace {
@@ -148,16 +164,16 @@ struct ScoreWs {
   void* rest;
   size_t rest_bytes;
 };
-bool carve_score_ws(int64_t B, void* ws, size_t ws_bytes, ScoreWs* o) {
+bool carve_score_ws(const dpb_score* h, int64_t B, void* ws, size_t ws_bytes, ScoreWs* o) {
   if (!ws) return false;
   WsCarver c(ws, ws_bytes);
-  o->raw = c.take<float>((size_t)B * DP);
-  o->xt = c.take<float>((size_t)B * D);
+  o->raw = c.take<float>((size_t)B * h->pose_dp);
+  o->xt = c.take<float>((size_t)B * h->pose_dim);
   c.off = align_up(c.off, 256);
   if (!c.ok()) return false;
   o->rest = c.base + c.off;
   o->rest_bytes = ws_bytes - c.off;
-  return o->rest_bytes >= simt_forward_ws_bytes(B);
+  return o->rest_bytes >= simt_forward_ws_bytes(B, h->pose_dp);
 }
 }  // namespace
 
@@ -179,10 +195,10 @@ extern "C" int dpb_score_forward(dpb_score_t* h, const float* x, const float* ta
     return tc_launch(h, j, st);
   }
   ScoreWs w;
-  if (!carve_score_ws(B, ws, ws_bytes, &w)) return fail(DPB_ENOMEM, "dpb_score_forward: workspace too small");
+  if (!carve_score_ws(h, B, ws, ws_bytes, &w)) return fail(DPB_ENOMEM, "dpb_score_forward: workspace too small");
   int rc = simt_forward_raw(h, x, table, t_index, w.raw, B, w.rest, w.rest_bytes, st);
   if (rc != DPB_OK) return rc;
-  return launch_scale_out(w.raw, row_scale, scale, out, B, st);
+  return launch_scale_out(w.raw, row_scale, scale, out, B, h->pose_dp, st);
 }
 
 // Predictor-corrector sampling with the Langevin corrector (sampling.py:456-461 with :282-302), all steps from one host
@@ -191,7 +207,7 @@ extern "C" int dpb_score_forward(dpb_score_t* h, const float* x, const float* ta
 // returning to the caller (the Python loop of round 1 was bound by its per-step host work at small batches).
 extern "C" size_t dpb_sampler_pc_workspace_bytes(dpb_score_t* h, int64_t B) {
   if (!h || B <= 0) return 0;
-  return dpb_score_workspace_bytes(h, B, 0) + 2 * align_up((size_t)B * D * 4, 256) + 256 + 1024;
+  return dpb_score_workspace_bytes(h, B, 0) + 2 * align_up((size_t)B * h->pose_dim * 4, 256) + 256 + 1024;
 }
 
 extern "C" int dpb_sampler_run_pc(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, const float* score_scale,
@@ -225,14 +241,14 @@ extern "C" int dpb_sampler_run_pc(dpb_score_t* h, float* x_io, const dpb_step_ta
     return tc_launch(h, j, st);
   }
   WsCarver c(ws, ws_bytes);
-  float* grad = c.take<float>((size_t)B * D);
-  float* z = c.take<float>((size_t)B * D);
+  float* grad = c.take<float>((size_t)B * h->pose_dim);
+  float* z = c.take<float>((size_t)B * h->pose_dim);
   float* sums = c.take<float>(2);
   c.off = align_up(c.off, 256);
   void* rest = static_cast<uint8_t*>(ws) + c.off;
   const size_t rest_bytes = ws_bytes - c.off;
   const int kp = noise_k;                              // predictor planes per step; the Langevin draw comes first
-  const size_t plane = (size_t)B * D;
+  const size_t plane = (size_t)B * h->pose_dim;
   for (int i = 0; i < tbl->n_steps; ++i) {
     const float* table_i = tbl->time_table + (size_t)i * NL * H;
     int rc = dpb_score_forward(h, x_io, table_i, nullptr, nullptr, score_scale[i], grad, B, flags & DPB_ENGINE_MASK, rest,
@@ -240,10 +256,11 @@ extern "C" int dpb_sampler_run_pc(dpb_score_t* h, float* x_io, const dpb_step_ta
     if (rc != DPB_OK) return rc;
     const float* zi = z;
     if (given) zi = noise + (size_t)i * (kp + 1) * plane;
-    else if ((rc = dpb_normal_fill(z, B, seed, step_offset + (uint64_t)i, 4, stream)) != DPB_OK) return rc;
+    else if ((rc = dpb_normal_fill_dim(z, B, seed, step_offset + (uint64_t)i, 4, h->pose_dim, stream)) != DPB_OK) return rc;
     DPB_CUDA_CHECK(cudaMemsetAsync(sums, 0, 2 * sizeof(float), st));
-    if ((rc = dpb_langevin_norms(grad, zi, sums, B, stream)) != DPB_OK) return rc;
-    if ((rc = dpb_langevin_update(x_io, nullptr, grad, zi, sums, snr, lang_alpha[i], B, stream)) != DPB_OK) return rc;
+    if ((rc = dpb_langevin_norms_dim(grad, zi, sums, B, h->pose_dim, stream)) != DPB_OK) return rc;
+    if ((rc = dpb_langevin_update_dim(x_io, nullptr, grad, zi, sums, snr, lang_alpha[i], B, h->pose_dim, stream)) != DPB_OK)
+      return rc;
     dpb_step_tables one{};
     one.n_steps = 1;
     one.coef = tbl->coef + (size_t)i * DPB_COEF_STRIDE;
@@ -257,7 +274,7 @@ extern "C" int dpb_sampler_run_pc(dpb_score_t* h, float* x_io, const dpb_step_ta
 }
 
 extern "C" size_t dpb_score_jvp_workspace_bytes(dpb_score_t* h, int64_t B) {
-  if (!h || B <= 0) return 0;
+  if (!h || B <= 0 || h->pose_dim != DPB_POSE_DIM) return 0;
   const size_t simt = simt_forward_ws_bytes(2 * B), tc = score_jvp_tc_ws_bytes(B);
   return (simt > tc ? simt : tc) + align_up((size_t)2 * B * DP * 4, 256) + 1024;
 }
@@ -266,6 +283,8 @@ extern "C" int dpb_score_jvp(dpb_score_t* h, const float* x, const float* v, con
                              const float* row_scale, float scale, float* out, float* jv, int64_t B, void* ws,
                              size_t ws_bytes, void* stream) {
   if (!h) return fail(DPB_EINVAL, "dpb_score_jvp: null handle");
+  if (h->pose_dim != DPB_POSE_DIM) return fail(DPB_EUNSUPPORTED, "dpb_score_jvp: the forward-mode derivative is built for 63-D (axis) "
+                                              "networks only, not for rot6d (126-D)");
   DeviceGuard guard(h->device);
   DPB_REQUIRE(x && v && table && out && jv, "dpb_score_jvp: x, v, table, out and jv are required");
   if (B <= 0) return DPB_OK;
@@ -280,9 +299,9 @@ extern "C" int dpb_score_jvp(dpb_score_t* h, const float* x, const float* v, con
   int rc = (!t_index && !force_fp32) ? score_jvp_tc_raw(h, x, v, table, raw, B, rest, ws_bytes - c.off, st)
                                      : simt_forward_jvp_raw(h, x, v, table, t_index, raw, B, rest, ws_bytes - c.off, st);
   if (rc != DPB_OK) return rc;
-  rc = launch_scale_out(raw, row_scale, scale, out, B, st);
+  rc = launch_scale_out(raw, row_scale, scale, out, B, DP, st);
   if (rc != DPB_OK) return rc;
-  return launch_scale_out(raw + (size_t)B * DP, row_scale, scale, jv, B, st);   // the scaling is linear: same factor
+  return launch_scale_out(raw + (size_t)B * DP, row_scale, scale, jv, B, DP, st);   // the scaling is linear: same factor
 }
 
 extern "C" int dpb_sampler_run(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, const float* obs,
@@ -309,19 +328,19 @@ extern "C" int dpb_sampler_run(dpb_score_t* h, float* x_io, const dpb_step_table
     return tc_launch(h, j, st);
   }
   ScoreWs w;
-  if (!carve_score_ws(B, ws, ws_bytes, &w)) return fail(DPB_ENOMEM, "dpb_sampler_run: workspace too small");
-  const size_t plane = (size_t)B * D;
+  if (!carve_score_ws(h, B, ws, ws_bytes, &w)) return fail(DPB_ENOMEM, "dpb_sampler_run: workspace too small");
+  const size_t plane = (size_t)B * h->pose_dim;
   for (int i = 0; i < tbl->n_steps; ++i) {
     const float* coef = tbl->coef + (size_t)i * DPB_COEF_STRIDE;
     const float* nz = given ? noise + (size_t)i * noise_k * plane : nullptr;
     const uint32_t step = (uint32_t)(step_offset + (uint64_t)i);
     int rc = DPB_OK;
-    if (impute) rc = launch_impute(x_io, coef, obs, mask, nz, seed, step, B, st);
+    if (impute) rc = launch_impute(x_io, coef, obs, mask, nz, seed, step, B, h->pose_dp, st);
     if (rc == DPB_OK)
       rc = simt_forward_raw(h, x_io, tbl->time_table + (size_t)i * NL * H, nullptr, w.raw, B, w.rest, w.rest_bytes, st);
     if (rc == DPB_OK)
       rc = launch_em_update(x_io, w.raw, coef, obs, mask, nz, noise_k, seed, step,
-                            traj ? traj + (size_t)i * plane : nullptr, x_mean, B, impute, st);
+                            traj ? traj + (size_t)i * plane : nullptr, x_mean, B, impute, h->pose_dp, st);
     if (rc != DPB_OK) return rc;
   }
   return DPB_OK;
@@ -351,11 +370,11 @@ extern "C" int dpb_prior_loss(dpb_score_t* h, const float* x0, const float* tabl
     return tc_launch(h, j, st);
   }
   ScoreWs w;
-  if (!carve_score_ws(B, ws, ws_bytes, &w)) return fail(DPB_ENOMEM, "dpb_prior_loss: workspace too small");
-  int rc = launch_perturb(x0, z, seed, (uint32_t)step, alpha, sd, w.xt, B, st);
+  if (!carve_score_ws(h, B, ws, ws_bytes, &w)) return fail(DPB_ENOMEM, "dpb_prior_loss: workspace too small");
+  int rc = launch_perturb(x0, z, seed, (uint32_t)step, alpha, sd, w.xt, B, h->pose_dp, st);
   if (rc == DPB_OK) rc = simt_forward_raw(h, w.xt, table, nullptr, w.raw, B, w.rest, w.rest_bytes, st);
   if (rc == DPB_OK)
     rc = launch_prior_loss(x0, w.xt, w.raw, alpha, sd, inv_sigma_std, wgt, 1.0f / divisor, loss_out, grad_out,
-                           row_loss, B, st);
+                           row_loss, B, h->pose_dp, st);
   return rc;
 }

@@ -76,6 +76,11 @@ struct WsCarver {
 // ---------------------------------------------------------------- geometry
 constexpr int D = DPB_POSE_DIM;     // 63
 constexpr int DP = 64;              // padded pose dim
+// The pose width is a property of the score handle: 63 (axis-angle) or 126 (rot6d), padded to DP = 64 or 128.
+// Kernels that depend on it are templated on the padded width; D and DP above are the 63-D instantiation.
+constexpr int D126 = DPB_POSE_DIM_ROT6D;
+constexpr int DP128 = 128;
+__host__ __device__ constexpr int pose_dim_of(int dp) { return dp == DP128 ? D126 : D; }
 constexpr int H = DPB_HIDDEN;       // 1024
 constexpr int E = DPB_EMBED;        // 512
 constexpr int NL = DPB_NUM_DENSE;   // 5 hidden-producing dense layers
@@ -83,9 +88,11 @@ constexpr int GROUP = 32;           // channels per GroupNorm group (1024/32)
 constexpr float GN_EPS = 1e-5f;
 
 // ---------------------------------------------------------------- Philox4x32-10 + Box-Muller
-// One counter = (row, step, slot*16 + quad) -> 4 normals for columns 4*quad..4*quad+3 of `row`.
-// Both engines (fp32 and tcgen05) call this with the same arguments, so the same seed gives the
-// same noise on either path.
+// One counter = (row, step, slot*quads + quad) -> 4 normals for columns 4*quad..4*quad+3 of `row`, where
+// quads = DP/4 is the number of column quads of the padded row: 16 for the 63-D layout, 32 for the 126-D one.
+// Every (slot, column) of a row therefore has its own counter word (slots 0..4 are in use); the 126-D layout
+// is a different stream from the 63-D one, not an extension of it.  Both engines (fp32 and tcgen05) call this
+// with the same arguments, so the same seed gives the same noise on either path.
 __host__ __device__ __forceinline__ uint32_t mulhilo32(uint32_t a, uint32_t b, uint32_t* hi) {
 #ifdef __CUDA_ARCH__
   *hi = __umulhi(a, b);
@@ -112,9 +119,9 @@ __host__ __device__ __forceinline__ void philox4x32_10(uint32_t c0, uint32_t c1,
 }
 
 __device__ __forceinline__ void normal4(uint64_t seed, uint64_t row, uint32_t step, uint32_t slot, uint32_t quad,
-                                        float z[4]) {
+                                        float z[4], uint32_t quads = 16) {
   uint32_t r[4];
-  philox4x32_10((uint32_t)row, (uint32_t)(row >> 32), step, slot * 16u + quad, (uint32_t)seed,
+  philox4x32_10((uint32_t)row, (uint32_t)(row >> 32), step, slot * quads + quad, (uint32_t)seed,
                 (uint32_t)(seed >> 32), r);
   // uniforms in (0,1]
   const float s = 2.3283064365386963e-10f;  // 2^-32

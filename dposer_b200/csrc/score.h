@@ -7,11 +7,12 @@
 struct dpb_score {
   int device = 0;
   int sm_count = 0;
+  int pose_dim = 63, pose_dp = 64;   // pose width D of this network (63 or 126) and its padded width DP (64 or 128)
   // ---- fp32 parameters on the device (exact engine + time path)
-  float* pre_w = nullptr;       // [1024, 64]  (K padded 63 -> 64 with zeros)
+  float* pre_w = nullptr;       // [1024, DP]  (K padded D -> DP with zeros)
   float* blk_w[4] = {};         // [1024, 1024]
-  float* post_w = nullptr;      // [64, 1024]  (N padded 63 -> 64 with zero rows)
-  float* post_b = nullptr;      // [64]
+  float* post_w = nullptr;      // [DP, 1024]  (N padded D -> DP with zero rows)
+  float* post_b = nullptr;      // [DP]
   float* lin_b[5] = {};         // pre_b, blk_b[0..3]            [1024]
   float* t_w[5] = {};           // pre_t_w, blk_t_w[0..3]        [1024, 512]
   float* t_b[5] = {};           // pre_t_b, blk_t_b[0..3]        [1024]
@@ -23,10 +24,10 @@ struct dpb_score {
   float* gn_packed = nullptr;   // [5][2][1024] gamma|beta, contiguous (tcgen05 epilogue staging)
   // ---- tensor-core operands
   __half* w16[4] = {};          // fp16 copies of blk_w          [1024, 1024]
-  __half* post16 = nullptr;     // fp16 copy of post_w           [64, 1024]
-  __nv_bfloat16* pre_split = nullptr;  // [1024, 192] = [hi | hi | lo] bf16 split of pre_w (K-extension)
+  __half* post16 = nullptr;     // fp16 copy of post_w           [DP, 1024]
+  __nv_bfloat16* pre_split = nullptr;  // [1024, 3 DP] = [hi | hi | lo] bf16 split of pre_w (K-extension)
   CUtensorMap tm_w[4];          // box {64 (K), 256 (N)} over w16[l]
-  CUtensorMap tm_post;          // box {64, 64}
+  CUtensorMap tm_post;          // box {64, DP / 2}
   CUtensorMap tm_pre;           // box {64, 256} over pre_split
   bool tc_ready = false;
   // TC scratch owned by the handle (sized by the grid, not by B): activations + x operand per CTA slot
@@ -49,8 +50,8 @@ namespace dpb {
 
 // ---- fp32 engine (score_simt.cu)
 int simt_time_table(dpb_score* h, const float* labels, int n, float* table, cudaStream_t st);
-size_t simt_forward_ws_bytes(int64_t B);
-// raw[B,64] = post_dense output (column 63 is padding); buffers carved from ws
+size_t simt_forward_ws_bytes(int64_t B, int dp = DP);
+// raw[B,DP] = post_dense output (columns D.. are padding); buffers carved from ws
 int simt_forward_jvp_raw(dpb_score* h, const float* x, const float* v, const float* table, const int32_t* t_index,
                          float* raw, int64_t B, void* ws, size_t ws_bytes, cudaStream_t st);
 int simt_forward_raw(dpb_score* h, const float* x, const float* table, const int32_t* t_index, float* raw,
@@ -64,7 +65,7 @@ struct TcJob {
   // mode 0: forward  out = raw*scale (row_scale optional)      mode 1: sampler      mode 2: prior loss
   int mode;
   int64_t B;
-  const float* x_in;        // forward / prior: x [B,63]
+  const float* x_in;        // forward / prior: x [B,D]
   float* x_io;              // sampler state
   const float* table;       // [n_steps,5,1024]
   const float* coef;        // [n_steps,8] (sampler)

@@ -232,13 +232,21 @@ __global__ void __launch_bounds__(256) gn_silu_jvp_kernel(const float* __restric
   *reinterpret_cast<float4*>(out + (M + m) * H + c) = od;
 }
 
-// x [B,63] -> xpad [B,64]
+// x [B,D] -> xpad [B,PDP]  (D = 63 / 126, PDP = 64 / 128)
+template <int PDP>
 __global__ void pad_x_kernel(const float* __restrict__ x, float* __restrict__ xp, int64_t B) {
+  constexpr int PD = pose_dim_of(PDP);
   int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= B * DP) return;
-  int64_t r = i / DP;
-  int c = (int)(i % DP);
-  xp[i] = (c < D) ? x[r * D + c] : 0.f;
+  if (i >= B * PDP) return;
+  int64_t r = i / PDP;
+  int c = (int)(i % PDP);
+  xp[i] = (c < PD) ? x[r * PD + c] : 0.f;
+}
+
+static void launch_pad_x(const float* x, float* xp, int64_t B, int dp, cudaStream_t st) {
+  const int64_t n = B * dp;
+  if (dp == DP128) pad_x_kernel<DP128><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, xp, B);
+  else pad_x_kernel<DP><<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, xp, B);
 }
 
 int simt_time_table(dpb_score* h, const float* labels, int n, float* table, cudaStream_t st) {
@@ -252,28 +260,26 @@ int simt_time_table(dpb_score* h, const float* labels, int n, float* table, cuda
   return DPB_OK;
 }
 
-size_t simt_forward_ws_bytes(int64_t B) {
-  // xpad [B,64] + three [B,1024] fp32 buffers
-  return align_up((size_t)B * DP * 4, 256) + 3 * align_up((size_t)B * H * 4, 256) + 1024;
+size_t simt_forward_ws_bytes(int64_t B, int dp) {
+  // xpad [B,DP] + three [B,1024] fp32 buffers
+  return align_up((size_t)B * dp * 4, 256) + 3 * align_up((size_t)B * H * 4, 256) + 1024;
 }
 
 int simt_forward_raw(dpb_score* h, const float* x, const float* table, const int32_t* t_index, float* raw,
                      int64_t B, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (B <= 0) return DPB_OK;
+  const int dp = h->pose_dp;
   WsCarver c(ws, ws_bytes);
-  float* xp = c.take<float>((size_t)B * DP);
+  float* xp = c.take<float>((size_t)B * dp);
   float* pre = c.take<float>((size_t)B * H);   // pre-activation scratch
   float* hbuf = c.take<float>((size_t)B * H);  // residual stream
   float* tbuf = c.take<float>((size_t)B * H);  // block intermediate
   if (!c.ok() || ws == nullptr) return fail(DPB_ENOMEM, "score forward: workspace too small");
   const int stride = NL * H;
   dim3 gemm_grid(H / BN, (unsigned)((B + BM - 1) / BM));
-  {
-    int64_t n = B * DP;
-    pad_x_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, xp, B);
-  }
+  launch_pad_x(x, xp, B, dp, st);
   // pre_dense + pre_gnorm + act   (model.py:166-169)
-  sgemm_bias_kernel<<<gemm_grid, 256, 0, st>>>(xp, h->pre_w, pre, B, H, DP, table, t_index, stride, nullptr, B);
+  sgemm_bias_kernel<<<gemm_grid, 256, 0, st>>>(xp, h->pre_w, pre, B, H, dp, table, t_index, stride, nullptr, B);
   gn_silu_kernel<<<(unsigned)B, 256, 0, st>>>(pre, h->gn_w[0], h->gn_b[0], nullptr, hbuf, B);
   for (int blk = 0; blk < 2; ++blk) {  // model.py:172-187
     int l1 = 1 + 2 * blk, l2 = 2 + 2 * blk;
@@ -284,16 +290,16 @@ int simt_forward_raw(dpb_score* h, const float* x, const float* table, const int
                                                  t_index, stride, nullptr, B);
     gn_silu_kernel<<<(unsigned)B, 256, 0, st>>>(pre, h->gn_w[l2], h->gn_b[l2], hbuf, hbuf, B);
   }
-  // post_dense (model.py:189), N padded to 64
-  dim3 post_grid(DP / BN, (unsigned)((B + BM - 1) / BM));
-  sgemm_bias_kernel<<<post_grid, 256, 0, st>>>(hbuf, h->post_w, raw, B, DP, H, nullptr, nullptr, 0, h->post_b, B);
+  // post_dense (model.py:189), N padded to DP (64 or 128)
+  dim3 post_grid(dp / BN, (unsigned)((B + BM - 1) / BM));
+  sgemm_bias_kernel<<<post_grid, 256, 0, st>>>(hbuf, h->post_w, raw, B, dp, H, nullptr, nullptr, 0, h->post_b, B);
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;
 }
 
 // raw[0:B] = net(x) and raw[B:2B] = (d net / d x) v  (both before the sigma division), fp32 engine: every GEMM runs on
 // the stacked rows [primal ; tangent] (the tangent rows skip the bias), every GroupNorm + SiLU on its forward-mode twin.
-// ws: simt_forward_ws_bytes(2 B).  Serves the Hutchinson divergence of lib/algorithms/advanced/likelihood.py:26-37:
+// ws: simt_forward_ws_bytes(2 B).  63-D handles only (dpb_score_jvp rejects 126-D).  Serves the Hutchinson divergence of lib/algorithms/advanced/likelihood.py:26-37:
 // eps . (J eps) is the scalar the reference gets from autograd's eps . (J^T eps).
 int simt_forward_jvp_raw(dpb_score* h, const float* x, const float* v, const float* table, const int32_t* t_index,
                          float* raw, int64_t B, void* ws, size_t ws_bytes, cudaStream_t st) {
@@ -307,11 +313,8 @@ int simt_forward_jvp_raw(dpb_score* h, const float* x, const float* v, const flo
   if (!c.ok() || ws == nullptr) return fail(DPB_ENOMEM, "score jvp: workspace too small");
   const int stride = NL * H;
   dim3 gemm_grid(H / BN, (unsigned)((B2 + BM - 1) / BM));
-  {
-    int64_t n = B * DP;
-    pad_x_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, xp, B);
-    pad_x_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(v, xp + (size_t)B * DP, B);
-  }
+  launch_pad_x(x, xp, B, DP, st);
+  launch_pad_x(v, xp + (size_t)B * DP, B, DP, st);
   sgemm_bias_kernel<<<gemm_grid, 256, 0, st>>>(xp, h->pre_w, pre, B2, H, DP, table, t_index, stride, nullptr, B);
   gn_silu_jvp_kernel<<<(unsigned)B, 256, 0, st>>>(pre, h->gn_w[0], h->gn_b[0], nullptr, hbuf, B);
   for (int blk = 0; blk < 2; ++blk) {
@@ -406,11 +409,8 @@ int score_jvp_tc_raw(dpb_score* h, const float* x, const float* v, const float* 
   JvpWs w;
   if (ws == nullptr || jvp_ws_layout(&w, B2, ws, ws_bytes) > ws_bytes) return fail(DPB_ENOMEM, "score jvp: workspace too small");
   const int M = (int)B2, Bi = (int)B;
-  {
-    int64_t n = B * DP;
-    pad_x_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(x, w.xp, B);
-    pad_x_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(v, w.xp + (size_t)B * DP, B);
-  }
+  launch_pad_x(x, w.xp, B, DP, st);
+  launch_pad_x(v, w.xp + (size_t)B * DP, B, DP, st);
 #define JTRY(expr) do { rc = (expr); if (rc != DPB_OK) return rc; } while (0)
   JTRY(split16(w.xp, M, DP, DP, &w.xp16, nullptr, st));
   JTRY(gemm_tc(w.xp16, o->Wpre, M, H, DP, w.pre, H, table, nullptr, nullptr, 0, st, Bi));

@@ -42,13 +42,10 @@ constexpr int CLUSTER = 2;   // CTAs (different row tiles) that share every weig
 constexpr int A_BYTES = TILE_M * BLOCK_K * 2;   // 16 KB
 constexpr int B_BYTES = CHUNK_N * BLOCK_K * 2 / (TWO_SM ? 2 : 1);  // this CTA's share of the weight tile
 constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-constexpr int POST_B_BYTES = DP * BLOCK_K * 2 / (TWO_SM ? 2 : 1);  // post_dense tile (N = 64)
-constexpr int XA_K = 192;
 constexpr int NUM_THREADS = 640;   // 4 single-lane role warps + 16 epilogue warps
 constexpr int EPI_THREADS = 512;
 constexpr int ROLE_REGS = 32;      // setmaxnreg: 640 threads start at 96 registers; the role warpgroup gives, the
 constexpr int EPI_REGS = 112;      // epilogue warpgroups take ((96 - 32) * 128 >= (112 - 96) * 512)
-constexpr int TCOLS = 16;          // pose columns per epilogue thread in the prologue / tail (64 / 4 warps per row quarter)
 static_assert(2 * H / 4 == EPI_THREADS, "parameter staging assumes one float4 of gamma|beta per epilogue thread");
 constexpr int PAR_BYTES = 2 * 3 * H * 4;   // [time bias | gamma | beta] x 1024 floats, double-buffered across layers
 constexpr int STG_BYTES = TILE_M * 128;          // one [128 rows x 64 fp16] SWIZZLE_128B box of outgoing activations
@@ -66,17 +63,31 @@ constexpr int NUM_BARS = 2 * STAGES + 4 + NSUB * 5 + 8;  // full, empty, tfull[2
 constexpr int OFF_PAR = STAGES * STAGE_BYTES;
 constexpr int OFF_STG = OFF_PAR + PAR_BYTES;     // 1024-aligned
 constexpr int OFF_BAR = OFF_STG + STG_TOTAL;
-constexpr int OFF_POSTB = (OFF_BAR + NUM_BARS * 8 + 16 + 15) / 16 * 16;   // post_dense bias (64 floats)
+constexpr int OFF_POSTB = (OFF_BAR + NUM_BARS * 8 + 16 + 15) / 16 * 16;   // post_dense bias (DP floats)
 static_assert(OFF_POSTB % 16 == 0, "post_b is read with 128-bit loads");
-constexpr int OFF_PCROW = OFF_POSTB + DP * 4;           // predictor-corrector mode: per-row squared norms [128][2]
-constexpr int SMEM_BYTES = OFF_PCROW + TILE_M * 2 * 4 + 1024;  // + alignment slack
 static_assert(OFF_STG % 1024 == 0, "staging boxes must be 1024-byte aligned for SWIZZLE_128B");
-static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB per-CTA shared memory limit");
 constexpr int MMA_M = TWO_SM ? 2 * TILE_M : TILE_M;
 constexpr uint32_t IDESC_F16_256 = ptx::umma_idesc_f16(MMA_M, CHUNK_N, 0);
 constexpr uint32_t IDESC_BF16_256 = ptx::umma_idesc_f16(MMA_M, CHUNK_N, 1);
-constexpr uint32_t IDESC_F16_64 = ptx::umma_idesc_f16(MMA_M, DP, 0);
 static_assert(!TWO_SM || CLUSTER == 2, "cta_group::2 needs clusters of exactly two CTAs");
+
+// What depends on the pose width: the kernel is instantiated for the padded width PDP = 64 (63-D axis-angle network)
+// and PDP = 128 (126-D rot6d network).
+template <int PDP>
+struct Width {
+  static constexpr int D = pose_dim_of(PDP);
+  static constexpr int XA_SLABS = PDP / BLOCK_K;   // 64-column slabs of x_hi (and of x_lo): 1 or 2
+  static constexpr int XA_K = 3 * PDP;             // input-layer K-extension [x_hi | x_lo | x_hi]: 192 or 384
+  static constexpr int TCOLS = PDP / 4;            // pose columns per epilogue thread in the prologue / tail (4 warps per row quarter)
+  static constexpr int POST_B_BYTES = PDP * BLOCK_K * 2 / (TWO_SM ? 2 : 1);   // this CTA's share of a post_dense tile (N = PDP)
+  static constexpr int OFF_PCROW = OFF_POSTB + PDP * 4;   // predictor-corrector mode: per-row squared norms [128][2]
+  static constexpr int SMEM_BYTES = OFF_PCROW + TILE_M * 2 * 4 + 1024;   // + alignment slack
+  static constexpr uint32_t IDESC_POST = ptx::umma_idesc_f16(MMA_M, PDP, 0);
+  static_assert(SMEM_BYTES <= 232448, "exceeds the 227 KB per-CTA shared memory limit");
+  // x occupies the A halves of the first 2 XA_SLABS ring stages during the input layer
+  static_assert(2 * XA_SLABS <= STAGES, "the input-layer operand needs 2 * XA_SLABS ring stages");
+  static_assert(TCOLS == 16 || TCOLS == 32, "the tail reads TCOLS accumulator columns with one tcgen05.ld");
+};
 
 struct KParams {
   int mode, n_steps, impute, noise_k, n_tiles;
@@ -311,14 +322,33 @@ __device__ __forceinline__ void gn_silu_group(const uint32_t* vr, const float* t
 // K-slab visited at loop position k: the boxes of the previous layer's last chunk are produced in the order
 // (hf0,gp0), (hf1,gp0), (hf0,gp1), (hf1,gp1) = slabs 12, 14, 13, 15, so positions 13 and 14 trade places
 __device__ __forceinline__ int kslab(int layer, int k) { return (layer > 0 && (k == 13 || k == 14)) ? 27 - k : k; }
-__device__ __forceinline__ int layer_nk(int layer) { return layer == 0 ? XA_K / BLOCK_K : H / BLOCK_K; }
+template <int PDP>
+__device__ __forceinline__ int layer_nk(int layer) { return layer == 0 ? Width<PDP>::XA_K / BLOCK_K : H / BLOCK_K; }
 __device__ __forceinline__ int layer_chunks(int layer) { return layer == 5 ? 1 : H / CHUNK_N; }
 
 // First-layer operand.  x[TCOLS] (fp32, columns c0..c0+TCOLS-1 of row r) -> bf16 hi and lo parts, written straight into
-// the A halves of ring stages 0 (hi) and 1 (lo) in the SWIZZLE_128B K-major layout the MMA reads ([128 rows x 64]:
-// row pitch 128 B, 16-byte chunk j of row r stored at chunk j ^ (r & 7)).  The first layer streams only weight tiles
-// through the ring, so the A halves are free while it runs; K slab 2 of [x_hi | x_lo | x_hi] reuses the hi tile.
-__device__ __forceinline__ void write_xa(uint32_t hi_base, uint32_t lo_base, int r, int c0, const float* x) {
+// the A halves of the ring stages in the SWIZZLE_128B K-major layout the MMA reads ([128 rows x 64]: row pitch 128 B,
+// 16-byte chunk j of row r stored at chunk j ^ (r & 7)).  x_hi column slab s (64 columns) goes to stage s, x_lo slab s
+// to stage XA_SLABS + s: stages 0 | 1 at 64 columns, 0, 1 | 2, 3 at 128.  The first layer streams only weight tiles
+// through the ring, so the A halves are free while it runs; the last third of [x_hi | x_lo | x_hi] reuses the hi tiles.
+// The caller passes the A half of stage 0 (xa_base); the thread's TCOLS columns lie inside one slab.
+// A half holding input-layer K slab ks (of 3 XA_SLABS), relative to ring stage 0
+template <int PDP>
+__device__ __forceinline__ uint32_t xa_stage_offset(int ks) {
+  constexpr int NS = Width<PDP>::XA_SLABS;
+  if constexpr (NS == 1) return ks == 1 ? STAGE_BYTES : 0;
+  else return (uint32_t)(ks < 2 * NS ? ks : ks - 2 * NS) * STAGE_BYTES;
+}
+
+template <int PDP>
+__device__ __forceinline__ void write_xa(uint32_t xa_base, int r, int c0, const float* x) {
+  constexpr int TCOLS = Width<PDP>::TCOLS;
+  uint32_t hi_base = xa_base, lo_base = xa_base + STAGE_BYTES;
+  if constexpr (Width<PDP>::XA_SLABS > 1) {
+    hi_base = xa_base + (uint32_t)(c0 / BLOCK_K) * STAGE_BYTES;
+    lo_base = hi_base + (uint32_t)Width<PDP>::XA_SLABS * STAGE_BYTES;
+    c0 %= BLOCK_K;
+  }
   uint32_t hi[TCOLS / 2], lo[TCOLS / 2];
 #pragma unroll
   for (int i = 0; i < TCOLS / 2; ++i) {
@@ -338,8 +368,10 @@ __device__ __forceinline__ void write_xa(uint32_t hi_base, uint32_t lo_base, int
 
 // Gaussian draws for this thread's TCOLS columns: caller-supplied plane or Philox (slot, step); the Philox
 // addressing (row, step, slot, quad = column / 4) does not depend on how columns are split over threads
+template <int PDP>
 __device__ __forceinline__ void draw_cols(const float* plane, long long row, int c0, unsigned long long seed,
                                           uint32_t step, uint32_t slot, float* z) {
+  constexpr int TCOLS = Width<PDP>::TCOLS, D = Width<PDP>::D;
   if (plane) {
 #pragma unroll
     for (int i = 0; i < TCOLS; ++i) {
@@ -348,16 +380,21 @@ __device__ __forceinline__ void draw_cols(const float* plane, long long row, int
     }
   } else {
 #pragma unroll
-    for (int j = 0; j < TCOLS / 4; ++j) normal4(seed, (uint64_t)row, step, slot, (uint32_t)(c0 / 4 + j), z + 4 * j);
+    for (int j = 0; j < TCOLS / 4; ++j)
+      normal4(seed, (uint64_t)row, step, slot, (uint32_t)(c0 / 4 + j), z + 4 * j, (uint32_t)(PDP / 4));
   }
 }
 
+template <int PDP>
 __global__ void __cluster_dims__(CLUSTER, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 score_tc_kernel(const __grid_constant__ KParams p,
                 const __grid_constant__ CUtensorMap tm_h, const __grid_constant__ CUtensorMap tm_t,
                 const __grid_constant__ CUtensorMap tm_pre, const __grid_constant__ CUtensorMap tm_w0,
                 const __grid_constant__ CUtensorMap tm_w1, const __grid_constant__ CUtensorMap tm_w2,
                 const __grid_constant__ CUtensorMap tm_w3, const __grid_constant__ CUtensorMap tm_post) {
+  // the pose width of this instantiation (these hide the 63-D namespace constants D / DP)
+  using Wd = Width<PDP>;
+  constexpr int DP = PDP, D = Wd::D, TCOLS = Wd::TCOLS;
   extern __shared__ uint8_t smem_raw[];
   // 1024-byte alignment for SWIZZLE_128B; offset arithmetic on the __shared__ array keeps ld/st.shared
   uint8_t* smem = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -443,8 +480,8 @@ score_tc_kernel(const __grid_constant__ KParams p,
           for (int layer = 0; layer < 6; ++layer) {
             const CUtensorMap* tm = layer == 0 ? &tm_pre : layer == 1 ? &tm_w0 : layer == 2 ? &tm_w1
                                   : layer == 3 ? &tm_w2 : layer == 4 ? &tm_w3 : &tm_post;
-            const uint32_t bytes = layer == 5 ? POST_B_BYTES : B_BYTES;
-            const int nk = layer_nk(layer), nc = layer_chunks(layer);
+            const uint32_t bytes = layer == 5 ? Wd::POST_B_BYTES : B_BYTES;
+            const int nk = layer_nk<PDP>(layer), nc = layer_chunks(layer);
             for (int chunk = 0; chunk < nc; ++chunk)
              for (int sub = 0; sub < NSUB; ++sub)
               for (int k = 0; k < nk; ++k) {
@@ -483,8 +520,8 @@ score_tc_kernel(const __grid_constant__ KParams p,
       for (SegIter it(worker, n_workers, n_units, p.n_steps); it.next(sg);)
         for (int step = sg.s0; step < sg.s1; ++step)
           for (int layer = 0; layer < 6; ++layer) {
-            const uint32_t idesc = layer == 0 ? IDESC_BF16_256 : layer == 5 ? IDESC_F16_64 : IDESC_F16_256;
-            const int nk = layer_nk(layer), nc = layer_chunks(layer);
+            const uint32_t idesc = layer == 0 ? IDESC_BF16_256 : layer == 5 ? Wd::IDESC_POST : IDESC_F16_256;
+            const int nk = layer_nk<PDP>(layer), nc = layer_chunks(layer);
             for (int cs = 0; cs < nc * NSUB; ++cs) {   // (chunk, sub) pairs; chunk_ctr & 1 == sub
               const uint32_t buf = chunk_ctr & 1;
               if (!DBG(64)) PROF_WAIT(0, ptx::mbar_wait(tempty_bar(buf), ((tph >> buf) & 1) ^ 1));
@@ -497,8 +534,9 @@ score_tc_kernel(const __grid_constant__ KParams p,
                 const int ks = kslab(layer, k);
                 // first chunk of a layer: the last four K slabs are still in the staging boxes of the previous layer
                 const bool direct = layer > 0 && cs == 0 && ks >= DIRECT_K0 && !DBG(64);
-                // first layer: x_hi | x_lo | x_hi, written by the epilogue into the A halves of ring stages 0 / 1
-                const uint32_t a_addr = layer == 0 ? smem_base + (ks == 1 ? STAGE_BYTES : 0)
+                // first layer: x_hi | x_lo | x_hi, written by the epilogue into the A halves of ring stages
+                // 0 .. 2 XA_SLABS - 1 (slab ks; the last third re-reads the x_hi stages)
+                const uint32_t a_addr = layer == 0 ? smem_base + xa_stage_offset<PDP>(ks)
                                       : direct ? stg_base + (ks - DIRECT_K0) * STG_BYTES : s_addr;
                 const uint64_t adesc = ptx::umma_desc_sw128(a_addr);
                 const uint64_t bdesc = ptx::umma_desc_sw128(s_addr + A_BYTES);
@@ -535,10 +573,12 @@ score_tc_kernel(const __grid_constant__ KParams p,
           for (int layer = 0; layer < 6; ++layer) {
             // layer input: x (shared memory, written by the epilogue) | H | T | H | T | H
             const CUtensorMap* tm = (layer == 2 || layer == 4) ? &tm_t : &tm_h;
-            const int nk = layer_nk(layer), nc = layer_chunks(layer);
+            const int nk = layer_nk<PDP>(layer), nc = layer_chunks(layer);
             if (layer == 1 && !DBG(64)) {
-              // the first layer's operand lives in the A halves of ring stages 0 / 1: no activation tile may land
-              // there before ALL first-layer MMAs have retired (= the accumulator of its last chunk is complete)
+              // the first layer's operand lives in the A halves of ring stages 0 .. 2 XA_SLABS - 1 (0 / 1, or 0 - 3 at
+              // 128 columns): no activation tile may land in ANY stage before ALL first-layer MMAs have retired (= the
+              // accumulator of its last chunk is complete).  This wait precedes the first load of the next layer, so it
+              // covers every stage the operand occupies.
               const uint32_t n = cctr - 1;
               PROF_WAIT(1, ptx::mbar_wait(tfull_bar(n & 1), (n >> 1) & 1));
             }
@@ -656,7 +696,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
     const int sg2 = ((warp - 4) >> 2) & 1;
     const int et = threadIdx.x - 128;
     const int r_in = q * 32 + lane;
-    const int c0 = hf * 32 + sg2 * TCOLS;   // first of this thread's TCOLS pose columns (prologue / tail)
+    const int c0 = hf * (2 * TCOLS) + sg2 * TCOLS;   // first of this thread's TCOLS pose columns (prologue / tail)
     const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
     uint32_t chunk_ctr = 0, tph = 0, scnt = 0;
     auto signal = [&](uint32_t bar) {  // generic-proxy shared-memory writes -> visible to the MMA (async proxy) reads
@@ -664,7 +704,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
       __syncwarp();
       if (lane == 0) ptx::mbar_arrive(bar);
     };
-    const uint32_t xa_hi = smem_base, xa_lo = smem_base + STAGE_BYTES;   // A halves of ring stages 0 and 1
+    const uint32_t xa_base = smem_base;   // A half of ring stage 0 (write_xa places the slabs)
     auto tempty_arrive = [&](uint32_t buf) {
       ptx::tc_fence_before();
       __syncwarp();
@@ -711,7 +751,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
             }
             if (p.impute && sg.s0 == 0 && !p.pc) {  // imputation that follows the (none) corrector of step 0, sampling.py:459
               float zc[TCOLS];
-              draw_cols(p.noise ? p.noise : nullptr, row, c0, p.seed, (uint32_t)p.step_offset, 0, zc);
+              draw_cols<PDP>(p.noise ? p.noise : nullptr, row, c0, p.seed, (uint32_t)p.step_offset, 0, zc);
               const float al = p.coef[3], sd = p.coef[4];
 #pragma unroll
               for (int i = 0; i < TCOLS; ++i) {
@@ -730,7 +770,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
             }
           } else {  // prior loss: x_t = alpha x0 + std z
             float z[TCOLS];
-            draw_cols(p.z, row, c0, p.seed, (uint32_t)p.step_offset, 3, z);
+            draw_cols<PDP>(p.z, row, c0, p.seed, (uint32_t)p.step_offset, 3, z);
 #pragma unroll
             for (int i = 0; i < TCOLS; ++i) {
               int col = c0 + i;
@@ -738,7 +778,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
             }
           }
         }
-        write_xa(xa_hi, xa_lo, r_in, c0, x);
+        write_xa<PDP>(xa_base, r_in, c0, x);
         signal(xa_bar(sub));
 #pragma unroll
         for (int i = 0; i < TCOLS; ++i) xs[sub][i] = x[i];
@@ -842,7 +882,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
           const uint32_t gstep = (uint32_t)(p.step_offset + (unsigned long long)lstep);
           const size_t plane = (size_t)p.B * D;
           float ca = 0.f, cb = 0.f, cc = 0.f, al = 0.f, sd = 0.f;
-          // given noise: [n, K, B, 63] planes of the predictor; with the corrector [n, K + 1, B, 63], its draw first
+          // given noise: [n, K, B, D] planes of the predictor; with the corrector [n, K + 1, B, D], its draw first
           const float* nzc = p.noise ? p.noise + (size_t)lstep * (p.noise_k + (p.pc ? 1 : 0)) * plane : nullptr;
           const float* nz = (nzc && p.pc) ? nzc + plane : nzc;
           float zp[TCOLS];
@@ -850,8 +890,8 @@ score_tc_kernel(const __grid_constant__ KParams p,
           for (int i = 0; i < TCOLS; ++i) zp[i] = 0.f;
           if (p.mode == 1 && valid) {
             ca = cf[0]; cb = cf[1]; cc = cf[2]; al = cf[3]; sd = cf[4];
-            if (corr) draw_cols(nzc, row, c0, p.seed, gstep, 4, zp);          // the Langevin draw (Philox slot 4)
-            else draw_cols(nz ? nz + (p.noise_k == 3 ? plane : 0) : nullptr, row, c0, p.seed, gstep, 1, zp);
+            if (corr) draw_cols<PDP>(nzc, row, c0, p.seed, gstep, 4, zp);          // the Langevin draw (Philox slot 4)
+            else draw_cols<PDP>(nz ? nz + (p.noise_k == 3 ? plane : 0) : nullptr, row, c0, p.seed, gstep, 1, zp);
           }
           if (p.mode == 1) {  // pin the draws above the wait (the compiler would otherwise sink them below it)
 #pragma unroll
@@ -861,7 +901,8 @@ score_tc_kernel(const __grid_constant__ KParams p,
           PROF_BEGIN(tail_t0)
           ptx::tc_fence_after();
           uint32_t vr[TCOLS];
-          ptx::tmem_ld_32x16(tmem_base + lane_addr + buf * CHUNK_N + c0, vr);
+          if constexpr (TCOLS == 32) ptx::tmem_ld_32x32(tmem_base + lane_addr + buf * CHUNK_N + c0, vr);
+          else ptx::tmem_ld_32x16(tmem_base + lane_addr + buf * CHUNK_N + c0, vr);
           ptx::tmem_ld_wait();
           tempty_arrive(buf);
 #ifdef DPB_TC_PROFILE_TAIL
@@ -889,11 +930,11 @@ score_tc_kernel(const __grid_constant__ KParams p,
             float x[TCOLS];
 #pragma unroll
             for (int i = 0; i < TCOLS; ++i) x[i] = xs[sub][i] + 1e-9f * raw[i];
-            write_xa(xa_hi, xa_lo, r_in, c0, x);
+            write_xa<PDP>(xa_base, r_in, c0, x);
             signal(xa_bar(sub));
           } else if (p.mode == 1 && corr) {
             // ---- Langevin corrector (sampling.py:282-302): grad = score, batch-global mean norms, x += step grad + sqrt(2 step) z
-            float* rowsq = reinterpret_cast<float*>(smem + OFF_PCROW);
+            float* rowsq = reinterpret_cast<float*>(smem + Wd::OFF_PCROW);
             float gsq = 0.f, zsq = 0.f;
             float grad[TCOLS];
 #pragma unroll
@@ -938,7 +979,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
             for (int i = 0; i < TCOLS; ++i) x[i] = valid ? (xs[sub][i] + stp * grad[i]) + sq * zp[i] : 0.f;
             if (valid && p.impute) {                         // imputation after the corrector (sampling.py:459, 413-422)
               float zc[TCOLS];
-              draw_cols(nz, row, c0, p.seed, gstep, 0, zc);
+              draw_cols<PDP>(nz, row, c0, p.seed, gstep, 0, zc);
 #pragma unroll
               for (int i = 0; i < TCOLS; ++i) {
                 int col = c0 + i;
@@ -950,7 +991,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
             }
 #pragma unroll
             for (int i = 0; i < TCOLS; ++i) xs[sub][i] = x[i];
-            write_xa(xa_hi, xa_lo, r_in, c0, x);             // the predictor sub-step always follows
+            write_xa<PDP>(xa_base, r_in, c0, x);             // the predictor sub-step always follows
             signal(xa_bar(sub));
           } else if (p.mode == 1) {
             float x[TCOLS];
@@ -970,7 +1011,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
               //  before anything reads them: the draw is skipped, results are identical)
               if (p.impute && (last || p.traj || p.pc)) {
                 float zi[TCOLS];
-                draw_cols(nz ? nz + 2 * plane : nullptr, row, c0, p.seed, gstep, 2, zi);
+                draw_cols<PDP>(nz ? nz + 2 * plane : nullptr, row, c0, p.seed, gstep, 2, zi);
 #pragma unroll
                 for (int i = 0; i < TCOLS; ++i) {
                   int col = c0 + i;
@@ -990,7 +1031,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
               if (!last && p.impute && !p.pc) {  // imputation in the corrector slot of the NEXT step precedes its score eval
                 float zc[TCOLS];
                 const float* nz1 = p.noise ? p.noise + (size_t)(step + 1) * p.noise_k * plane : nullptr;
-                draw_cols(nz1, row, c0, p.seed, gstep + 1, 0, zc);
+                draw_cols<PDP>(nz1, row, c0, p.seed, gstep + 1, 0, zc);
                 const float al1 = cf[DPB_COEF_STRIDE + 3], sd1 = cf[DPB_COEF_STRIDE + 4];
 #pragma unroll
                 for (int i = 0; i < TCOLS; ++i) {
@@ -1013,10 +1054,10 @@ score_tc_kernel(const __grid_constant__ KParams p,
             for (int i = 0; i < TCOLS; ++i) xs[sub][i] = x[i];
             if (step + 1 < sg.s1) {  // (a segment that stops mid-chain leaves x in x_io for the cluster that continues)
 #ifdef DPB_TC_PROFILE_TAIL
-              PROF_WAIT(2, write_xa(xa_hi, xa_lo, r_in, c0, x));
+              PROF_WAIT(2, write_xa<PDP>(xa_base, r_in, c0, x));
               PROF_WAIT(1, signal(xa_bar(sub)));
 #else
-              write_xa(xa_hi, xa_lo, r_in, c0, x);
+              write_xa<PDP>(xa_base, r_in, c0, x);
               signal(xa_bar(sub));
 #endif
             }
@@ -1024,7 +1065,7 @@ score_tc_kernel(const __grid_constant__ KParams p,
             float acc = 0.f;
             if (valid) {
               float z[TCOLS];
-              draw_cols(p.z, row, c0, p.seed, (uint32_t)p.step_offset, 3, z);
+              draw_cols<PDP>(p.z, row, c0, p.seed, (uint32_t)p.step_offset, 3, z);
               float racc = 0.f;
 #pragma unroll
               for (int i = 0; i < TCOLS; ++i) {
@@ -1097,26 +1138,27 @@ int make_tmap_2d(CUtensorMap* m, CUtensorMapDataType dt, const void* ptr, uint64
 
 int tc_prepare(dpb_score* h, const dpb_score_weights* w) {
   h->tc_ready = false;
-  // fp16 copies of the square layers and post_dense (zero row 63), bf16 hi/hi/lo split of pre_dense
+  const int hd = h->pose_dim, hdp = h->pose_dp, xa_k = 3 * hdp;
+  // fp16 copies of the square layers and post_dense (zero rows D..DP-1), bf16 hi/hi/lo split of pre_dense
   std::vector<__half> buf((size_t)H * H);
   for (int l = 0; l < 4; ++l) {
     for (size_t i = 0; i < (size_t)H * H; ++i) buf[i] = __float2half_rn(w->blk_w[l][i]);
     DPB_CUDA_CHECK(cudaMalloc((void**)&h->w16[l], buf.size() * sizeof(__half)));
     DPB_CUDA_CHECK(cudaMemcpy(h->w16[l], buf.data(), buf.size() * sizeof(__half), cudaMemcpyHostToDevice));
   }
-  std::vector<__half> post((size_t)DP * H, __float2half_rn(0.f));
-  for (size_t i = 0; i < (size_t)D * H; ++i) post[i] = __float2half_rn(w->post_w[i]);
+  std::vector<__half> post((size_t)hdp * H, __float2half_rn(0.f));
+  for (size_t i = 0; i < (size_t)hd * H; ++i) post[i] = __float2half_rn(w->post_w[i]);
   DPB_CUDA_CHECK(cudaMalloc((void**)&h->post16, post.size() * sizeof(__half)));
   DPB_CUDA_CHECK(cudaMemcpy(h->post16, post.data(), post.size() * sizeof(__half), cudaMemcpyHostToDevice));
-  std::vector<__nv_bfloat16> pre((size_t)H * tc::XA_K, __float2bfloat16_rn(0.f));
+  std::vector<__nv_bfloat16> pre((size_t)H * xa_k, __float2bfloat16_rn(0.f));
   for (int o = 0; o < H; ++o)
-    for (int k = 0; k < D; ++k) {
-      float v = w->pre_w[(size_t)o * D + k];
+    for (int k = 0; k < hd; ++k) {
+      float v = w->pre_w[(size_t)o * hd + k];
       __nv_bfloat16 hi = __float2bfloat16_rn(v);
       __nv_bfloat16 lo = __float2bfloat16_rn(v - __bfloat162float(hi));
-      pre[(size_t)o * tc::XA_K + k] = hi;         // pairs with x_hi
-      pre[(size_t)o * tc::XA_K + 64 + k] = hi;    // pairs with x_lo
-      pre[(size_t)o * tc::XA_K + 128 + k] = lo;   // pairs with x_hi
+      pre[(size_t)o * xa_k + k] = hi;             // pairs with x_hi
+      pre[(size_t)o * xa_k + hdp + k] = hi;       // pairs with x_lo
+      pre[(size_t)o * xa_k + 2 * hdp + k] = lo;   // pairs with x_hi
     }
   DPB_CUDA_CHECK(cudaMalloc((void**)&h->pre_split, pre.size() * sizeof(__nv_bfloat16)));
   DPB_CUDA_CHECK(cudaMemcpy(h->pre_split, pre.data(), pre.size() * sizeof(__nv_bfloat16), cudaMemcpyHostToDevice));
@@ -1168,21 +1210,26 @@ int tc_prepare(dpb_score* h, const dpb_score_weights* w) {
   for (int l = 0; l < 4 && rc == DPB_OK; ++l)
     rc = make_tmap_2d(&h->tm_w[l], CU_TENSOR_MAP_DATA_TYPE_FLOAT16, h->w16[l], H, H, tc::BLOCK_K,
                       tc::CHUNK_N / tc::CLUSTER, 2);
-  if (rc == DPB_OK) rc = make_tmap_2d(&h->tm_post, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, h->post16, H, DP, tc::BLOCK_K,
-                                    DP / tc::CLUSTER, 2);
+  if (rc == DPB_OK) rc = make_tmap_2d(&h->tm_post, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, h->post16, H, hdp, tc::BLOCK_K,
+                                    hdp / tc::CLUSTER, 2);
   if (rc == DPB_OK)
-    rc = make_tmap_2d(&h->tm_pre, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, h->pre_split, tc::XA_K, H, tc::BLOCK_K,
+    rc = make_tmap_2d(&h->tm_pre, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, h->pre_split, xa_k, H, tc::BLOCK_K,
                       tc::CHUNK_N / tc::CLUSTER, 2);
   if (rc == DPB_OK)
     rc = make_tmap_2d(&h->tm_act_h, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, h->act_h, H, rows, tc::BLOCK_K, tc::TILE_M, 2);
   if (rc == DPB_OK)
     rc = make_tmap_2d(&h->tm_act_t, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, h->act_t, H, rows, tc::BLOCK_K, tc::TILE_M, 2);
   if (rc != DPB_OK) return rc;
-  DPB_CUDA_CHECK(cudaFuncSetAttribute(tc::score_tc_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      tc::SMEM_BYTES));
+  if (hdp == DP128)
+    DPB_CUDA_CHECK(cudaFuncSetAttribute(tc::score_tc_kernel<DP128>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        tc::Width<DP128>::SMEM_BYTES));
+  else
+    DPB_CUDA_CHECK(cudaFuncSetAttribute(tc::score_tc_kernel<DP>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                        tc::Width<DP>::SMEM_BYTES));
   DPB_CUDA_CHECK(cudaMalloc((void**)&h->pc_buf, (2 * PC_MAX_STEPS + 4) * sizeof(float)));
   h->tc_ready = true;
-  return tcs_prepare(h);
+  // the small-batch engine (score_small.cu) is built for the 63-D network only; 126-D handles always use the kernel above
+  return hd == DPB_POSE_DIM ? tcs_prepare(h) : DPB_OK;
 }
 
 // the fused predictor-corrector mode needs every CTA to own one tile for the whole run (grid-wide norms per step)
@@ -1244,7 +1291,7 @@ int tc_launch(dpb_score* h, const TcJob& j, cudaStream_t st) {
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3((unsigned)grid);
     cfg.blockDim = dim3(tc::NUM_THREADS);
-    cfg.dynamicSmemBytes = tc::SMEM_BYTES;
+    cfg.dynamicSmemBytes = h->pose_dp == DP128 ? tc::Width<DP128>::SMEM_BYTES : tc::Width<DP>::SMEM_BYTES;
     cfg.stream = st;
     cudaLaunchAttribute attr[1];
     int n_attr = 0;
@@ -1259,8 +1306,12 @@ int tc_launch(dpb_score* h, const TcJob& j, cudaStream_t st) {
     }
     cfg.attrs = attr;
     cfg.numAttrs = n_attr;
-    DPB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, tc::score_tc_kernel, p, h->tm_act_h, h->tm_act_t, h->tm_pre, h->tm_w[0],
-                                      h->tm_w[1], h->tm_w[2], h->tm_w[3], h->tm_post));
+    if (h->pose_dp == DP128)
+      DPB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, tc::score_tc_kernel<DP128>, p, h->tm_act_h, h->tm_act_t, h->tm_pre,
+                                        h->tm_w[0], h->tm_w[1], h->tm_w[2], h->tm_w[3], h->tm_post));
+    else
+      DPB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, tc::score_tc_kernel<DP>, p, h->tm_act_h, h->tm_act_t, h->tm_pre, h->tm_w[0],
+                                        h->tm_w[1], h->tm_w[2], h->tm_w[3], h->tm_post));
   }
   DPB_CUDA_CHECK(cudaGetLastError());
 #ifdef DPB_TC_PROFILE

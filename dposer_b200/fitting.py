@@ -42,6 +42,9 @@ class MotionDenoise(MotionPrior):
     def __init__(self, config, args, diffusion_model, body_model, sde, normalizer, sde_N=1000, dposer_weight=1.0,
                  out_path=None, debug=False, batch_size=1, seq_len=None):
         """batch_size = total rows (frames).  seq_len = frames per independent sequence (default: one sequence)."""
+        if getattr(diffusion_model, 'is_rot6d', False):
+            raise NotImplementedError('MotionDenoise runs the 63-D axis prior natively; a rot6d (126-D) prior needs an '
+                                      'axis-to-rot6d kernel and its Jacobian in the native step chain')
         sde.N = sde_N                                            # run/motion_denoising.py:91
         super().__init__(diffusion_model, sde, config.training.continuous, batch_size)
         self.args, self.debug, self.device = args, debug, args.device
@@ -173,6 +176,9 @@ class SMPLify:
 
     def __init__(self, body_model, step_size=1e-2, batch_size=32, num_iters=100, focal_length=5000, args=None,
                  pose_prior=None, per_problem=True):
+        if pose_prior is not None and getattr(pose_prior.model, 'is_rot6d', False):
+            raise NotImplementedError('SMPLify runs the 63-D axis prior natively; a rot6d (126-D) DPoser prior needs an '
+                                      'axis-to-rot6d kernel and its Jacobian in the native step chain')
         self.smpl = body_model
         self.device = getattr(args, 'device', None)
         self.focal_length = focal_length

@@ -47,6 +47,9 @@ def get_likelihood_fn(sde, inverse_scaler, hutchinson_type='Rademacher', rtol=1e
     """likelihood.py:40-113.  ``likelihood_fn(model, data, epsilon=None)``: ``epsilon`` fixes the probe (parity tests)."""
 
     def likelihood_fn(model, data, epsilon=None):
+        if getattr(model, 'is_rot6d', False):
+            raise NotImplementedError('likelihood evaluation (score-network JVP) is built for the 63-D axis network, not '
+                                      'for rot6d (126-D) score networks')
         with torch.no_grad():
             L.require_cuda(data, 'data')
             data = data.to(torch.float32)

@@ -58,6 +58,9 @@ def _tensor_struct(model, pick):
 class _Engine:
     def __init__(self, model, B, device):
         from .model import embedding_freqs
+        if getattr(model, 'is_rot6d', False):
+            raise NotImplementedError('the training kernels are built for the 63-D axis network, not for rot6d (126-D) '
+                                      'score networks')
         if not model._geometry_ok:
             raise NotImplementedError('the training kernels are built for the shipped geometry (63-D pose, hidden 1024, '
                                       'embed 512, 2 blocks)')

@@ -70,8 +70,7 @@ class Posenormalizer:
     """lib/dataset/AMASS.py:187-259.  ``data_path`` may be the reference's ``.../train`` directory (with
     {axis,rot6d}_normalize{1,2}.pt) or None for the AMASS statistics shipped in dposer_b200/data/amass_stats[_rot6d].npz
     (extracted from the reference's own files).  ``rot_rep='rot6d'`` normalises 126-D poses (``from_axis`` / ``to_axis``
-    convert at the boundary, AMASS.py:200-201,254-256); the score-net kernels themselves are built for the shipped 63-D
-    axis-angle geometry only."""
+    convert at the boundary, AMASS.py:200-201,254-256); the score-net kernels run 63-D (axis) and 126-D (rot6d) networks."""
 
     def __init__(self, data_path=None, device='cuda:0', normalize=True, min_max=True, rot_rep=None):
         assert rot_rep in ['rot6d', 'axis']

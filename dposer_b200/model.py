@@ -84,7 +84,9 @@ class ScoreModelFC(nn.Module):
             setattr(self, f'b{idx + 1}_dense2_t', nn.Linear(embed_dim, hidden_dim))
             setattr(self, f'b{idx + 1}_gnorm2', nn.GroupNorm(32, num_channels=hidden_dim))
         self.post_dense = nn.Linear(hidden_dim, n_poses * pose_dim)
-        self._geometry_ok = (n_poses * pose_dim == L.POSE_DIM and hidden_dim == L.HIDDEN and
+        # input / output width D: 63 (axis-angle, pose_dim=3) or 126 (rot6d, pose_dim=6)
+        self.pose_width = n_poses * pose_dim
+        self._geometry_ok = (self.pose_width in L.POSE_DIMS and hidden_dim == L.HIDDEN and
                              embed_dim == L.EMBED and n_blocks == 2)
         self._h = None
         self._ws = {}
@@ -105,8 +107,8 @@ class ScoreModelFC(nn.Module):
         if dev.type != 'cuda':
             raise RuntimeError('dposer_b200.ScoreModelFC runs on CUDA only (no CPU fallback): call .cuda() first')
         if not self._geometry_ok:
-            raise NotImplementedError('kernels are built for the shipped geometry: 63-D pose, hidden 1024, '
-                                      'embed 512, 2 blocks (configs/subvp/amass_scorefc_continuous.py)')
+            raise NotImplementedError('kernels are built for the shipped geometry: 63-D (axis) or 126-D (rot6d) pose, '
+                                      'hidden 1024, embed 512, 2 blocks (configs/subvp/amass_scorefc_continuous.py)')
         ver = self._param_versions()
         if self._h is not None and self._h.versions == ver:
             return self._h
@@ -131,7 +133,7 @@ class ScoreModelFC(nn.Module):
         w.post_w, w.post_b = hp(self.post_dense.weight), hp(self.post_dense.bias)
         w.emb_freqs = hp(embedding_freqs(L.EMBED))
         out = C.c_void_p()
-        L.check(lib.dpb_score_create(C.byref(out), C.byref(w), dev.index or 0), 'dpb_score_create')
+        L.check(lib.dpb_score_create_dim(C.byref(out), C.byref(w), self.pose_width, dev.index or 0), 'dpb_score_create_dim')
         self._h = _Handle(out, dev, ver)
         return self._h
 
@@ -162,11 +164,12 @@ class ScoreModelFC(nn.Module):
         a device reduction and (b) every schedule scalar is the CPU-fp32 value the reference would compute
         (``1 - exp(2 lmc)`` loses ~5e-4 relative at t=1e-3 to a single ulp of exp, so the device's exp must
         not be used for it).  The time path is evaluated once per distinct label."""
+        self.check_width(x, 'batch')
         h = self.handle()
         L.require_cuda(x, 'batch')
         x = x.detach().to(torch.float32).contiguous()
         B = x.shape[0]
-        out = torch.empty(B, L.POSE_DIM, dtype=torch.float32, device=x.device)
+        out = torch.empty(B, self.pose_width, dtype=torch.float32, device=x.device)
         if B == 0:
             return out
         labels = labels.detach().to(device='cpu', dtype=torch.float32).reshape(-1)
@@ -189,8 +192,20 @@ class ScoreModelFC(nn.Module):
                                            B, self.engine, L.ptr(ws), ws.numel(), L.current_stream(x.device)))
         return out
 
+    def check_width(self, x, name, rows=None):
+        """``x`` must be [B, D] with D the network's pose width (63 axis-angle, 126 rot6d) and, if given, B = ``rows``:
+        the kernels index every such buffer as [B, D], so a tensor of the other width must be rejected before them."""
+        if x.dim() != 2 or x.shape[1] != self.pose_width or (rows is not None and x.shape[0] != rows):
+            want = f'[{"B" if rows is None else rows}, {self.pose_width}]'
+            raise ValueError(f'{name}: expected {want} for this {self.pose_width}-D score network, got {list(x.shape)}')
+
+    @property
+    def is_rot6d(self):
+        return self.pose_width == L.POSE_DIM_ROT6D
+
     def forward(self, batch, t, condition=None, mask=None):
-        """batch [B,63], t [B] (labels, i.e. t*999 when called through score_fn) -> [B,63]  (model.py:141-196)."""
+        """batch [B,D], t [B] (labels, i.e. t*999 when called through score_fn) -> [B,D]  (model.py:141-196);
+        D = 63 (axis-angle) or 126 (rot6d)."""
         if self.training:
             raise NotImplementedError('ScoreModelFC.forward is the inference path; training goes through dposer_b200.losses '
                                       '(get_step_fn / get_sde_loss_fn: loss and gradients in one native call)')

@@ -77,6 +77,9 @@ class _PriorBase:
         return float(vec_t.reshape(-1)[0])
 
     def _fused_loss(self, x_0, t, weighted, divisor, z=None):
+        self.model.check_width(x_0, 'x_0')
+        if z is not None:
+            self.model.check_width(z, 'z', x_0.shape[0])
         seed = mutils.host_seed() if z is None else 0
         return _PriorLossFn.apply(x_0, self, t, weighted, divisor, z, seed)
 
@@ -93,6 +96,7 @@ class _PriorBase:
         so the N steps are ONE ``dpb_sampler_run`` with an N-row coefficient table (noise coefficient 0): with the tcgen05
         engine a single persistent kernel, like the reverse-SDE sampler."""
         from . import sampling
+        self.model.check_width(x_t, 'x_t')
         t0, t1 = self._host_t(t), self._host_t(t_end)
         traj = torch.linspace(0, 1, N + 1)
         traj = (1 - traj) * t0 + traj * t1                      # linear_interpolation (lib/utils/misc.py:58-61)
@@ -119,6 +123,9 @@ class _PriorBase:
 
     def _ddim_loss(self, x_0, vec_t, weighted, divisor, n, z=None):
         """multi_denoise=True branch: only the final squared error is differentiable w.r.t. x_0."""
+        self.model.check_width(x_0, 'x_0')
+        if z is not None:
+            self.model.check_width(z, 'z', x_0.shape[0])
         z = torch.randn_like(x_0) if z is None else z
         mean, std = self.sde.marginal_prob(x_0, vec_t)
         x0_hat, snr = self.multi_step_denoise(mean + std[:, None] * z, vec_t, t_end=vec_t / (2 * n), N=n)
@@ -135,7 +142,7 @@ class DPoserComp(_PriorBase):
         self.data_loss = nn.MSELoss(reduction='mean')
 
     def loss(self, x_0, vec_t, weighted=False, multi_denoise=False, z=None):
-        """mean over B*63 of w (x0 - sg[x0_hat])^2  (run/completion.py:131-149)."""
+        """mean over B*D of w (x0 - sg[x0_hat])^2  (run/completion.py:131-149)."""
         if multi_denoise:
             return self._ddim_loss(x_0, vec_t, weighted, None, 10, z)
         return self._fused_loss(x_0, self._host_t(vec_t), bool(weighted), float(x_0.numel()), z)
@@ -153,6 +160,12 @@ class DPoserComp(_PriorBase):
         with its closed-form gradient, the masked-MSE cotangent, fused Adam (no framework op, no autograd).
         ``z_list`` (parity mode): the Gaussian draw of every step; ``graphs``: capture / replay every step as a CUDA graph."""
         from . import steps as S
+        self.model.check_width(observation, 'observation')
+        if mask.shape[-1] != self.model.pose_width:
+            raise ValueError(f'mask: expected its last dimension to be {self.model.pose_width}, got {list(mask.shape)}')
+        if z_list is not None:
+            for z in z_list:
+                self.model.check_width(z, 'z_list entry', observation.shape[0])
         L.require_cuda(observation, 'observation')
         dev = observation.device
         total_steps = iterations * steps_per_iter
@@ -179,7 +192,8 @@ class DPoserComp(_PriorBase):
         pri.schedule([t for _, _, t in sched])
         g_data = torch.empty_like(x)
         zbuf = torch.empty_like(x) if z_list is not None else None
-        opt = S.Adam(x, 0, 63, lr)
+        D = self.model.pose_width
+        opt = S.Adam(x, 0, D, lr)
         wd = self.get_loss_weights()
         seed = mutils.host_seed() if z_list is None else 0
         sg = S.StepGraphs(graphs and z_list is None)
@@ -195,7 +209,7 @@ class DPoserComp(_PriorBase):
             pri(x, k, bool(quan_t), float(x.numel()), z=z, seed=seed, step=k)
             L.check(lib.dpb_masked_mse_grad(L.ptr(x), L.ptr(obs), L.ptr(msk), L.ptr(g_data), x.numel(),
                                             L.current_stream(dev)))
-            opt.step(g_data, 0, 63, wd['data'](1.0, it), g2=pri.grad, off2=0, ld2=63, s2=wd['dposer'](1.0, it))
+            opt.step(g_data, 0, D, wd['data'](1.0, it), g2=pri.grad, off2=0, ld2=D, s2=wd['dposer'](1.0, it))
 
         for k in range(total_steps):
             sg.run(k, lambda k=k: one_step(k))

@@ -53,6 +53,7 @@ def get_sampling_fn(config, sde, shape, inverse_scaler, eps, device=None, return
 
 def _run_steps(model, x, coef, table, obs, mask, noise, seed, step_offset, traj, x_mean, impute, engine=None):
     """One dpb_sampler_run over the rows of ``coef`` (device fp32 [n,8]) / ``table`` ([n,5,1024])."""
+    model.check_width(x, 'x')
     h = model.handle()
     B = x.shape[0]
     tbl = L.StepTables(coef.shape[0], C.c_void_p(coef.data_ptr()), C.c_void_p(table.data_ptr()))
@@ -75,19 +76,32 @@ def get_pc_sampler(sde, shape, predictor, corrector, inverse_scaler, snr, n_step
     device = torch.device(device)
 
     def pc_sampler(model, observation=None, mask=None, z=None, start_step=0, args=None, noise=None):
-        """``noise`` (optional, parity mode): device tensor [N-start, K, B, 63] of the Gaussian draws in the
+        """``noise`` (optional, parity mode): device tensor [N-start, K, B, D] of the Gaussian draws in the
         reference's order -- K=1 (predictor) or K=3 with completion (after-corrector, predictor, after-predictor)."""
         with torch.no_grad():
+            if len(shape) != 2 or shape[1] != model.pose_width:
+                raise ValueError(f'sampler shape {tuple(shape)} does not match the {model.pose_width}-D score network')
+            task = getattr(args, 'task', None) if args is not None else None
+            impute = task == 'completion'
+            start_t = start_step if task == 'denoise' else 0
+            n_run = sde.N - start_t
+            if z is not None:
+                model.check_width(z, 'z')
+            B = shape[0] if z is None else z.shape[0]
+            if impute:
+                model.check_width(observation, 'observation', B)
+                model.check_width(mask, 'mask', B)
+            if noise is not None:
+                # [n, K, B, D]: K = 1 predictor draw (+2 imputation draws) (+1 Langevin draw first)
+                k = (3 if impute else 1) + (0 if corrector == 'none' else 1)
+                if noise.dim() != 4 or noise.shape[0] < n_run or tuple(noise.shape[1:]) != (k, B, model.pose_width):
+                    raise ValueError(f'noise: expected [>= {n_run}, {k}, {B}, {model.pose_width}], got {list(noise.shape)}')
+                noise = noise.contiguous()
             if device.type != 'cuda':
                 raise RuntimeError('dposer_b200 samplers run on CUDA only (no CPU fallback)')
             x = (sde.prior_sampling(shape) if z is None else z).to(device=device, dtype=torch.float32).contiguous()
             if z is not None:
                 x = x.clone()
-            B = x.shape[0]
-            task = getattr(args, 'task', None) if args is not None else None
-            impute = task == 'completion'
-            start_t = start_step if task == 'denoise' else 0
-            n_run = sde.N - start_t
             timesteps = mutils.timestep_grid(sde, eps)
             if predictor == 'none':
                 raise NotImplementedError("predictor 'none' (corrector-only sampling) is not supported")
@@ -152,6 +166,9 @@ def get_ode_sampler(sde, shape, inverse_scaler, denoise=False, rtol=1e-5, atol=1
         return sde.reverse(score_fn, probability_flow=True).sde(x, t)[0]
 
     def ode_sampler(model, z=None):
+        if method == 'RK45' and device.type == 'cuda' and getattr(model, 'is_rot6d', False):
+            raise NotImplementedError('the device RK45 probability-flow ODE is built for the 63-D axis network, not for '
+                                      'rot6d (126-D) score networks')
         with torch.no_grad():
             x = (sde.prior_sampling(shape) if z is None else z).to(device)
             if method == 'RK45' and device.type == 'cuda':

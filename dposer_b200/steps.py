@@ -50,7 +50,7 @@ class PriorStep:
     def __init__(self, model, sde, continuous, rows, device):
         self.model, self.sde, self.continuous = model, sde, continuous
         self.loss = torch.empty(1, dtype=torch.float32, device=device)
-        self.grad = torch.empty(rows, 63, dtype=torch.float32, device=device)
+        self.grad = torch.empty(rows, model.pose_width, dtype=torch.float32, device=device)
         self.ws = model.workspace(rows, device)
         self.tables, self.scalars = None, None
 

@@ -34,13 +34,14 @@ def default_config():
     )
 
 
-def make_score_model(seed=42, config=None):
+def make_score_model(seed=42, config=None, pose_dim=3):
     """SURVEY 8(d) "Score weights": default init under torch.manual_seed(seed) in the reference's module
-    order, then every GroupNorm weight~U(0.5,1.5), bias~N(0,0.1^2) (same generator, module order)."""
+    order, then every GroupNorm weight~U(0.5,1.5), bias~N(0,0.1^2) (same generator, module order).
+    pose_dim=3: the 63-D axis-angle network; pose_dim=6: the 126-D rot6d one."""
     from .model import ScoreModelFC
     config = config or default_config()
     torch.manual_seed(seed)
-    m = ScoreModelFC(config, n_poses=21, pose_dim=3, hidden_dim=1024, embed_dim=512, n_blocks=2)
+    m = ScoreModelFC(config, n_poses=21, pose_dim=pose_dim, hidden_dim=1024, embed_dim=512, n_blocks=2)
     for mod in m.modules():
         if isinstance(mod, torch.nn.GroupNorm):
             with torch.no_grad():

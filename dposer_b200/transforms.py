@@ -6,8 +6,9 @@ reference builds them on third-party ``torchgeometry`` (``angle_axis_to_rotation
 properties (round trips, orthonormality, agreement with the LBS oracle's Rodrigues) and against a restatement of
 torchgeometry's published algorithms (oracle/tgm_ref.py); the Gram-Schmidt leg is pinned bit-exactly to the reference.
 ``misc.Posenormalizer(rot_rep='rot6d')`` and ``misc.create_mask(observation_type='mean')`` call them at the data boundary;
-the hot-path kernels take the shipped ``rot_rep='axis'`` (63-D) configuration only (a 126-D score net would need its own
-first / last layer geometry)."""
+the score-net kernels take both representations (63-D axis, 126-D rot6d score networks: ``ScoreModelFC(config, 21, 6)``).
+The native SMPLify / motion-denoising chains (``fitting.py``) run the axis prior only: a rot6d prior there would need this
+conversion and its Jacobian as a kernel inside the step."""
 import torch
 import torch.nn.functional as F
 

@@ -39,8 +39,10 @@ extern "C" {
 #define DPB_ENOMEM (-3)       /* workspace too small or allocation failure */
 #define DPB_EUNSUPPORTED (-4) /* feature not available (maps to NotImplementedError) */
 
-/* network geometry (configs/subvp/amass_scorefc_continuous.py:36-45 + defaults) */
+/* network geometry (configs/subvp/amass_scorefc_continuous.py:36-45 + defaults).  DPB_POSE_DIM is the axis-angle
+ * width; a score handle may instead be created for the rot6d width DPB_POSE_DIM_ROT6D (dpb_score_create_dim). */
 #define DPB_POSE_DIM 63
+#define DPB_POSE_DIM_ROT6D 126
 #define DPB_HIDDEN 1024
 #define DPB_EMBED 512
 #define DPB_NUM_DENSE 5 /* pre_dense, b1_dense1, b1_dense2, b2_dense1, b2_dense2 */
@@ -66,7 +68,7 @@ int dpb_device_info(int device, int* sm_count, int* cc_major, int* cc_minor);
  * ---------------------------------------------------------------------------------------- */
 typedef struct {
   /* all HOST fp32 pointers, nn.Linear layout [out, in] row-major; state_dict key in comments */
-  const float* pre_w;        /* pre_dense.weight        [1024, 63]   */
+  const float* pre_w;        /* pre_dense.weight        [1024, D]  (D = the handle's pose width, 63 or 126) */
   const float* pre_b;        /* pre_dense.bias          [1024]       */
   const float* pre_t_w;      /* pre_dense_t.weight      [1024, 512]  */
   const float* pre_t_b;      /* pre_dense_t.bias        [1024]       */
@@ -80,12 +82,19 @@ typedef struct {
   const float* blk_t_b[4];   /* ... .bias [1024] */
   const float* blk_gn_w[4];  /* b{1,2}_gnorm{1,2}.weight [1024] */
   const float* blk_gn_b[4];  /* ... .bias [1024] */
-  const float* post_w;       /* post_dense.weight [63,1024] */
-  const float* post_b;       /* post_dense.bias   [63] */
+  const float* post_w;       /* post_dense.weight [D,1024] */
+  const float* post_b;       /* post_dense.bias   [D] */
   const float* emb_freqs;    /* [256] exp(-k ln(1e4)/255) evaluated by the host in fp32 (model.py:41-43) */
 } dpb_score_weights;
 
+/* a 63-D (axis-angle, ScoreModelFC(config, 21, 3)) network */
 int dpb_score_create(dpb_score_t** h, const dpb_score_weights* w, int device);
+/* pose_dim = 63 (axis-angle) or 126 (rot6d, ScoreModelFC(config, 21, 6)); any other value: DPB_EUNSUPPORTED.
+ * Every entry point that takes the handle reads D = pose_dim from it; "[B,D]" below means that width.
+ * Not built for D = 126: dpb_score_jvp (DPB_EUNSUPPORTED). */
+int dpb_score_create_dim(dpb_score_t** h, const dpb_score_weights* w, int pose_dim, int device);
+/* D of the handle (63 or 126), or DPB_EINVAL for a null handle */
+int dpb_score_pose_dim(dpb_score_t* h);
 int dpb_score_destroy(dpb_score_t* h);
 
 /* Time path, hoisted (model.py:161-167,174,181 with utils.py:152): for each of n labels
@@ -95,8 +104,8 @@ int dpb_score_time_table(dpb_score_t* h, const float* labels, int n, float* tabl
 
 size_t dpb_score_workspace_bytes(dpb_score_t* h, int64_t B, int flags);
 
-/* out[B,63] = post_dense(...)(x) * scale.
- *   x         DEVICE fp32 [B,63]
+/* out[B,D] = post_dense(...)(x) * scale.
+ *   x         DEVICE fp32 [B,D]
  *   table     DEVICE fp32 [n,5,1024] from dpb_score_time_table
  *   t_index   DEVICE int32 [B] row -> table entry, or NULL (every row uses entry 0)
  *   row_scale DEVICE fp32 [B] or NULL (then `scale` is used for every row).  The caller folds
@@ -106,8 +115,8 @@ int dpb_score_forward(dpb_score_t* h, const float* x, const float* table, const 
                       const float* row_scale, float scale, float* out, int64_t B, int flags,
                       void* ws, size_t ws_bytes, void* stream);
 
-/* Forward-mode derivative of dpb_score_forward (fp32 engine): out [B,63] as dpb_score_forward, jv [B,63] =
- * (d out / d x) v for a direction v [B,63], with the same row_scale / scale applied to both.  Replaces the autograd
+/* Forward-mode derivative of dpb_score_forward (fp32 engine), 63-D handles only: out [B,63] as dpb_score_forward,
+ * jv [B,63] = (d out / d x) v for a direction v [B,63], with the same row_scale / scale applied to both.  Replaces the autograd
  * call of the Hutchinson-Skilling trace estimator in lib/algorithms/advanced/likelihood.py:26-37: the scalar
  * eps . (J eps) it needs is what the reference computes as eps . (J^T eps).  ws: dpb_score_jvp_workspace_bytes. */
 size_t dpb_score_jvp_workspace_bytes(dpb_score_t* h, int64_t B);
@@ -132,13 +141,13 @@ typedef struct {
 #define DPB_SAMPLER_IMPUTE (1 << 4)      /* args.task == 'completion' */
 #define DPB_SAMPLER_NOISE_GIVEN (1 << 5) /* consume caller-supplied Gaussian draws (parity mode) */
 
-/*   x_io      DEVICE fp32 [B,63] in: x_T (or z), out: x after the last step
- *   obs,mask  DEVICE fp32 [B,63] (only with DPB_SAMPLER_IMPUTE)
- *   noise     DEVICE fp32: with NOISE_GIVEN, [n_steps, K, B, 63] where K=1 (predictor draw) or
+/*   x_io      DEVICE fp32 [B,D] in: x_T (or z), out: x after the last step
+ *   obs,mask  DEVICE fp32 [B,D] (only with DPB_SAMPLER_IMPUTE)
+ *   noise     DEVICE fp32: with NOISE_GIVEN, [n_steps, K, B, D] where K=1 (predictor draw) or
  *             K=3 with IMPUTE (draw after corrector, predictor draw, draw after predictor --
  *             the reference's order, sampling.py:459-460).  Otherwise NULL: Philox4x32-10
- *             keyed by (seed, row, step+step_offset, column).
- *   traj      DEVICE fp32 [n_steps,B,63] or NULL;  x_mean DEVICE fp32 [B,63] or NULL.
+ *             keyed by (seed, row, step+step_offset, column); see dpb_normal_fill_dim for the layout.
+ *   traj      DEVICE fp32 [n_steps,B,D] or NULL;  x_mean DEVICE fp32 [B,D] or NULL.
  */
 int dpb_sampler_run(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, const float* obs,
                     const float* mask, const float* noise, uint64_t seed, uint64_t step_offset,
@@ -152,10 +161,14 @@ int dpb_sampler_run(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, con
 int dpb_langevin_norms(const float* grad, const float* noise, float* sums, int64_t B, void* stream);
 int dpb_langevin_update(float* x_io, float* x_mean, const float* grad, const float* noise,
                         const float* sums, float snr, float alpha, int64_t B, void* stream);
+/* the same on rows of pose_dim (63 or 126) columns; the two above mean pose_dim = 63 */
+int dpb_langevin_norms_dim(const float* grad, const float* noise, float* sums, int64_t B, int pose_dim, void* stream);
+int dpb_langevin_update_dim(float* x_io, float* x_mean, const float* grad, const float* noise, const float* sums,
+                            float snr, float alpha, int64_t B, int pose_dim, void* stream);
 /* Predictor-corrector sampling with the Langevin corrector, all n_steps from ONE call (replaces the loop body
  * sampling.py:456-461 with LangevinCorrector.update_fn :282-302 and the predictor of dpb_sampler_run):
  *   score_scale HOST [n]: -1 / (sigma * std) of each step (score = raw * score_scale); lang_alpha HOST [n]: the alpha of
- *   sampling.py:287-291; noise (DPB_SAMPLER_NOISE_GIVEN): DEVICE [n, K+1, B, 63], the Langevin draw first, then the K
+ *   sampling.py:287-291; noise (DPB_SAMPLER_NOISE_GIVEN): DEVICE [n, K+1, B, D], the Langevin draw first, then the K
  *   planes of dpb_sampler_run; otherwise Philox slot 4 serves the corrector.  Batch norms are over the B rows given.
  *   With the tcgen05 engine and at most one 128-row tile per SM (B <= 18 944) all steps run in ONE persistent kernel;
  *   columns 5 and 6 of tbl->coef (DEVICE, spare) are then overwritten with score_scale / lang_alpha. */
@@ -164,8 +177,13 @@ int dpb_sampler_run_pc(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, 
                        const float* lang_alpha, float snr, const float* obs, const float* mask, const float* noise,
                        uint64_t seed, uint64_t step_offset, float* traj, float* x_mean, int64_t B, int flags, void* ws,
                        size_t ws_bytes, void* stream);
-/* fills out[n] with N(0,1) draws of the library's Philox stream (row-major [B,63] addressing) */
+/* fills out [B, pose_dim] with N(0,1) draws of the library's Philox stream.  Draw (row, column c) of (step, slot) is
+ * Box-Muller output c % 4 of the Philox4x32-10 block with key = seed and counter = (row lo, row hi, step,
+ * slot * DP/4 + c/4), DP = 64 for pose_dim 63 and 128 for 126: every (slot, column) of a row has its own counter.
+ * Slots: 0 imputation before the score, 1 predictor, 2 imputation after the predictor, 3 prior-loss z, 4 Langevin.
+ * dpb_normal_fill means pose_dim = 63. */
 int dpb_normal_fill(float* out, int64_t B, uint64_t seed, uint64_t step, int slot, void* stream);
+int dpb_normal_fill_dim(float* out, int64_t B, uint64_t seed, uint64_t step, int slot, int pose_dim, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * DPoser prior loss  (replaces DPoserComp.loss run/completion.py:131-149,
@@ -175,8 +193,9 @@ int dpb_normal_fill(float* out, int64_t B, uint64_t seed, uint64_t step, int slo
  * loss = sum_all( w (x0-x0_hat)^2 ) / divisor, w = 0.5 or 0.5*sqrt(1+alpha/std) ;
  * grad = 2 w (x0-x0_hat)/divisor  (x0_hat is detached in the reference).
  *   table      DEVICE fp32 [1,5,1024] time table of this t
- *   z          DEVICE fp32 [B,63] Gaussian draw or NULL (Philox with seed/step)
- *   loss_out   DEVICE fp32 [1] (overwritten), grad_out DEVICE fp32 [B,63] or NULL
+ *   x0         DEVICE fp32 [B,D]
+ *   z          DEVICE fp32 [B,D] Gaussian draw or NULL (Philox with seed/step)
+ *   loss_out   DEVICE fp32 [1] (overwritten), grad_out DEVICE fp32 [B,D] or NULL
  *   row_loss   DEVICE fp32 [B] or NULL: per-row sums of w (x0-x0_hat)^2 (for per-problem normalisation)
  */
 int dpb_prior_loss(dpb_score_t* h, const float* x0, const float* table, float alpha, float std,
