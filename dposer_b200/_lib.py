@@ -51,7 +51,8 @@ EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create
            'dpb_motion_loss', 'dpb_camera_fit_loss', 'dpb_adam_step', 'dpb_affine_cols', 'dpb_joint_map_gather',
            'dpb_joint_map_scatter', 'dpb_masked_mse_grad', 'dpb_seq_smooth3', 'dpb_train_create', 'dpb_train_destroy',
            'dpb_train_loss_grad', 'dpb_train_adam_scratch_bytes', 'dpb_train_grad_norm', 'dpb_train_adam', 'dpb_ema_update', 'dpb_train_set_seed_pointer', 'dpb_gemm_nt_workspace_bytes', 'dpb_gemm_nt', 'dpb_train_forward', 'dpb_train_backward', 'dpb_rows_axpby', 'dpb_weighted_sqdiff', 'dpb_rk45_stage', 'dpb_rk45_scratch_bytes', 'dpb_rk45_error',
-           'dpb_pf_ode_rhs']
+           'dpb_pf_ode_rhs', 'dpb_selfisect_create', 'dpb_selfisect_destroy', 'dpb_selfisect_workspace_bytes',
+           'dpb_selfisect_run']
 
 _lib = None
 
@@ -146,12 +147,18 @@ def load():
     lib.dpb_rk45_error.argtypes = [vp, vp, vp, i64, f64, f64, f64, vp, vp]
     lib.dpb_pf_ode_rhs.argtypes = [vp, vp, vp, vp, f32, f32, vp, i64, vp]
     lib.dpb_mean_point_error.argtypes = [vp, vp, i64, C.c_int, vp, C.c_int, vp, vp]
+    lib.dpb_selfisect_create.argtypes = [C.POINTER(vp), _i32p, C.c_int, C.c_int, C.c_int]
+    lib.dpb_selfisect_destroy.argtypes = [vp]
+    lib.dpb_selfisect_workspace_bytes.argtypes = [vp, i64]
+    lib.dpb_selfisect_workspace_bytes.restype = sz
+    lib.dpb_selfisect_run.argtypes = [vp, vp, i64, vp, vp, vp, sz, vp]
     for name in EXPORTS:
         fn = getattr(lib, name)
         if name not in ('dpb_last_error', 'dpb_score_workspace_bytes', 'dpb_lbs_workspace_bytes',
                         'dpb_lbs_backward_scratch_bytes', 'dpb_lbs_backward_scratch_bytes_joints',
                         'dpb_score_jvp_workspace_bytes', 'dpb_sampler_pc_workspace_bytes',
-                        'dpb_train_adam_scratch_bytes', 'dpb_gemm_nt_workspace_bytes', 'dpb_rk45_scratch_bytes'):
+                        'dpb_train_adam_scratch_bytes', 'dpb_gemm_nt_workspace_bytes', 'dpb_rk45_scratch_bytes',
+                        'dpb_selfisect_workspace_bytes'):
             fn.restype = C.c_int
     _lib = lib
     return lib

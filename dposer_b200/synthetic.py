@@ -124,6 +124,59 @@ def full_pose_from(inputs, model_type='smpl'):
     return pose, torch.cat([inputs['betas'], torch.zeros(B, 10)], dim=1)
 
 
+def uv_sphere(n_rings=82, n_lon=84, radius=1.0, center=(0., 0., 0.)):
+    """Closed UV sphere: two poles and n_rings rings of n_lon vertices, faces wound outward.  The defaults give
+    SMPL's counts (V = 6890, F = 13776); (101, 104) gives V = 10506, F = 21008 (more faces than SMPL-X's 20908).
+    Returns fp32 vertices [V,3] and int32 faces [2 n_lon n_rings, 3] as numpy arrays."""
+    th = np.pi * np.arange(1, n_rings + 1) / (n_rings + 1)
+    ph = 2 * np.pi * np.arange(n_lon) / n_lon
+    ring = np.stack([np.sin(th)[:, None] * np.cos(ph), np.sin(th)[:, None] * np.sin(ph),
+                     np.repeat(np.cos(th)[:, None], n_lon, 1)], -1).reshape(-1, 3)
+    v = np.concatenate([[[0., 0., 1.]], ring, [[0., 0., -1.]]]) * radius + np.asarray(center)
+    r = lambda i, j: 1 + i * n_lon + (j % n_lon)                           # noqa: E731  ring i (0-based), longitude j
+    j = np.arange(n_lon)
+    south = 1 + n_rings * n_lon
+    faces = [np.stack([np.zeros(n_lon, int), r(0, j), r(0, j + 1)], 1)]
+    for i in range(n_rings - 1):
+        a, b, c, d = r(i, j), r(i + 1, j), r(i + 1, j + 1), r(i, j + 1)
+        faces += [np.stack([a, b, c], 1), np.stack([a, c, d], 1)]
+    faces.append(np.stack([np.full(n_lon, south), r(n_rings - 1, j + 1), r(n_rings - 1, j)], 1))
+    return v.astype(np.float32), np.concatenate(faces).astype(np.int32)
+
+
+def dented_sphere(depth, seed, n_rings=82, n_lon=84, cap_deg=(65., 80.), jitter=0.01):
+    """A UV sphere with a seeded cap pushed inward: cap height h (along a random axis u) becomes h (1 - 2 depth w),
+    w = 1 inside cap_deg[0] and a smoothstep to 0 at cap_deg[1].  depth = 0: the sphere; depth = 0.5 flattens the
+    cap onto the equatorial plane; depth = 1 mirrors it onto the opposite wall, where the two sheets interpenetrate
+    wherever the jitter crosses (the most self-intersection); depth > 1 pushes it through the wall.  Before the dent
+    every vertex moves radially by a smooth seeded field of amplitude `jitter` (a few low-frequency waves), so that
+    no pair of faces is exactly degenerate.  Returns fp32 vertices [V,3] (the faces are uv_sphere's)."""
+    v, _ = uv_sphere(n_rings, n_lon)
+    g = np.random.default_rng(seed)
+    p = v.astype(np.float64)
+    rad = np.zeros(len(p))
+    for _ in range(4):
+        k = g.normal(size=3)
+        k *= g.uniform(10., 24.) / np.linalg.norm(k)
+        rad += g.uniform(0.5, 1.) * np.sin(p @ k + g.uniform(0, 2 * np.pi))
+    p *= (1 + jitter * rad / 4)[:, None]
+    u = g.normal(size=3)
+    u /= np.linalg.norm(u)
+    h = p @ u
+    c_in, c_out = np.cos(np.radians(cap_deg[0])), np.cos(np.radians(cap_deg[1]))
+    t = np.clip((h / np.linalg.norm(p, axis=1) - c_out) / (c_in - c_out), 0, 1)
+    w = t * t * (3 - 2 * t)
+    p -= (2 * depth * w * h)[:, None] * u
+    return p.astype(np.float32)
+
+
+def two_spheres(n_rings=40, n_lon=48, offset=1.0):
+    """Two overlapping unit UV spheres (centres `offset` apart along x) as one two-component mesh."""
+    v0, f0 = uv_sphere(n_rings, n_lon, center=(0., 0., 0.))
+    v1, f1 = uv_sphere(n_rings, n_lon, center=(offset, 0.01, 0.02))
+    return np.concatenate([v0, v1]), np.concatenate([f0, f1 + len(v0)]).astype(np.int32)
+
+
 def completion_inputs(n_partial=4096, hypotheses=10, seed=21, normalizer=None):
     """c3 inputs: normalised toy poses tiled (+N(0,0.05^2)), legs masked, x hypotheses."""
     from .misc import create_mask, Posenormalizer

@@ -427,6 +427,25 @@ int dpb_apd_partial(const float* joints, int64_t B, int n_joints, int64_t row0, 
 int dpb_mean_point_error(const float* a, const float* c, int64_t B, int n_points, const int32_t* idx,
                          int n_idx, float* out, void* stream);
 
+/* Self-intersection metric (replaces self_intersections_percentage lib/utils/metric.py:41-89, pymeshlab on the CPU).
+ * A pair of distinct faces intersects according to s, the number of vertex ids they share: s = 0 the closed triangles
+ * have a common point; s = 1 the edge opposite the shared vertex, moved halfway to it, crosses the other face's open
+ * interior (either way round); s = 2 never; s = 3 always; a zero-area face never.  A face is selected when it is in an
+ * intersecting pair; SI = 100 * selected / n_faces.  Every decision is the sign of an fp64 expression of the fp32
+ * inputs (the full rule: dposer_b200/metric.py).  Deterministic; no host synchronisation (graph-capturable).
+ *   create: faces HOST int32 [n_faces,3], every id in [0, n_vertices) (DPB_EINVAL otherwise), uploaded once;
+ *           n_faces > 32768: DPB_EUNSUPPORTED.  One handle serves any number of meshes of that topology.
+ *   run:    vertices DEVICE fp32 [B, n_vertices, 3] (e.g. dpb_lbs_forward's verts);
+ *           counts DEVICE int32 [B]: selected faces of each mesh, -1 when a face references a non-finite vertex;
+ *           selection DEVICE uint8 [B, n_faces] (1 = selected, all 0 for a non-finite mesh) or NULL;
+ *           ws DEVICE, dpb_selfisect_workspace_bytes(h, B) bytes, any contents. */
+typedef struct dpb_selfisect dpb_selfisect_t;
+int dpb_selfisect_create(dpb_selfisect_t** h, const int32_t* faces, int n_faces, int n_vertices, int device);
+int dpb_selfisect_destroy(dpb_selfisect_t* h);
+size_t dpb_selfisect_workspace_bytes(dpb_selfisect_t* h, int64_t B);
+int dpb_selfisect_run(dpb_selfisect_t* h, const float* vertices, int64_t B, int32_t* counts, uint8_t* selection,
+                      void* ws, size_t ws_bytes, void* stream);
+
 #ifdef __cplusplus
 }
 #endif
