@@ -52,7 +52,7 @@ EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create
            'dpb_joint_map_scatter', 'dpb_masked_mse_grad', 'dpb_seq_smooth3', 'dpb_train_create', 'dpb_train_destroy',
            'dpb_train_loss_grad', 'dpb_train_adam_scratch_bytes', 'dpb_train_grad_norm', 'dpb_train_adam', 'dpb_ema_update', 'dpb_train_set_seed_pointer', 'dpb_gemm_nt_workspace_bytes', 'dpb_gemm_nt', 'dpb_train_forward', 'dpb_train_backward', 'dpb_rows_axpby', 'dpb_weighted_sqdiff', 'dpb_rk45_stage', 'dpb_rk45_scratch_bytes', 'dpb_rk45_error',
            'dpb_pf_ode_rhs', 'dpb_selfisect_create', 'dpb_selfisect_destroy', 'dpb_selfisect_workspace_bytes',
-           'dpb_selfisect_run']
+           'dpb_selfisect_run', 'dpb_procrustes']
 
 _lib = None
 
@@ -152,6 +152,7 @@ def load():
     lib.dpb_selfisect_workspace_bytes.argtypes = [vp, i64]
     lib.dpb_selfisect_workspace_bytes.restype = sz
     lib.dpb_selfisect_run.argtypes = [vp, vp, i64, vp, vp, vp, sz, vp]
+    lib.dpb_procrustes.argtypes = [vp, vp, i64, C.c_int, vp, C.c_int, vp, vp, vp, vp]
     for name in EXPORTS:
         fn = getattr(lib, name)
         if name not in ('dpb_last_error', 'dpb_score_workspace_bytes', 'dpb_lbs_workspace_bytes',

@@ -7,7 +7,7 @@ PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, 'csrc')
 LIBDIR = os.path.join(PKG, 'lib')
 LIB = os.path.join(LIBDIR, 'libdposer_b200.so')
-SOURCES = ['api.cu', 'score_simt.cu', 'score_tc.cu', 'score_small.cu', 'sampler.cu', 'lbs.cu', 'lbs_bwd.cu', 'lbs_bwd_tc.cu', 'lbs_skin_bwd_tc.cu', 'lbs_tc.cu', 'lbs_fused2.cu', 'lbs_fused3.cu', 'metrics.cu', 'fit.cu', 'fitstep.cu', 'gemm_tc.cu', 'train.cu', 'rk45.cu', 'selfisect.cu']
+SOURCES = ['api.cu', 'score_simt.cu', 'score_tc.cu', 'score_small.cu', 'sampler.cu', 'lbs.cu', 'lbs_bwd.cu', 'lbs_bwd_tc.cu', 'lbs_skin_bwd_tc.cu', 'lbs_tc.cu', 'lbs_fused2.cu', 'lbs_fused3.cu', 'metrics.cu', 'fit.cu', 'fitstep.cu', 'gemm_tc.cu', 'train.cu', 'rk45.cu', 'selfisect.cu', 'procrustes.cu']
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17',
               '-Xcompiler', '-fPIC', '--expt-relaxed-constexpr']
 

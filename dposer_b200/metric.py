@@ -35,6 +35,33 @@ edge's end points relative to the plane, n . (x - q0), then either the three sig
 (q_i+1 - a)) all >= 0 or all <= 0, or, for an edge in the plane, in-plane orientations n . ((q - p) x (r - p)) and
 on-segment dot products; s = 1 uses the same volumes, strictly.  Both implementations also require the closed fp32
 AABBs of the two faces to overlap, an exact test that no intersecting pair fails.
+
+Procrustes-aligned point error PA-MPJPE / PA-MPVPE (``compute_similarity_transform``, ``reconstruction_error``)
+------------------------------------------------------------------------------------------------------------
+The reference computes it in lib/utils/transforms.py with numpy, one sample at a time; that file is not part of the
+checkout this was built from, so parity is unpinned and the rule is this project's: the similarity Procrustes with the
+reflection correction, as in HMR / SPIN's ``compute_similarity_transform``.  For one sample with predicted points
+``S1 [n,3]`` and target points ``S2 [n,3]`` (fp32 inputs, evaluated in float64)::
+
+    mu1, mu2 = mean(S1), mean(S2);  X1 = S1 - mu1;  X2 = S2 - mu2
+    var1 = sum(X1**2);  K = X1^T X2                      # 3x3
+    U, s, Vh = svd(K);  V = Vh^T
+    Z = diag(1, 1, sign(det(U V^T)))                     # det is +-1, never 0
+    R = V Z U^T;  scale = trace(R K) / var1;  t = mu2 - scale R mu1
+    S1_hat = scale S1 R^T + t                            # row-vector form
+    err = mean_k ||S1_hat[k] - S2[k]||                   # in the input's units (metres)
+
+- **Subset.** An optional point subset ``idx`` selects the points that both fit the transform and are measured;
+  ``S1_hat`` applies that transform to all ``n`` points.
+- **NaN rows.** A row whose selected points hold a non-finite coordinate gets NaN for ``err``, its parameters and its
+  aligned points; so does a row with ``var1 == 0`` (all selected predicted points coincide, or one point).  A
+  non-finite coordinate outside the subset only makes its own aligned point non-finite.  Other rows are unaffected.
+- **Uniqueness.** ``R`` is unique when the smallest singular value of ``K`` is simple (coplanar point sets included).
+  For collinear sets ``R`` is not unique, but ``S1_hat`` and ``err`` are.
+
+The kernel (``csrc/procrustes.cu``) accumulates the moments in fp64 after shifting each row by its first selected
+point, and finds ``R`` as the top eigenvector of Horn's 4x4 quaternion matrix of ``K``: the proper rotation maximising
+``trace(R K)``, which is ``V Z U^T`` above.  ``oracle/procrustes_ref.py`` restates the rule with an SVD.
 """
 import hashlib
 
@@ -81,11 +108,14 @@ def mean_point_error_mm(a, b, idx=None):
 
 
 class Evaler:
-    """lib/dataset/AMASS.py:263-324 -- MPVPE / MPJPE per sample (mm), min over hypotheses."""
+    """lib/dataset/AMASS.py:263-324 -- MPVPE / MPJPE per sample (mm), min over hypotheses.  With
+    ``procrustes=True`` the results also hold ``pa_mpvpe_all`` and ``pa_mpjpe_body``: the same errors after similarity
+    alignment (``reconstruction_error``) over the same point subsets, in mm."""
 
-    def __init__(self, body_model, part=None, vert_idx=None):
+    def __init__(self, body_model, part=None, vert_idx=None, procrustes=False):
         self.body_model = body_model
         self.part = part
+        self.procrustes = procrustes
         if part is not None:
             self.joint_idx = np.array(getattr(BodyPartIndices, part)) + 1     # skip pelvis
             self.vert_idx = None if vert_idx is None else np.asarray(vert_idx)
@@ -95,12 +125,17 @@ class Evaler:
     def eval_bodys(self, outs, gts):
         body_gt = self.body_model(pose_body=gts)
         body_out = self.body_model(pose_body=outs)
-        return {'mpvpe_all': mean_point_error_mm(body_out.v, body_gt.v, self.vert_idx).cpu().numpy(),
-                'mpjpe_body': mean_point_error_mm(body_out.Jtr, body_gt.Jtr, self.joint_idx).cpu().numpy()}
+        res = {'mpvpe_all': mean_point_error_mm(body_out.v, body_gt.v, self.vert_idx).cpu().numpy(),
+               'mpjpe_body': mean_point_error_mm(body_out.Jtr, body_gt.Jtr, self.joint_idx).cpu().numpy()}
+        if self.procrustes:
+            res['pa_mpvpe_all'] = (reconstruction_error(body_out.v, body_gt.v, None, self.vert_idx) * 1000).cpu().numpy()
+            res['pa_mpjpe_body'] = (reconstruction_error(body_out.Jtr, body_gt.Jtr, None, self.joint_idx) * 1000) \
+                .cpu().numpy()
+        return res
 
     def multi_eval_bodys(self, outs, gts):
         res = [self.eval_bodys(outs[:, h], gts) for h in range(outs.shape[1])]
-        return {k: np.min([r[k] for r in res], axis=0) for k in ('mpvpe_all', 'mpjpe_body')}
+        return {k: np.min([r[k] for r in res], axis=0) for k in res[0]}
 
 
 class MeshTopology:
@@ -194,3 +229,73 @@ def self_intersections_percentage(vertices, faces, return_selection=False):
         pct = pct[0]
         sel = None if sel is None else sel[0]
     return (pct, sel.bool()) if return_selection else pct
+
+
+def _procrustes(S1, S2, idx, want_aligned, want_params):
+    """Checks (ValueError before any library call; RuntimeError for CPU tensors), then one dpb_procrustes launch.
+    Returns (single, err [B], aligned [B,n,3] or None, params [B,13] or None), fp32 on the inputs' device."""
+    for name, x in (('S1', S1), ('S2', S2)):
+        if not isinstance(x, torch.Tensor) or x.dim() not in (2, 3) or x.shape[-1] != 3 or x.shape[-2] == 0 or \
+                (x.dim() == 3 and x.shape[0] == 0):
+            raise ValueError(f'{name} must be a tensor of shape [B,n,3] or [n,3], got {getattr(x, "shape", None)}')
+        if not x.is_floating_point():
+            raise ValueError(f'{name} must be floating point, got {x.dtype}')
+    if S1.shape != S2.shape:
+        raise ValueError(f'S1 and S2 must have the same shape, got {tuple(S1.shape)} and {tuple(S2.shape)}')
+    n = S1.shape[-2]
+    ix = None
+    if idx is not None:
+        ix = np.asarray(idx.detach().cpu().numpy() if isinstance(idx, torch.Tensor) else idx)
+        if ix.ndim != 1 or ix.size == 0 or not np.issubdtype(ix.dtype, np.integer):
+            raise ValueError(f'idx must be a non-empty 1-D integer sequence, got {ix.dtype} {ix.shape}')
+        if ix.min() < 0 or ix.max() >= n:
+            raise ValueError(f'idx entries must lie in [0, {n}), got [{ix.min()}, {ix.max()}]')
+    L.require_cuda(S1, 'S1')
+    L.require_cuda(S2, 'S2')
+    if S1.device != S2.device:
+        raise ValueError(f'S1 and S2 must be on the same device, got {S1.device} and {S2.device}')
+    single = S1.dim() == 2
+    a = (S1.detach()[None] if single else S1.detach()).to(torch.float32).contiguous()
+    b = (S2.detach()[None] if single else S2.detach()).to(torch.float32).contiguous()
+    B = a.shape[0]
+    if ix is not None:
+        ix = torch.as_tensor(ix.astype(np.int32), device=a.device)
+    err = torch.empty(B, dtype=torch.float32, device=a.device)
+    aligned = torch.empty_like(a) if want_aligned else None
+    params = torch.empty(B, 13, dtype=torch.float32, device=a.device) if want_params else None
+    L.check(L.load().dpb_procrustes(L.ptr(a), L.ptr(b), B, n, L.ptr(ix), 0 if ix is None else ix.numel(), L.ptr(err),
+                                    L.ptr(aligned), L.ptr(params), L.current_stream(a.device)))
+    return single, err, aligned, params
+
+
+def compute_similarity_transform(S1, S2, idx=None, return_params=False):
+    """S1_hat: ``S1`` aligned to ``S2`` by the similarity transform of this module's docstring (reference
+    lib/utils/transforms.py).  S1, S2: [B,n,3] or a single [n,3] pair, floating point, on CUDA (fp32 is used as is);
+    ``idx``: optional host sequence of point ids that fit the transform (every point is still transformed).
+    Returns fp32 S1_hat of S1's shape, and with ``return_params=True`` also ``(scale [B], R [B,3,3], t [B,3])``
+    (without the batch dimension for a single pair).  NaN rows as in the docstring.  No host synchronisation unless
+    ``idx`` is given (it is uploaded); there is no CPU fallback."""
+    single, _, aligned, params = _procrustes(S1, S2, idx, True, return_params)
+    if single:
+        aligned = aligned[0]
+    if not return_params:
+        return aligned
+    scale, R, t = params[:, 0], params[:, 1:10].reshape(-1, 3, 3), params[:, 10:]
+    if single:
+        scale, R, t = scale[0], R[0], t[0]
+    return aligned, (scale, R, t)
+
+
+def reconstruction_error(S1, S2, reduction='mean', idx=None):
+    """PA-MPJPE / PA-MPVPE: the mean distance after similarity alignment, in the input's units (reference
+    lib/utils/transforms.py).  Per row over the selected points ``idx`` (all when None); ``reduction`` 'mean' or 'sum'
+    over rows gives a 0-d tensor, None the fp32 per-row errors [B] (0-d for a single [n,3] pair).  The row reduction
+    runs on the device in fp64; with ``idx=None`` the call never synchronises with the host."""
+    if reduction not in ('mean', 'sum', None):
+        raise ValueError(f"reduction must be 'mean', 'sum' or None, got {reduction!r}")
+    single, err, _, _ = _procrustes(S1, S2, idx, False, False)
+    if reduction == 'mean':
+        return err.double().mean().float()
+    if reduction == 'sum':
+        return err.double().sum().float()
+    return err[0] if single else err

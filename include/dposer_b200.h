@@ -427,6 +427,20 @@ int dpb_apd_partial(const float* joints, int64_t B, int n_joints, int64_t row0, 
 int dpb_mean_point_error(const float* a, const float* c, int64_t B, int n_points, const int32_t* idx,
                          int n_idx, float* out, void* stream);
 
+/* Procrustes-aligned point error, PA-MPJPE / PA-MPVPE (replaces compute_similarity_transform / reconstruction_error
+ * of lib/utils/transforms.py, numpy on the CPU, one sample at a time).  Per row: the similarity transform (scale s,
+ * proper rotation R, translation t) minimising sum_k ||s R s1[k] + t - s2[k]||^2 over the points idx selects (all
+ * when idx is NULL), fitted in fp64, and err = mean over those points of ||s R s1[k] + t - s2[k]|| (the full rule:
+ * dposer_b200/metric.py).  Deterministic; no host synchronisation (graph-capturable).
+ *   s1, s2   DEVICE fp32 [B, n_points, 3] (prediction, target);
+ *   idx      DEVICE int32 [n_idx] or NULL; entries are not range-checked here;
+ *   err      DEVICE fp32 [B], in the input's units; NaN for a row whose selected points hold a non-finite
+ *            coordinate, or whose selected predicted points all coincide (n_idx == 1 included);
+ *   aligned  DEVICE fp32 [B, n_points, 3] or NULL: s R s1[k] + t for every point;
+ *   params   DEVICE fp32 [B, 13] or NULL: s, R (row-major), t.  NaN rows are NaN throughout. */
+int dpb_procrustes(const float* s1, const float* s2, int64_t B, int n_points, const int32_t* idx, int n_idx,
+                   float* err, float* aligned, float* params, void* stream);
+
 /* Self-intersection metric (replaces self_intersections_percentage lib/utils/metric.py:41-89, pymeshlab on the CPU).
  * A pair of distinct faces intersects according to s, the number of vertex ids they share: s = 0 the closed triangles
  * have a common point; s = 1 the edge opposite the shared vertex, moved halfway to it, crosses the other face's open
