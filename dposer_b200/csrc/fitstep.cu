@@ -8,7 +8,9 @@
 //   adam_kernel                                    torch.optim.Adam's update (the reference's optimiser in
 //       run/completion.py:178, run/motion_denoising.py:217, run/smplify.py:206,236), fused with the gradient assembly
 //   affine_cols_kernel                             Posenormalizer z-score (lib/dataset/AMASS.py:187-259)
-//   joint_map kernels                              lib/body_model/smpl.py:70 joints[:, joint_map] and its adjoint
+//   axis_to_rot6d kernels                          Posenormalizer.offline_normalize(from_axis=True) of a rot6d prior
+//       (run/smplify.py:109-115, lib/utils/transforms.py:237-255) and its vector-Jacobian product
+//   joint_map kernels                             lib/body_model/smpl.py:70 joints[:, joint_map] and its adjoint
 #include <cmath>
 
 #include "common.cuh"
@@ -171,6 +173,92 @@ __global__ void affine_cols_kernel(const float* __restrict__ x, int64_t ldx, con
   out[r * ldo + c] = inverse ? xv * sd[c] + mean[c] : (xv - mean[c]) / sd[c];
 }
 
+// ---- axis-angle -> normalised rot6d, one thread per (row, joint).  With theta = |a| and K = [a]x:
+//   R = I + A K + B K^2,                       A = sin t / t, B = (1 - cos t) / t^2
+//   dR/da_i = C a_i K + A [e_i]x + D a_i K^2 + B ([e_i]x K + K [e_i]x),   C = A' / t, D = B' / t
+// rot6d = (R00, R01, R10, R11, R20, R21), transforms.axis_angle_to_rot6d's [:, :3, :2] layout.
+//
+// Series branch: below theta = 1.2 the four coefficients come from their Taylor series through theta^8, above it from
+// the closed forms.  In fp32 the closed forms lose to cancellation as theta falls (C and D worst, D ~ 1e-6 relative at
+// 1.2 and 2e-6 at 0.9); the five-term series is within 2.5e-7 relative everywhere below 1.2 (its first dropped term is
+// largest for A: theta^10 / 11!).  The three-term series (through theta^4) cannot do this: where its truncation error
+// falls to 1e-6 (theta ~ 0.5), the closed form of D is already 1e-5 off.  Both figures are measured against fp64.
+// theta = 0 lands in the series branch and needs no special case; a non-finite coordinate fails the comparison,
+// takes the closed form and turns the joint's outputs into NaN (every output entry carries a B or D factor).
+struct Rot6dCoefs {
+  float A, B, C, D;
+};
+
+__device__ __forceinline__ Rot6dCoefs rot6d_coefs(float t2) {
+  Rot6dCoefs k;
+  if (t2 < 1.44f) {
+    k.A = 1.f + t2 * (-1.f / 6 + t2 * (1.f / 120 + t2 * (-1.f / 5040 + t2 * (1.f / 362880))));
+    k.B = 0.5f + t2 * (-1.f / 24 + t2 * (1.f / 720 + t2 * (-1.f / 40320 + t2 * (1.f / 3628800))));
+    k.C = -1.f / 3 + t2 * (1.f / 30 + t2 * (-1.f / 840 + t2 * (1.f / 45360 + t2 * (-1.f / 3991680))));
+    k.D = -1.f / 12 + t2 * (1.f / 180 + t2 * (-1.f / 6720 + t2 * (1.f / 453600 + t2 * (-1.f / 47900160))));
+  } else {
+    const float t = sqrtf(t2);
+    float s, c;
+    sincosf(t, &s, &c);
+    const float it2 = 1.f / t2;
+    k.A = s / t;
+    k.B = (1.f - c) * it2;
+    k.C = (t * c - s) / (t2 * t);
+    k.D = (t * s - 2.f * (1.f - c)) * (it2 * it2);
+  }
+  return k;
+}
+
+__global__ void __launch_bounds__(256) axis_to_rot6d_kernel(const float* __restrict__ x, int64_t ldx,
+                                                             const float* __restrict__ mean, const float* __restrict__ sd,
+                                                             float* __restrict__ out, int64_t ldo, int64_t rows, int nj) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows * nj) return;
+  const int64_t r = i / nj;
+  const int j = (int)(i % nj);
+  const float* a = x + r * ldx + 3 * j;
+  const float a0 = a[0], a1 = a[1], a2 = a[2];
+  const float q0 = a0 * a0, q1 = a1 * a1, q2 = a2 * a2;
+  const Rot6dCoefs k = rot6d_coefs(q0 + q1 + q2);
+  // K^2 = a a^T - theta^2 I; its diagonal as -(sum of the other two squares), free of cancellation
+  const float rot[6] = {1.f - k.B * (q1 + q2), -k.A * a2 + k.B * a0 * a1,
+                        k.A * a2 + k.B * a0 * a1, 1.f - k.B * (q0 + q2),
+                        -k.A * a1 + k.B * a0 * a2, k.A * a0 + k.B * a1 * a2};
+  float* o = out + r * ldo + 6 * j;
+#pragma unroll
+  for (int c = 0; c < 6; ++c) o[c] = (rot[c] - mean[6 * j + c]) / sd[6 * j + c];
+}
+
+// g_x_i = <G, dR/da_i> with G = the cotangent of R (rows 0..2, columns 0..1 from g / std, column 2 zero):
+//   g_x = a (C <G,K> + D (a^T G a - theta^2 tr G) - 2 B tr G) + A w + B (G a + G^T a),
+// where w = (G21 - G12, G02 - G20, G10 - G01) is the vector of G's skew part (<G, [v]x> = v . w).
+__global__ void __launch_bounds__(256) axis_to_rot6d_vjp_kernel(const float* __restrict__ x, int64_t ldx,
+                                                                 const float* __restrict__ sd, const float* __restrict__ g,
+                                                                 int64_t ldg, float* __restrict__ g_x, int64_t ldgx,
+                                                                 int64_t rows, int nj) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows * nj) return;
+  const int64_t r = i / nj;
+  const int j = (int)(i % nj);
+  const float* a = x + r * ldx + 3 * j;
+  const float a0 = a[0], a1 = a[1], a2 = a[2];
+  const float t2 = a0 * a0 + a1 * a1 + a2 * a2;
+  const Rot6dCoefs k = rot6d_coefs(t2);
+  const float* gr = g + r * ldg + 6 * j;
+  const float G00 = gr[0] / sd[6 * j], G01 = gr[1] / sd[6 * j + 1], G10 = gr[2] / sd[6 * j + 2],
+              G11 = gr[3] / sd[6 * j + 3], G20 = gr[4] / sd[6 * j + 4], G21 = gr[5] / sd[6 * j + 5];
+  const float w0 = G21, w1 = -G20, w2 = G10 - G01;           // G02 = G12 = 0
+  const float trG = G00 + G11;
+  const float Ga0 = G00 * a0 + G01 * a1, Ga1 = G10 * a0 + G11 * a1, Ga2 = G20 * a0 + G21 * a1;    // G a
+  const float Gta0 = G00 * a0 + G10 * a1 + G20 * a2, Gta1 = G01 * a0 + G11 * a1 + G21 * a2;       // G^T a (third: 0)
+  const float aGa = a0 * Ga0 + a1 * Ga1 + a2 * Ga2;
+  const float s = k.C * (a0 * w0 + a1 * w1 + a2 * w2) + k.D * (aGa - t2 * trG) - 2.f * k.B * trG;
+  float* o = g_x + r * ldgx + 3 * j;
+  o[0] = s * a0 + k.A * w0 + k.B * (Ga0 + Gta0);
+  o[1] = s * a1 + k.A * w1 + k.B * (Ga1 + Gta1);
+  o[2] = s * a2 + k.A * w2 + k.B * Ga2;
+}
+
 // cotangent of mean((x*m - o*m)^2) (nn.MSELoss 'mean' on masked tensors, run/completion.py:197): 2 m^2 (x - o) / n
 __global__ void masked_mse_grad_kernel(const float* __restrict__ x, const float* __restrict__ o,
                                        const float* __restrict__ m, float* __restrict__ g, int64_t n) {
@@ -275,6 +363,35 @@ extern "C" int dpb_affine_cols(const float* x, int64_t ldx, const float* mean, c
   PtrDeviceGuard guard(x);
   const int64_t n = rows * cols;
   affine_cols_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, ldx, mean, sd, out, ldo, rows, cols, inverse, squash);
+  DPB_CUDA_CHECK(cudaGetLastError());
+  return DPB_OK;
+}
+
+extern "C" int dpb_axis_to_rot6d_cols(const float* x, int64_t ldx, const float* mean, const float* sd, float* out,
+                                      int64_t ldo, int64_t rows, int n_joints, void* stream) {
+  DPB_REQUIRE(x && mean && sd && out && n_joints > 0 && rows >= 0, "dpb_axis_to_rot6d_cols: bad argument");
+  DPB_REQUIRE(ldx >= 3 * (int64_t)n_joints && ldo >= 6 * (int64_t)n_joints,
+              "dpb_axis_to_rot6d_cols: row strides must cover 3 * n_joints inputs and 6 * n_joints outputs");
+  if (rows == 0) return DPB_OK;
+  PtrDeviceGuard guard(x);
+  const int64_t n = rows * n_joints;
+  axis_to_rot6d_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, ldx, mean, sd, out, ldo, rows,
+                                                                                      n_joints);
+  DPB_CUDA_CHECK(cudaGetLastError());
+  return DPB_OK;
+}
+
+extern "C" int dpb_axis_to_rot6d_cols_vjp(const float* x, int64_t ldx, const float* sd, const float* g, int64_t ldg,
+                                          float* g_x, int64_t ldgx, int64_t rows, int n_joints, void* stream) {
+  DPB_REQUIRE(x && sd && g && g_x && n_joints > 0 && rows >= 0, "dpb_axis_to_rot6d_cols_vjp: bad argument");
+  DPB_REQUIRE(ldx >= 3 * (int64_t)n_joints && ldg >= 6 * (int64_t)n_joints && ldgx >= 3 * (int64_t)n_joints,
+              "dpb_axis_to_rot6d_cols_vjp: row strides must cover 3 * n_joints inputs / gradients and 6 * n_joints "
+              "cotangents");
+  if (rows == 0) return DPB_OK;
+  PtrDeviceGuard guard(x);
+  const int64_t n = rows * n_joints;
+  axis_to_rot6d_vjp_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, ldx, sd, g, ldg, g_x, ldgx,
+                                                                                          rows, n_joints);
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;
 }

@@ -12,6 +12,19 @@ No framework op runs inside an Adam step: the computation graph of each referenc
 the native kernels by hand (``steps.py``): normalise -> prior loss + closed-form gradient -> LBS forward -> loss
 kernels (value + cotangents) -> LBS backward -> fused Adam.  With ``graphs=True`` every step index is captured once
 into a CUDA graph and replayed for every further batch of independent problems that reuses the buffers.
+
+The prior's input follows the score network's width, chosen once when the buffers are set up:
+
+* 63-D (axis-angle) network: x0 = (pose - mean_poses) / std_poses, and Adam scales the prior's gradient by 1 / std.
+* 126-D (rot6d) network: x0 = normalize(axis_angle_to_rot6d(pose)) with the normaliser's active rule
+  (``Posenormalizer.column_affine``), and the prior's gradient returns to the axis-angle pose through the Jacobian of
+  that map (``steps.axis_to_rot6d_cols`` / ``axis_to_rot6d_cols_vjp``).  This is what ``prior.DPoser.forward`` (and
+  the reference's SMPLify prior, run/smplify.py:109-115) computes.  This project applies the same input to the
+  motion-denoising prior: the reference's motion loop normalises without ``from_axis`` (run/motion_denoising.py:238),
+  so it cannot take a rot6d network at all.
+
+The normaliser must match the network: a rot6d network with an axis normaliser, or the reverse, raises ValueError; a
+rot6d network with a normaliser that has no ``rot_rep`` (no rot6d statistics) raises NotImplementedError.
 """
 import math
 
@@ -25,6 +38,23 @@ from .prior import MotionPrior
 
 # constants.JOINT_IDS of ['OP Neck', 'OP RHip', 'OP LHip', 'Right Hip', 'Left Hip'] (run/smplify.py:136-137)
 IGN_JOINTS = [1, 9, 12, 27, 28]
+
+
+def _prior_input(model, normalizer, who):
+    """True for a 126-D (rot6d) prior, False for a 63-D one.  A 126-D prior takes its input rule from a
+    Posenormalizer(rot_rep='rot6d') (``column_affine``); a normaliser without ``rot_rep`` is read as 63-D axis
+    statistics, as before, so it serves the axis prior only.  A normaliser of the other representation is a ValueError."""
+    rot6d = model.pose_width == L.POSE_DIM_ROT6D
+    want = 'rot6d' if rot6d else 'axis'
+    rep = getattr(normalizer, 'rot_rep', None)
+    if rot6d and rep is None:
+        raise NotImplementedError(f'{who}: the native chain feeds a rot6d (126-D) prior through a '
+                                  f"Posenormalizer(rot_rep='rot6d'); got {type(normalizer).__name__}, which has no "
+                                  'rot6d statistics')
+    if (rep or 'axis') != want:
+        raise ValueError(f'{who}: a {model.pose_width}-D score network needs a Posenormalizer(rot_rep={want!r}), '
+                         f'got rot_rep={rep!r}')
+    return rot6d
 
 
 def _quan_t(strategy, N, total, step, trun, sample_time, offset):
@@ -42,9 +72,7 @@ class MotionDenoise(MotionPrior):
     def __init__(self, config, args, diffusion_model, body_model, sde, normalizer, sde_N=1000, dposer_weight=1.0,
                  out_path=None, debug=False, batch_size=1, seq_len=None):
         """batch_size = total rows (frames).  seq_len = frames per independent sequence (default: one sequence)."""
-        if getattr(diffusion_model, 'is_rot6d', False):
-            raise NotImplementedError('MotionDenoise runs the 63-D axis prior natively; a rot6d (126-D) prior needs an '
-                                      'axis-to-rot6d kernel and its Jacobian in the native step chain')
+        self.rot6d = _prior_input(diffusion_model, normalizer, 'MotionDenoise')
         sde.N = sde_N                                            # run/motion_denoising.py:91
         super().__init__(diffusion_model, sde, config.training.continuous, batch_size)
         self.args, self.debug, self.device = args, debug, args.device
@@ -79,12 +107,17 @@ class MotionDenoise(MotionPrior):
         core = self.body_model.core
         rows = self.batch_size
         f = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)   # noqa: E731
-        b = dict(dev=dev, full_pose=f(rows, core.J * 3), shape=f(rows, core.S), x0=f(rows, 63), target=f(rows, 22, 3),
-                 z=f(rows, 63), lbs=S.LbsStep(core, rows, dev, need_verts=True),
-                 prior=S.PriorStep(self.model, self.sde, self.continuous, rows, dev),
-                 mean=self.Normalizer.mean_poses.to(dev).float().contiguous(),
-                 std=self.Normalizer.std_poses.to(dev).float().contiguous(), graphs=None, sched_key=None, seed=0)
-        b['inv_std'] = (1.0 / b['std']).contiguous()
+        pw = self.model.pose_width
+        b = dict(dev=dev, full_pose=f(rows, core.J * 3), shape=f(rows, core.S), x0=f(rows, pw), target=f(rows, 22, 3),
+                 z=f(rows, pw), lbs=S.LbsStep(core, rows, dev, need_verts=True),
+                 prior=S.PriorStep(self.model, self.sde, self.continuous, rows, dev), graphs=None, sched_key=None, seed=0)
+        if self.rot6d:
+            mean, std = self.Normalizer.column_affine()
+            b['g_axis'] = f(rows, 63)                   # the prior's gradient w.r.t. the axis-angle body pose
+        else:
+            mean, std = self.Normalizer.mean_poses, self.Normalizer.std_poses
+        b['mean'], b['std'] = mean.to(dev).float().contiguous(), std.to(dev).float().contiguous()
+        b['inv_std'] = None if self.rot6d else (1.0 / b['std']).contiguous()
         b['opt'] = S.Adam(b['full_pose'], 3, 63, 0.03)
         self._bufs = b
         return b
@@ -136,16 +169,22 @@ class MotionDenoise(MotionPrior):
 
         def one_step(k):
             it = sched[k][0]
-            S.affine_cols(b['full_pose'], 3, J3, b['mean'], b['std'], b['x0'])          # Posenormalizer (:238)
+            if self.rot6d:
+                S.axis_to_rot6d_cols(b['full_pose'], 3, b['mean'], b['std'], b['x0'])
+            else:
+                S.affine_cols(b['full_pose'], 3, J3, b['mean'], b['std'], b['x0'])      # Posenormalizer (:238)
             z = None
             if z_list is not None:
                 b['z'].copy_(z_list[k].to(dev))
                 z = b['z']
-            pri(b['x0'], k, False, float(self.batch_size_divisor), z=z, seed=seed, step=k)   # DPoser_loss (:251)
+            g_prior = pri(b['x0'], k, False, float(self.batch_size_divisor), z=z, seed=seed, step=k)   # DPoser_loss (:251)
+            if self.rot6d:
+                S.axis_to_rot6d_cols_vjp(b['full_pose'], 3, b['std'], g_prior, b['g_axis'])
+                g_prior = b['g_axis']
             lbs.forward(b['shape'], b['full_pose'], None)                               # body model (:255)
             S.motion_loss(lbs, b['target'], L_, 22, wd['temp'](1.0, it), wd['data'](1.0, it))   # :256-262
             lbs.backward(b['shape'], b['full_pose'], use_verts=True)
-            opt.step(lbs.g_pose, 3, J3, 1.0, g2=pri.grad, off2=0, ld2=63, s2=wd['dposer'](1.0, it),
+            opt.step(lbs.g_pose, 3, J3, 1.0, g2=g_prior, off2=0, ld2=63, s2=wd['dposer'](1.0, it),
                      col_scale2=b['inv_std'])                                           # Adam (:266-268)
 
         for k in range(total_steps):
@@ -176,9 +215,7 @@ class SMPLify:
 
     def __init__(self, body_model, step_size=1e-2, batch_size=32, num_iters=100, focal_length=5000, args=None,
                  pose_prior=None, per_problem=True):
-        if pose_prior is not None and getattr(pose_prior.model, 'is_rot6d', False):
-            raise NotImplementedError('SMPLify runs the 63-D axis prior natively; a rot6d (126-D) DPoser prior needs an '
-                                      'axis-to-rot6d kernel and its Jacobian in the native step chain')
+        self.rot6d = pose_prior is not None and _prior_input(pose_prior.model, pose_prior.Normalizer, 'SMPLify')
         self.smpl = body_model
         self.device = getattr(args, 'device', None)
         self.focal_length = focal_length
@@ -231,7 +268,8 @@ class SMPLify:
         jmap = smpl.joint_map.to(device=dev, dtype=torch.int32).contiguous()
         K = jmap.numel()
         j49, g49, loss_b = f(B, K, 3), f(B, K, 3), f(B)
-        g_cam, g_fit_pose, g_fit_betas, x0 = f(B, 3), f(B, J3), f(B, S_), f(B, 63)
+        pw = self.pose_prior.model.pose_width if self.pose_prior is not None else 63
+        g_cam, g_fit_pose, g_fit_betas, x0 = f(B, 3), f(B, J3), f(B, S_), f(B, pw)
         conf = joints_conf.contiguous().float()
 
         def forward_joints(no_save=False):
@@ -266,13 +304,15 @@ class SMPLify:
             pri = S.PriorStep(pp.model, pp.sde, pp.continuous, B, dev)
             qts = [self.sample_discrete_time(k) for k in range(total)] + [self.sample_discrete_time(self.num_iters - 1)]
             pri.schedule([float(pp.timesteps[int(q)]) for q in qts])
-            mean = pp.Normalizer.mean_poses.to(dev).float().contiguous()
-            std = pp.Normalizer.std_poses.to(dev).float().contiguous()
-            inv_std = (1.0 / std).contiguous()
+            mean, std = pp.Normalizer.column_affine() if self.rot6d else (pp.Normalizer.mean_poses,
+                                                                          pp.Normalizer.std_poses)
+            mean, std = mean.to(dev).float().contiguous(), std.to(dev).float().contiguous()
+            inv_std = None if self.rot6d else (1.0 / std).contiguous()
+            g_axis = f(B, 63) if self.rot6d else None   # the prior's gradient w.r.t. the axis-angle body pose
         opt_b, opt_s = S.Adam(full_pose, 3, 63, self.step_size), S.Adam(shape, 0, 10, self.step_size)
         opt_g2 = S.Adam(full_pose, 0, 3, self.step_size)
         seed = mutils.host_seed() if z_list is None else 0
-        zbuf = f(B, 63)
+        zbuf = f(B, pw)
         stage_weights = [dict(zip(self.loss_weights.keys(), vals)) for vals in zip(*self.loss_weights.values())]
 
         def body_step(k, w):
@@ -285,12 +325,18 @@ class SMPLify:
             backward_joints(False)
             g2 = None
             if pp is not None:
-                S.affine_cols(full_pose, 3, J3, mean, std, x0)
+                if self.rot6d:
+                    S.axis_to_rot6d_cols(full_pose, 3, mean, std, x0)         # offline_normalize(from_axis=True)
+                else:
+                    S.affine_cols(full_pose, 3, J3, mean, std, x0)
                 z = None
                 if z_list is not None:
                     zbuf.copy_(z_list[k].to(dev))
                     z = zbuf
                 g2 = pri(x0, k, True, 1.0, z=z, seed=seed, step=k)          # DPoser.forward: weighted, sum / 1 per image
+                if self.rot6d:
+                    S.axis_to_rot6d_cols_vjp(full_pose, 3, std, g2, g_axis)
+                    g2 = g_axis
             opt_b.step(lbs.g_pose, 3, J3, 1.0, g2=g2, off2=0, ld2=63, s2=float(w['pose_prior_weight']) ** 2,
                        col_scale2=inv_std if pp is not None else None, g3=g_fit_pose, off3=0, ld3=J3, s3=1.0)
             opt_s.step(lbs.g_shape, 0, S_, 1.0, g3=g_fit_betas, off3=0, ld3=S_, s3=1.0)

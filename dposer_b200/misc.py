@@ -103,6 +103,16 @@ class Posenormalizer:
         mean, std = self._stats(poses, self.mean_poses, self.std_poses)
         return (poses - mean) / std
 
+    def column_affine(self):
+        """(mean, std), one entry per column, with offline_normalize(poses) == (poses - mean) / std under the active
+        rule: z-score as stored; min-max as mean = (lo + hi) / 2, std = (hi - lo) / 2; normalize=False as 0 / 1.
+        The native fitting chains take this form (``steps.axis_to_rot6d_cols``)."""
+        if not self.normalize:
+            return torch.zeros_like(self.mean_poses), torch.ones_like(self.std_poses)
+        if self.min_max:
+            return (self.min_poses + self.max_poses) / 2, (self.max_poses - self.min_poses) / 2
+        return self.mean_poses, self.std_poses
+
     def offline_denormalize(self, poses, to_axis=False):
         assert len(poses.shape) in (2, 3)
         if self.normalize:

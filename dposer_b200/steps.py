@@ -115,6 +115,48 @@ def affine_cols(x, off, ld, mean, std, out, inverse=False, out_off=0, out_ld=Non
                                      float(squash), L.current_stream(out.device)))
 
 
+def _rot6d_operands(x, off, rows, nj, cols):
+    """Checks of the two rot6d calls, all before any library call: ``x`` [rows, ld] holds 3 * nj axis-angle columns
+    from ``off``; ``cols`` lists (name, tensor, width): a [rows, width] matrix, or for width None the 6 * nj per-column
+    statistics.  Shapes first (ValueError), then devices (RuntimeError for a CPU tensor)."""
+    if x.dim() != 2 or nj < 1 or x.shape[0] != rows or off < 0 or off + 3 * nj > x.shape[1]:
+        raise ValueError(f'x: expected {rows} rows holding {3 * nj} axis-angle columns from column {off}, '
+                         f'got {list(x.shape)}')
+    for name, t, width in cols:
+        if (t.numel() != 6 * nj) if width is None else (list(t.shape) != [rows, width]):
+            raise ValueError(f'{name}: expected {[6 * nj] if width is None else [rows, width]}, got {list(t.shape)}')
+    named = [('x', x)] + [c[:2] for c in cols]
+    for name, t in named:
+        if t.dtype != torch.float32 or not t.is_contiguous():
+            raise ValueError(f'{name}: expected a contiguous float32 tensor, got {t.dtype}')
+    for name, t in named:
+        L.require_cuda(t, name)
+        if t.device != x.device:
+            raise ValueError(f'{name}: on {t.device}, x on {x.device}')
+
+
+def axis_to_rot6d_cols(x, off, mean, std, out):
+    """out[r, 6j:6j+6] = (rot6d(x[r, off+3j : off+3j+3]) - mean[6j:6j+6]) / std[6j:6j+6] for the out.shape[1] / 6
+    joints (dpb_axis_to_rot6d_cols): the input of a rot6d prior from the axis-angle pose inside ``x``."""
+    nj = out.shape[-1] // 6
+    if out.dim() != 2 or out.shape[1] != 6 * nj:
+        raise ValueError(f'out: expected 6 columns per joint, got {list(out.shape)}')
+    _rot6d_operands(x, off, out.shape[0], nj, [('out', out, 6 * nj), ('mean', mean, None), ('std', std, None)])
+    L.check(L.load().dpb_axis_to_rot6d_cols(_p(x, off), x.shape[1], L.ptr(mean), L.ptr(std), L.ptr(out), out.shape[1],
+                                            x.shape[0], nj, L.current_stream(x.device)))
+
+
+def axis_to_rot6d_cols_vjp(x, off, std, g, g_x):
+    """g_x [rows, 3 n] = the cotangent of x[:, off:off+3n] given g [rows, 6 n], the cotangent of axis_to_rot6d_cols'
+    output (dpb_axis_to_rot6d_cols_vjp)."""
+    nj = g.shape[-1] // 6
+    if g.dim() != 2 or g.shape[1] != 6 * nj:
+        raise ValueError(f'g: expected 6 columns per joint, got {list(g.shape)}')
+    _rot6d_operands(x, off, g.shape[0], nj, [('g', g, 6 * nj), ('g_x', g_x, 3 * nj), ('std', std, None)])
+    L.check(L.load().dpb_axis_to_rot6d_cols_vjp(_p(x, off), x.shape[1], L.ptr(std), L.ptr(g), g.shape[1], L.ptr(g_x),
+                                                g_x.shape[1], x.shape[0], nj, L.current_stream(x.device)))
+
+
 def motion_loss(lbs, target, seq_len, n_data, w_temp, w_data, seq_terms=None):
     L.check(L.load().dpb_motion_loss(L.ptr(lbs.verts), L.ptr(lbs.joints), L.ptr(target), lbs.rows, seq_len, lbs.core.V,
                                      lbs.core.n_out, n_data, float(w_temp), float(w_data), L.ptr(lbs.g_verts),

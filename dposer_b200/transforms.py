@@ -7,8 +7,9 @@ properties (round trips, orthonormality, agreement with the LBS oracle's Rodrigu
 torchgeometry's published algorithms (oracle/tgm_ref.py); the Gram-Schmidt leg is pinned bit-exactly to the reference.
 ``misc.Posenormalizer(rot_rep='rot6d')`` and ``misc.create_mask(observation_type='mean')`` call them at the data boundary;
 the score-net kernels take both representations (63-D axis, 126-D rot6d score networks: ``ScoreModelFC(config, 21, 6)``).
-The native SMPLify / motion-denoising chains (``fitting.py``) run the axis prior only: a rot6d prior there would need this
-conversion and its Jacobian as a kernel inside the step."""
+With a rot6d prior the native SMPLify / motion-denoising chains (``fitting.py``) do not call this module: the
+axis -> rot6d map of ``axis_angle_to_rot6d`` and its Jacobian run as kernels inside the step
+(``steps.axis_to_rot6d_cols`` / ``axis_to_rot6d_cols_vjp``), tested against float64 autograd through this function."""
 import torch
 import torch.nn.functional as F
 

@@ -317,6 +317,19 @@ int dpb_masked_mse_grad(const float* x, const float* obs, const float* mask, flo
  * score weights use it to bring the sampler's output into a plausible angle range before the body model. */
 int dpb_affine_cols(const float* x, int64_t ldx, const float* mean, const float* std, float* out, int64_t ldo,
                     int64_t rows, int cols, int inverse, float squash, void* stream);
+/* The input of a rot6d (126-D) prior from axis-angle poses: Posenormalizer.offline_normalize(poses, from_axis=True)
+ * (run/smplify.py:109-115, with axis_angle_to_rot6d of lib/utils/transforms.py:237-255), on strided views.  For joint j
+ * of row r, a = x[r*ldx + 3j .. 3j+2] and R = I + (sin t / t)[a]x + ((1 - cos t) / t^2)[a]x^2 (t = |a|):
+ *   out[r*ldo + 6j + k] = (rot6d_k - mean[6j+k]) / std[6j+k],   rot6d = (R00, R01, R10, R11, R20, R21).
+ * mean / std [6 n_joints] express every rule of the normaliser: z-score; min-max as mean = (lo + hi) / 2,
+ * std = (hi - lo) / 2; no normalisation as 0 / 1.  The map is smooth through t = 0 (series below t = 1.2, see
+ * fitstep.cu); a non-finite coordinate gives NaN in that joint's 6 outputs only. */
+int dpb_axis_to_rot6d_cols(const float* x, int64_t ldx, const float* mean, const float* std, float* out, int64_t ldo,
+                           int64_t rows, int n_joints, void* stream);
+/* Its vector-Jacobian product: g_x[r*ldgx + 3j + i] = sum_k (g[r*ldg + 6j+k] / std[6j+k]) d rot6d_k / d a_i, recomputed
+ * from x (nothing is saved by the forward); NaN in a joint's 3 entries when its input is non-finite. */
+int dpb_axis_to_rot6d_cols_vjp(const float* x, int64_t ldx, const float* std, const float* g, int64_t ldg, float* g_x,
+                               int64_t ldgx, int64_t rows, int n_joints, void* stream);
 /* out[r,c] = w0 x[r-1,c] + w1 x[r,c] + w2 x[r+1,c] inside each sequence of seq_len rows, zero-padded at its ends
  * (gaussian_smoothing(window_size=3), lib/utils/misc.py:84-95, per sequence as in run/motion_denoising.py:281-285);
  * keep_ends != 0 copies the first and last row of every sequence instead.  out must not alias x. */
