@@ -295,9 +295,8 @@ extern "C" int dpb_score_jvp(dpb_score_t* h, const float* x, const float* v, con
     return fail(DPB_ENOMEM, "dpb_score_jvp: workspace too small");
   void* rest = static_cast<uint8_t*>(ws) + c.off;
   // batch-uniform time (the likelihood's case): every contraction on tcgen05; per-row tables keep the fp32 SGEMM path
-  static const bool force_fp32 = getenv("DPB_JVP_FP32") && atoi(getenv("DPB_JVP_FP32")) != 0;
-  int rc = (!t_index && !force_fp32) ? score_jvp_tc_raw(h, x, v, table, raw, B, rest, ws_bytes - c.off, st)
-                                     : simt_forward_jvp_raw(h, x, v, table, t_index, raw, B, rest, ws_bytes - c.off, st);
+  int rc = !t_index ? score_jvp_tc_raw(h, x, v, table, raw, B, rest, ws_bytes - c.off, st)
+                    : simt_forward_jvp_raw(h, x, v, table, t_index, raw, B, rest, ws_bytes - c.off, st);
   if (rc != DPB_OK) return rc;
   rc = launch_scale_out(raw, row_scale, scale, out, B, DP, st);
   if (rc != DPB_OK) return rc;

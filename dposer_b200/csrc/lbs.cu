@@ -4,8 +4,6 @@
 //
 // Follows smplx==0.1.28 lbs()/SMPL.forward/SMPLX.forward as called by the reference at
 // lib/body_model/body_model.py:75-88 and lib/body_model/smpl.py:67-78 (SURVEY.md Appendix A.6).
-#include <cstdlib>
-
 #include "lbs.h"
 
 #include <algorithm>
@@ -609,18 +607,16 @@ extern "C" int dpb_lbs_forward(dpb_lbs_t* h, const float* betas, const float* fu
   dpb_lbs* hv = compact ? h->sub : h;
   const bool use_tc = n_verts > 0 && hv && hv->tc_ready && w.featop &&
                       (engine == DPB_LBS_ENGINE_TC || (engine == DPB_ENGINE_AUTO && B >= 64));
-  const int fused_sel = getenv("DPB_LBS_FUSED") ? atoi(getenv("DPB_LBS_FUSED")) : 3;   // A/B timing only: 0 two kernels, 1 first fused kernel, 2 / 3 CTA-pair kernels
   // const-tail calls (DPB_LBS_CONST_TAIL) read the pruned basis; everything else the full one
   const bool want_tail = (flags & DPB_LBS_CONST_TAIL) != 0;
   if (want_tail) DPB_REQUIRE(h->tailv.n_var > 0 || !h->tc_ready, "dpb_lbs_forward: DPB_LBS_CONST_TAIL without dpb_lbs_set_const_tail");
   // (the compact model's variants have the same K layout: the pose kernel's operands serve both)
   const LbsVariant var = !use_tc ? ((want_tail && h->tailv.dirs16) ? h->tailv : lbs_full_variant(h))
                                  : ((want_tail && hv->tailv.dirs16) ? hv->tailv : lbs_full_variant(hv));
-  // measured (profiles/r2_lbs_fused3_experiments.md): the 128-pose-group kernel wins for SMPL-sized joint counts (one
-  // skinning K slab), the 96-pose-group kernel for SMPL-X (two slabs: its three T buffers hide the longer chunks)
-  const bool use_fused3 = use_tc && fused_sel == 3 && w.skinop && h->jp == 32 && lbs_fused3_fits(hv, var);
-  const bool use_fused2 = use_fused3 || (use_tc && fused_sel >= 2 && w.skinop && lbs_fused2_fits(hv, var));
-  const bool use_fused = use_fused2 || (use_tc && !compact && fused_sel != 0 && w.skinop && var.n_var == h->J && lbs_tc_fused_fits(h));
+  // blend + skinning in one CTA-pair kernel, chosen by the padded joint count: the 128-pose-group kernel for one
+  // skinning K slab (jp = 32, SMPL), the 96-pose-group kernel for two (jp = 64, SMPL-X)
+  const bool use_fused3 = use_tc && w.skinop && lbs_fused3_fits(hv, var);
+  const bool use_fused = use_fused3 || (use_tc && w.skinop && lbs_fused2_fits(hv, var));
   // the fused kernel's operands come straight out of the pose kernel (pad rows of the last pose group are zeroed)
   __half* fop = use_fused ? w.featop : nullptr;
   __half* sop = use_fused ? w.skinop : nullptr;
@@ -633,7 +629,7 @@ extern "C" int dpb_lbs_forward(dpb_lbs_t* h, const float* betas, const float* fu
     }
   }
   // forward-only fused calls (DPB_LBS_NO_SAVE): nothing downstream reads the fp32 transforms / features
-  const bool no_save = (flags & DPB_LBS_NO_SAVE) && use_fused2;
+  const bool no_save = (flags & DPB_LBS_NO_SAVE) && use_fused;
   float* A_o = no_save ? nullptr : w.A;
   float* G_o = no_save ? nullptr : w.G;
   float* feat_o = no_save ? nullptr : w.feat;
@@ -652,13 +648,10 @@ extern "C" int dpb_lbs_forward(dpb_lbs_t* h, const float* betas, const float* fu
     if (!compact && engine == DPB_LBS_ENGINE_TC && !use_tc)
       return fail(DPB_EUNSUPPORTED, "dpb_lbs_forward: tensor-core engine unavailable");
     if (use_tc) {
-      if (use_fused2) {
-        // blend + skinning in one tcgen05 kernel on CTA pairs: the blended vertices stay in TMEM
+      if (use_fused) {
+        // the blended vertices stay in TMEM
         int rc = use_fused3 ? lbs_fused3(hv, var, w.featop, w.skinop, vout, B, st)
                             : lbs_fused2(hv, var, w.featop, w.skinop, vout, B, st);
-        if (rc != DPB_OK) return rc;
-      } else if (use_fused) {
-        int rc = lbs_tc_fused(h, nullptr, nullptr, w.featop, nullptr, nullptr, w.skinop, verts, B, st);
         if (rc != DPB_OK) return rc;
       } else {
       // blend on tcgen05 (writes v_posed into verts), then skin in place with the transforms from the pose kernel

@@ -104,9 +104,6 @@ int lbs_tc_skin(dpb_lbs* h, const float* A, const float* transl, __half* skinop,
 bool lbs_tc_skin_fits(const dpb_lbs* h);
 int lbs_tc_skin_adjoint(dpb_lbs* h, const float* A, __half* skinop, const float* g_verts, const float* gextra,
                         bool have_extra, const float* scale, __half* gvp16, int64_t B, cudaStream_t st);
-bool lbs_tc_fused_fits(const dpb_lbs* h);
-int lbs_tc_fused(dpb_lbs* h, const float* betas, const float* feat, __half* featop, const float* A, const float* transl,
-                 __half* skinop, float* verts, int64_t B, cudaStream_t st);
 inline LbsVariant lbs_full_variant(const dpb_lbs* h) {
   LbsVariant v;
   v.n_var = h->J; v.p_feat = h->P; v.kext = h->kext; v.dirs16 = h->dirs16; v.tm_dirs = h->tm_dirs;

@@ -16,8 +16,6 @@
 //
 // This is the adjoint of lbs.cu (smplx 0.1.28 lbs(); reference call sites lib/body_model/body_model.py:75-88,
 // run/motion_denoising.py:255-268, run/smplify.py:243-258 where autograd differentiates the smplx ops).
-#include <cstdlib>
-
 #include "lbs.h"
 
 namespace dpb {
@@ -637,9 +635,9 @@ extern "C" int dpb_lbs_backward(dpb_lbs_t* h, const float* betas, const float* f
     float* gvp = reinterpret_cast<float*>(sp + align_up((size_t)B * h->V * 3 * 4, 256));
     float* gout = reinterpret_cast<float*>(sp + align_up((size_t)B * h->V * 3 * 4, 256) + bwd_gvp_bytes(h, B));
     float* scale = reinterpret_cast<float*>(sp + bwd_scratch_bytes(h, B) - align_up((size_t)B * 4, 256));
-    // skinning adjoint (dL/dA) and transposed blend on tcgen05 unless DPB_LBS_BWD_FP32=1 asks for the round-1 kernels
-    // (shared-memory atomics + fp32 SGEMM; A/B timing)
-    const bool tcT = h->bt_ready && h->sb_ready && w.skinop && lbs_tc_skin_fits(h) && !(getenv("DPB_LBS_BWD_FP32") && atoi(getenv("DPB_LBS_BWD_FP32")));
+    // skinning adjoint (dL/dA) and transposed blend on tcgen05 where the model's operands exist, else the round-1
+    // kernels (shared-memory atomics + fp32 SGEMM)
+    const bool tcT = h->bt_ready && h->sb_ready && w.skinop && lbs_tc_skin_fits(h);
     __half* gvp16 = tcT ? reinterpret_cast<__half*>(gvp) : nullptr;
     // v_posed recompute with the basis the forward used (const-tail: K = 224 instead of 512 for SMPL-X)
     const LbsVariant bvar = ((flags & DPB_LBS_CONST_TAIL) && h->tailv.dirs16) ? h->tailv : lbs_full_variant(h);
@@ -675,8 +673,7 @@ extern "C" int dpb_lbs_backward(dpb_lbs_t* h, const float* betas, const float* f
     }
   } else if (!full && have_extra && h->sub && h->sub->bt_ready && h->sub->sb_ready && w.featop && w.skinop &&
              lbs_tc_skin_fits(h->sub) && scratch &&
-             scratch_bytes >= bwd_scratch_bytes(h->sub, B) &&
-             !(getenv("DPB_LBS_BWD_FP32") && atoi(getenv("DPB_LBS_BWD_FP32")))) {
+             scratch_bytes >= bwd_scratch_bytes(h->sub, B)) {
     // joints-only mode: the cotangents of the compact vertex set go through the same tensor-core pass
     int rc = bwd_vertex_pass_tc(h->sub, (flags & DPB_LBS_CONST_TAIL) != 0, w, betas, w.gextra, nullptr, false,
                                 static_cast<uint8_t*>(scratch), B, st);

@@ -2,10 +2,10 @@
 // SMPL and (with the constant hand / face tail folded away) SMPL-X.  Replaces smplx 0.1.28 lbs() as called from
 // lib/body_model/body_model.py:75-88 and lib/body_model/smpl.py:67-78 (SURVEY.md App. A.6).
 //
-// Why a second kernel (profiles/r1_ncu_full_summary_final.md, lbs_fused_tc_kernel): tensor pipe 49 % active, the
-// MMA warp waited 63 % of the time for a T buffer and the eight epilogue warps ran one dependent instruction every
-// ~5 cycles.  The tensor work itself is fixed by the 3-product fp16 split (hi.hi + hi.lo + lo.hi), so the whole gap
-// is overlap.  Changes:
+// Why a second kernel (profiles/r1_ncu_full_summary_final.md, the round-1 single-CTA fused kernel): tensor pipe 49 %
+// active, the MMA warp waited 63 % of the time for a T buffer and the eight epilogue warps ran one dependent
+// instruction every ~5 cycles.  The tensor work itself is fixed by the 3-product fp16 split (hi.hi + hi.lo + lo.hi),
+// so the whole gap is overlap.  Changes:
 //   * CTA pair, M = 256: each CTA keeps its own 128-vertex tile of the blend basis / skinning weights (A operands)
 //     and only HALF of every pose-side B operand, so an N = 96 MMA fetches 32 + 12 cycles of shared memory for 48
 //     cycles of math (N = 128 on one CTA: 32 + 32 for 64 -- the pipe and the epilogue's staging compete for the same
@@ -46,13 +46,13 @@ constexpr int NCH = (NP + CP - 1) / CP;        // 20 chunks per group (the last 
 constexpr int NT = 3;                          // T buffers
 constexpr int NSETS = 3;                       // epilogue warp sets (12 warps: 84 TMEM values live per thread need ~150 registers)
 constexpr int NUM_THREADS = 128 + NSETS * 128; // 512
-// pose-side (B) operand tiles: a CTA of a pair (cta_group::2) holds half of the rows, a single CTA all of them
-constexpr int f_slab(bool pair) { return (pair ? NP / 2 : NP) * BK * 2; }   // 6 / 12 KB: poses x 64 k
-constexpr int s_slab(bool pair) { return (pair ? NS / 2 : NS) * BK * 2; }   // 4 / 8 KB: transform rows x 64 k
+// pose-side (B) operand tiles: each CTA of a pair (cta_group::2) holds half of the rows
+constexpr int F_SLAB = NP / 2 * BK * 2;        // 6 KB: poses x 64 k
+constexpr int S_SLAB = NS / 2 * BK * 2;        // 4 KB: transform rows x 64 k
 constexpr int T_COL0 = 3 * NP;                 // 288: first T column
 constexpr int ROLE_REGS = 72, EPI_REGS = 144;  // setmaxnreg: 128 * 72 + 384 * 144 <= 65536
 static_assert(NCH >= NSETS, "every epilogue set handles at least one chunk per tile");
-static_assert(T_COL0 + NT * NS <= 512 && f_slab(true) % 1024 == 0 && s_slab(true) % 1024 == 0, "TMEM / SWIZZLE_128B layout");
+static_assert(T_COL0 + NT * NS <= 512 && F_SLAB % 1024 == 0 && S_SLAB % 1024 == 0, "TMEM / SWIZZLE_128B layout");
 
 struct Params {
   int V, V_pad, n_tp;        // vertices, padded vertices, tile PAIRS (n_vt / 2)
@@ -63,16 +63,14 @@ struct Params {
                              // 4 = no TMEM load of D, 16 = no skinning chunks, 32 = no blend (results are garbage)
 };
 
-template <int JSLABS, int ASTAGES, int SSTAGES, int WBUFS, bool PAIR>
+template <int JSLABS, int ASTAGES, int SSTAGES, int WBUFS>
 struct Smem {
   static constexpr int NSLABS_MAX = 7;
-  static constexpr int F_SLAB = f_slab(PAIR), S_SLAB = s_slab(PAIR);
   static constexpr int OFF_F = 0;
   static constexpr int OFF_A = OFF_F + NSLABS_MAX * F_SLAB;                 // 43008 (1024-aligned)
   static constexpr int OFF_W = OFF_A + ASTAGES * A_SLAB;
   static constexpr int OFF_S = OFF_W + WBUFS * JSLABS * A_SLAB;
-  static constexpr int OFF_STG = OFF_S + SSTAGES * JSLABS * S_SLAB;         // per-warp store staging: 12 warps x CP poses x 384 B
-  static constexpr int OFF_BAR = OFF_STG + NSETS * 4 * CP * 384;
+  static constexpr int OFF_BAR = OFF_S + SSTAGES * JSLABS * S_SLAB;
   static constexpr int NBARS = 2 * ASTAGES + 2 * SSTAGES + 4 + 2 + 2 + 2 * NT;
   static constexpr int BYTES = OFF_BAR + NBARS * 8 + 16 + 1024;             // + tmem slot + alignment slack
   static_assert(OFF_A % 1024 == 0 && OFF_W % 1024 == 0 && OFF_S % 1024 == 0, "operand tiles are 1024-byte aligned");
@@ -81,22 +79,17 @@ struct Smem {
 
 // KH16 = K16 steps of the hi half of the blend K, NSLABS = 64-wide slabs of [hi | lo]; JS = K16 steps of the hi half of
 // the skinning K (joints + translation slot, padded), JSLABS = its 64-wide slabs.  Compile-time: the issuer's loops
-// unroll and every descriptor is base + constant.  STAGED: transpose each pose's 32 x (x,y,z) through shared memory
-// so that the global stores are three full 128-byte lines per warp instead of three stride-12 scatters.
-// PAIR: CTA pair with cta_group::2 MMAs (M = 256, pose-side operands split between the CTAs, the leader issues, barriers
-// cross the pair) / single-CTA cta_group::1 MMAs (M = 128, every barrier local: the MMA -> epilogue -> MMA round trip of
-// a T buffer is ~2.5x shorter, which is what bounds the skinning phase -- measured 488 cycles per chunk on pairs with
-// an EMPTY epilogue against 192 cycles of MMA).
-template <int KH16, int NSLABS, int JS, int JSLABS, int ASTAGES, int SSTAGES, int WBUFS, bool STAGED, bool PAIR>
+// unroll and every descriptor is base + constant.  CTA pair with cta_group::2 MMAs: M = 256, pose-side operands split
+// between the CTAs, the leader issues, barriers cross the pair.
+template <int KH16, int NSLABS, int JS, int JSLABS, int ASTAGES, int SSTAGES, int WBUFS>
 __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(NUM_THREADS, 1)
 lbs_fused2_kernel(const __grid_constant__ Params p, const __grid_constant__ CUtensorMap tm_dirs,
                   const __grid_constant__ CUtensorMap tm_feat, const __grid_constant__ CUtensorMap tm_w,
                   const __grid_constant__ CUtensorMap tm_s) {
-  using L = Smem<JSLABS, ASTAGES, SSTAGES, WBUFS, PAIR>;
-  constexpr int F_SLAB = L::F_SLAB, S_SLAB = L::S_SLAB;
-  constexpr uint32_t IDESC_BLEND = ptx::umma_idesc_f16(PAIR ? 2 * TILE_V : TILE_V, NP, 0);
-  constexpr uint32_t IDESC_SKIN = ptx::umma_idesc_f16(PAIR ? 2 * TILE_V : TILE_V, NS, 0);
-  constexpr int NC = PAIR ? 2 : 1;               // CTAs that feed one MMA stream
+  using L = Smem<JSLABS, ASTAGES, SSTAGES, WBUFS>;
+  constexpr uint32_t IDESC_BLEND = ptx::umma_idesc_f16(2 * TILE_V, NP, 0);
+  constexpr uint32_t IDESC_SKIN = ptx::umma_idesc_f16(2 * TILE_V, NS, 0);
+  constexpr int NC = 2;                          // CTAs that feed one MMA stream
   static_assert(NSLABS <= L::NSLABS_MAX && 2 * KH16 <= 4 * NSLABS && 2 * JS <= 4 * JSLABS, "K geometry");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
@@ -129,35 +122,24 @@ lbs_fused2_kernel(const __grid_constant__ Params p, const __grid_constant__ CUte
     for (int b = 0; b < NT; ++b) { ptx::mbar_init(tfull(b), 1); ptx::mbar_init(tempty(b), NC * 4); }  // one set (both CTAs)
     ptx::fence_barrier_init();
   }
-  if (warp == 2) {
-    if (PAIR) ptx::tmem_alloc_2sm(ptx::smem_u32(tmem_slot), 512);
-    else ptx::tmem_alloc(ptx::smem_u32(tmem_slot), 512);
-  }
+  if (warp == 2) ptx::tmem_alloc_2sm(ptx::smem_u32(tmem_slot), 512);
   ptx::tc_fence_before();
   __syncthreads();
   ptx::cluster_sync();       // the peer's barriers are initialised before anyone arrives on them remotely
   ptx::tc_fence_after();
   const uint32_t tmem_base = *tmem_slot;
-  const uint32_t crank = PAIR ? ptx::cluster_ctarank() : 0;   // single-CTA mode: every CTA is its own worker
+  const uint32_t crank = ptx::cluster_ctarank();
   constexpr uint16_t CMASK = 3;
-  const long long worker = PAIR ? blockIdx.x >> 1 : blockIdx.x, n_workers = PAIR ? gridDim.x >> 1 : gridDim.x;
-  // role-independent wrappers: the pair variant signals the leader's barriers and multicasts commits
-  auto expect = [&](uint32_t fullbar, uint32_t bytes) {
-    if (PAIR) ptx::mbar_arrive_expect_tx_cluster(ptx::mapa(fullbar, 0), bytes);
-    else ptx::mbar_arrive_expect_tx(fullbar, bytes);
-  };
+  const long long worker = blockIdx.x >> 1, n_workers = gridDim.x >> 1;
+  // both CTAs signal the leader's barriers; commits are multicast to the pair
+  auto expect = [&](uint32_t fullbar, uint32_t bytes) { ptx::mbar_arrive_expect_tx_cluster(ptx::mapa(fullbar, 0), bytes); };
   auto load = [&](uint32_t dst, const CUtensorMap* tm, uint32_t fullbar, int c0, int c1) {
-    if (PAIR) ptx::tma_load_2d_2sm(dst, tm, ptx::mapa(fullbar, 0), c0, c1);
-    else ptx::tma_load_2d(dst, tm, fullbar, c0, c1);
+    ptx::tma_load_2d_2sm(dst, tm, ptx::mapa(fullbar, 0), c0, c1);
   };
   auto mma = [&](uint32_t taddr, uint64_t ad, uint64_t bd, uint32_t idesc, uint32_t acc) {
-    if (PAIR) ptx::mma_f16_ss_2sm(taddr, ad, bd, idesc, acc);
-    else ptx::mma_f16_ss(taddr, ad, bd, idesc, acc);
+    ptx::mma_f16_ss_2sm(taddr, ad, bd, idesc, acc);
   };
-  auto commit = [&](uint32_t b) {
-    if (PAIR) ptx::mma_commit_2sm_mcast(b, CMASK);
-    else ptx::mma_commit(b);
-  };
+  auto commit = [&](uint32_t b) { ptx::mma_commit_2sm_mcast(b, CMASK); };
   const long long i0 = p.n_items * worker / n_workers, i1 = p.n_items * (worker + 1) / n_workers;
   const int n_my = (int)(i1 - i0);                 // items of this pair
   const int grp0 = (int)(i0 / p.n_tp), tp0 = (int)(i0 % p.n_tp);
@@ -213,7 +195,7 @@ lbs_fused2_kernel(const __grid_constant__ Params p, const __grid_constant__ CUte
       uint32_t stage = 0, phase = 0, fph = 0;
       int grp = grp0, tp = tp0;
       for (int it = 0; it < n_my; ++it, advance(grp, tp)) {
-        const int tile = PAIR ? 2 * tp + (int)crank : tp;
+        const int tile = 2 * tp + (int)crank;
         if (it == 0 || tp == 0) {
           ptx::mbar_wait(fempty, fph ^ 1);   // the previous group's blends are done with the operand
           fph ^= 1;
@@ -240,7 +222,7 @@ lbs_fused2_kernel(const __grid_constant__ Params p, const __grid_constant__ CUte
       uint32_t stage = 0, phase = 0, tc = 0;
       int grp = grp0, tp = tp0;
       for (int it = 0; it < n_my; ++it, ++tc, advance(grp, tp)) {
-        const int tile = PAIR ? 2 * tp + (int)crank : tp;
+        const int tile = 2 * tp + (int)crank;
         const uint32_t wb = tc % WBUFS;
         ptx::mbar_wait(wempty(wb), ((tc / WBUFS) & 1) ^ 1);
         if (ptx::elect_one()) {
@@ -331,17 +313,14 @@ lbs_fused2_kernel(const __grid_constant__ Params p, const __grid_constant__ CUte
     const int set = (warp - 4) >> 2;
     const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
     const size_t pstride = (size_t)p.V * 3;
-    const uint32_t l_tempty0 = PAIR ? ptx::mapa(tempty(0), 0) : tempty(0), l_dempty = PAIR ? ptx::mapa(dempty, 0) : dempty;
-    auto arrive = [&](uint32_t b) { if (PAIR) ptx::mbar_arrive_cluster(b); else ptx::mbar_arrive(b); };
-    float* stg = reinterpret_cast<float*>(smem + L::OFF_STG) + (warp - 4) * CP * 96;   // [CP poses][96 floats]
+    const uint32_t l_tempty0 = ptx::mapa(tempty(0), 0), l_dempty = ptx::mapa(dempty, 0);
+    auto arrive = [&](uint32_t b) { ptx::mbar_arrive_cluster(b); };
     uint32_t dph = 0, tc = 0;
     int grp = grp0, tp = tp0;
     for (int it = 0; it < n_my; ++it, ++tc, advance(grp, tp)) {
-      const int tile = PAIR ? 2 * tp + (int)crank : tp;
+      const int tile = 2 * tp + (int)crank;
       const int v0 = tile * TILE_V + q * 32;
       const int v = v0 + lane;
-      const bool full_rows = v0 + 32 <= p.V;
-      const int n_floats = max(0, min(32, p.V - v0)) * 3;
       // this set's chunks of the tile are set, set+3, ...: with NSETS == NT they all use T buffer (tc*NCH + set) % NT
       // shifted by nothing, and the barrier phase flips once per chunk
       uint32_t cc = tc * NCH + set;
@@ -396,42 +375,7 @@ lbs_fused2_kernel(const __grid_constant__ Params p, const __grid_constant__ CUte
           o[i][1] = fmaf(T[3], x, fmaf(T[4], y, fmaf(T[5], z, T[10])));
           o[i][2] = fmaf(T[6], x, fmaf(T[7], y, fmaf(T[8], z, T[11])));
         }
-        if (STAGED) {
-          // transpose through shared memory: lane l holds vertex l's (x,y,z); memory wants, per pose, 96 consecutive
-          // floats -> 3 conflict-free STS, 3 LDS and 3 full-line STG per pose, all CP poses in flight together
-          __syncwarp();                       // the previous chunk's LDS are done before its buffer is overwritten
-#pragma unroll
-          for (int i = 0; i < CP; ++i) {
-            stg[i * 96 + 3 * lane + 0] = o[i][0];
-            stg[i * 96 + 3 * lane + 1] = o[i][1];
-            stg[i * 96 + 3 * lane + 2] = o[i][2];
-          }
-          __syncwarp();
-          float r[CP][3];
-#pragma unroll
-          for (int i = 0; i < CP; ++i)
-#pragma unroll
-            for (int k = 0; k < 3; ++k) r[i][k] = stg[i * 96 + 32 * k + lane];
-          float* dst = p.verts + (size_t)b0 * pstride + (size_t)v0 * 3 + lane;
-          if (n_ok == CP && full_rows) {
-#pragma unroll
-            for (int i = 0; i < CP; ++i) {
-              float* w = dst + (size_t)i * pstride;
-              w[0] = r[i][0];
-              w[32] = r[i][1];
-              w[64] = r[i][2];
-            }
-          } else {
-#pragma unroll
-            for (int i = 0; i < CP; ++i)
-              if (i < n_ok) {
-                float* w = dst + (size_t)i * pstride;
-#pragma unroll
-                for (int k = 0; k < 3; ++k)
-                  if (32 * k + lane < n_floats) w[32 * k] = r[i][k];
-              }
-          }
-        } else if (v < p.V) {
+        if (v < p.V) {
           // each lane stores its vertex's 12 bytes; the warp's 32 records are one contiguous 384-byte run
           float* dst = p.verts + (size_t)b0 * pstride + (size_t)v * 3;
 #pragma unroll
@@ -451,19 +395,19 @@ lbs_fused2_kernel(const __grid_constant__ Params p, const __grid_constant__ CUte
   ptx::cluster_sync();       // no CTA leaves while the peer may still arrive on its barriers / read its operands
   if (warp == 2) {
     ptx::tc_fence_after();
-    if (PAIR) ptx::tmem_dealloc_2sm(tmem_base, 512);
-    else ptx::tmem_dealloc(tmem_base, 512);
+    ptx::tmem_dealloc_2sm(tmem_base, 512);
   }
 }
 
 }  // namespace lt2
 
+// Two skinning K slabs (jp = 64: SMPL-X with the const tail).  Measured (profiles/r2_lbs_fused3_experiments.md): the
+// 96-pose-group kernel wins there, its three T buffers hide the longer chunks; lbs_fused3 wins for one slab (jp = 32).
 bool lbs_fused2_fits(const dpb_lbs* h, const LbsVariant& v) {
   if (!h->tc_ready || !v.dirs16) return false;
   if (v.kext != 448) return false;                      // instantiated for a 224-wide blend K (SMPL; SMPL-X const tail)
   if (h->J >= h->jp) return false;                      // needs the spare joint slot for the translation
-  if (h->jp != 32 && h->jp != 64) return false;
-  return true;
+  return h->jp == 64;
 }
 
 // verts[B,V,3] = skinned vertices.  featop [B_pad, kext] and skinop [B_pad*12, 2*jp] were written by the pose kernel.
@@ -471,44 +415,26 @@ int lbs_fused2(dpb_lbs* h, const LbsVariant& v, __half* featop, __half* skinop, 
                cudaStream_t st) {
   const int K2 = v.kext, Jp = h->jp;
   const int64_t B_pad = (B + 127) / 128 * 128;          // rows that physically exist (lbs_tc_ws_bytes); TMA zero-fills beyond
-  const int pair = getenv("DPB_LBS_PAIR") ? atoi(getenv("DPB_LBS_PAIR")) : 1;       // A/B timing only (read per call)
-  const int staged = getenv("DPB_LBS_STAGED") ? atoi(getenv("DPB_LBS_STAGED")) : 0;
   CUtensorMap tm_feat, tm_s;
-  int rc = make_tmap_2d(&tm_feat, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, featop, K2, (uint64_t)B_pad, lt2::BK,
-                        pair ? lt2::NP / 2 : lt2::NP, 2);
+  int rc = make_tmap_2d(&tm_feat, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, featop, K2, (uint64_t)B_pad, lt2::BK, lt2::NP / 2, 2);
   if (rc == DPB_OK)
     rc = make_tmap_2d(&tm_s, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, skinop, 2 * Jp, (uint64_t)B_pad * 12, lt2::BK,
-                      pair ? lt2::NS / 2 : lt2::NS, 2);
+                      lt2::NS / 2, 2);
   if (rc != DPB_OK) return rc;
   lt2::Params p{};
   p.V = h->V;
   p.V_pad = h->n_cols_pad;
-  p.n_tp = h->n_cols_pad / lt2::TILE_V / (pair ? 2 : 1);
+  p.n_tp = h->n_cols_pad / lt2::TILE_V / 2;
   p.B = B;
   p.n_items = (long long)((B + lt2::NP - 1) / lt2::NP) * p.n_tp;
   p.verts = verts;
   p.debug = getenv("DPB_LBS_DEBUG") ? atoi(getenv("DPB_LBS_DEBUG")) : 0;
-  void (*kern)(lt2::Params, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap) = nullptr;
-  size_t smem = 0;
-#define DPB_PICK(JS_, JSL_, AS_, SS_, WB_, PAIR_)                                                        \
-  do {                                                                                                   \
-    kern = staged ? lt2::lbs_fused2_kernel<14, 7, JS_, JSL_, AS_, SS_, WB_, true, PAIR_>                 \
-                  : lt2::lbs_fused2_kernel<14, 7, JS_, JSL_, AS_, SS_, WB_, false, PAIR_>;               \
-    smem = lt2::Smem<JSL_, AS_, SS_, WB_, PAIR_>::BYTES;                                                  \
-  } while (0)
-  if (Jp == 32) {
-    if (pair) DPB_PICK(2, 1, 5, 10, 2, true);
-    else DPB_PICK(2, 1, 4, 4, 1, false);        // F 84 KB + A 64 + W 16 + S 32 + staging 23
-  } else {
-    if (pair) DPB_PICK(4, 2, 4, 6, 1, true);
-    else DPB_PICK(4, 2, 3, 2, 1, false);        // F 84 KB + A 48 + W 32 + S 32 + staging 23
-  }
-#undef DPB_PICK
+  auto kern = lt2::lbs_fused2_kernel<14, 7, 4, 2, 4, 6, 1>;
+  const size_t smem = lt2::Smem<2, 4, 6, 1>::BYTES;
   DPB_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int grid = h->sm_count & ~1;                                   // whole clusters of two
   const long long max_workers = p.n_items < 1 ? 1 : p.n_items;
-  const long long per = pair ? 2 : 1;
-  if (grid / per > max_workers) grid = (int)((per * max_workers + 1) & ~1LL);
+  if (grid / 2 > max_workers) grid = (int)(2 * max_workers);
   kern<<<grid, lt2::NUM_THREADS, smem, st>>>(p, v.tm_dirs, tm_feat, h->tm_wop, tm_s);
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;

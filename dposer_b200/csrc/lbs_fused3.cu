@@ -379,11 +379,13 @@ lbs_fused3_kernel(const __grid_constant__ Params p, const __grid_constant__ CUte
 
 }  // namespace lt3
 
+// One skinning K slab (jp = 32: SMPL).  Measured (profiles/r2_lbs_fused3_experiments.md): the 128-pose-group kernel
+// wins there; lbs_fused2 wins for two slabs (jp = 64).
 bool lbs_fused3_fits(const dpb_lbs* h, const LbsVariant& v) {
   if (!h->tc_ready || !v.dirs16) return false;
   if (v.kext != 448) return false;                      // instantiated for a 224-wide blend K (SMPL; SMPL-X const tail)
   if (h->J >= h->jp) return false;                      // needs the spare joint slot for the translation
-  if (h->jp != 32 && h->jp != 64) return false;
+  if (h->jp != 32) return false;
   if ((h->n_cols_pad / lt3::TILE_V) % 2) return false;  // whole tile pairs
   return true;
 }
@@ -407,15 +409,8 @@ int lbs_fused3(dpb_lbs* h, const LbsVariant& v, __half* featop, __half* skinop, 
   p.n_items = (long long)((B + lt3::NP - 1) / lt3::NP) * p.n_tp;
   p.verts = verts;
   p.debug = getenv("DPB_LBS_DEBUG") ? atoi(getenv("DPB_LBS_DEBUG")) : 0;
-  void (*kern)(lt3::Params, CUtensorMap, CUtensorMap, CUtensorMap, CUtensorMap) = nullptr;
-  size_t smem = 0;
-  if (Jp == 32) {
-    kern = lt3::lbs_fused3_kernel<14, 7, 2, 1, 6, 8>;   // F 56 KB + A 96 + W 32 + S 32
-    smem = lt3::Smem<1, 6, 8>::BYTES;
-  } else {
-    kern = lt3::lbs_fused3_kernel<14, 7, 4, 2, 4, 4>;   // F 56 KB + A 64 + W 64 + S 32
-    smem = lt3::Smem<2, 4, 4>::BYTES;
-  }
+  auto kern = lt3::lbs_fused3_kernel<14, 7, 2, 1, 6, 8>;   // F 56 KB + A 96 + W 32 + S 32
+  const size_t smem = lt3::Smem<1, 6, 8>::BYTES;
   DPB_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   int grid = h->sm_count & ~1;                                   // whole clusters of two
   const long long max_workers = p.n_items < 1 ? 1 : p.n_items;

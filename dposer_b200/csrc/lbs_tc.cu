@@ -19,7 +19,6 @@
 #include <vector>
 
 #include <cmath>
-#include <cstdlib>
 
 #include "lbs.h"
 #include "ptx.cuh"
@@ -597,281 +596,6 @@ __global__ void __launch_bounds__(128) lbs_skinop_kernel(const float* __restrict
   for (int i = lane; i < 3 * Jp; i += 32) dst[i] = src[i];  // 12 rows x 2 Jp halves = 3 Jp vectors of 16 bytes
 }
 
-
-// ------------------------------------------------------------------------------------------------------------
-// Fused blend + skinning (models whose padded joint count fits one 64-wide [hi | lo] slab and whose 128-pose blend
-// operand fits shared memory, i.e. SMPL): the blended vertices never leave the SM.
-//   unit        = (pose group of 128 poses, half of the vertex tiles); the group's blend operand stays in SMEM
-//   per tile    blend MMAs (N = 128) -> D_x | D_y | D_z in TMEM columns 0..383 (single buffer)
-//               then 26 chunks of 5 poses: T[v, (pose, e)] = sum_j w[v,j] A[pose,j,e] as 6 MMAs with N = 64 into one
-//               of two 64-column buffers (columns 384..511); warp set h = chunk & 1 owns buffer h
-//   epilogue    thread = vertex: T (60 columns) and the chunk's 5 x (x,y,z) of D -> skinned vertex -> staged,
-//               coalesced stores.  The tile's blend accumulators are released after the last chunk.
-//   warp 0  TMA: blend operand (per unit), basis slabs (ring);  warp 3  TMA: skin weights (per tile), transform chunks
-//   warp 1  MMA issuer;  warp 2  TMEM allocator;  warps 4-11 epilogue (warp set h = (warp - 4) >> 2)
-// HBM traffic is the output only (5.4 GB for 65 536 SMPL poses instead of 16.4 GB through the two-kernel path).
-constexpr int FU_NP = 128;                 // poses per group: D_x | D_y | D_z take 384 TMEM columns, two 64-column T
-                                           // buffers the rest.  Measured: 96 poses / three T buffers / 6-stage ring 3.44 ms,
-                                           // 128 poses / two T buffers / 4-stage ring 3.30 ms (an M = 128 MMA costs about
-                                           // 32 + N/4 cycles of operand fetch, so the blend is cheapest per pose at N = 128)
-constexpr int FU_CP = 5;                   // poses per skinning chunk (N = 60 -> 64)
-constexpr int FU_NCHUNK = (FU_NP + FU_CP - 1) / FU_CP;   // 26 (even: chunk parity = warp set across tiles)
-constexpr int FU_NT = 2;                   // T buffers (ring over chunks)
-constexpr int FU_ASTAGES = 4;
-constexpr int FU_SSTAGES = 3;
-constexpr int FU_S_BYTES = 64 * BK * 2;    // one transform chunk: 64 rows x 64 k fp16
-constexpr int FU_B_SLAB = FU_NP * BK * 2;
-constexpr uint32_t FU_IDESC_BLEND = ptx::umma_idesc_f16(TILE_V, FU_NP, 0);
-constexpr uint32_t FU_IDESC_SKIN = ptx::umma_idesc_f16(TILE_V, 64, 0);
-constexpr int FU_NBARS = 2 * FU_ASTAGES + 2 * FU_SSTAGES + 6 + 2 * FU_NT;
-static_assert(FU_NCHUNK % 2 == 0 && 3 * FU_NP + FU_NT * 64 <= 512 && FU_B_SLAB % 1024 == 0, "fused LBS TMEM / SMEM layout");
-
-struct FusedParams {
-  int V, V_pad, n_vt, vsplit;
-  int ksteps_half, n_slabs;   // blend K (as KParams)
-  int jsteps;                 // K16 steps of the hi part of the skinning K: Jp / 16
-  int64_t B;
-  int n_units;                // pose groups x vsplit
-  const float* v_template;
-  float* verts;
-};
-
-// HALF = K16 steps of the hi part of the blend K, NSLABS = 64-wide slabs of [hi | lo], JS = K16 steps of the hi part of
-// the skinning K: compile-time so that the issuer's loops unroll and every descriptor is base + constant (with
-// run-time geometry the single issuing thread spent ~100 cycles of address arithmetic per 48-cycle MMA).
-template <int HALF, int NSLABS, int JS>
-__global__ void __launch_bounds__(NUM_THREADS, 1)
-lbs_fused_tc_kernel(const __grid_constant__ FusedParams p, const __grid_constant__ CUtensorMap tm_dirs,
-                    const __grid_constant__ CUtensorMap tm_feat, const __grid_constant__ CUtensorMap tm_w,
-                    const __grid_constant__ CUtensorMap tm_s) {
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = smem_raw + ((1024u - (ptx::smem_u32(smem_raw) & 1023u)) & 1023u);
-  const uint32_t smem_base = ptx::smem_u32(smem);
-  const uint32_t b_base = smem_base;                                   // resident blend operand
-  const uint32_t a_base = b_base + p.n_slabs * FU_B_SLAB;              // basis slab ring
-  const uint32_t w_base = a_base + FU_ASTAGES * A_SLAB;                // skin weights of the current tile
-  const uint32_t s_base = w_base + A_SLAB;                             // transform chunk ring
-  const uint32_t bar_base = s_base + FU_SSTAGES * FU_S_BYTES;
-  auto afull = [&](uint32_t s) { return bar_base + 8u * s; };
-  auto aempty = [&](uint32_t s) { return bar_base + 8u * (FU_ASTAGES + s); };
-  auto sfull = [&](uint32_t s) { return bar_base + 8u * (2 * FU_ASTAGES + s); };
-  auto sempty = [&](uint32_t s) { return bar_base + 8u * (2 * FU_ASTAGES + FU_SSTAGES + s); };
-  const uint32_t bar2 = bar_base + 8u * (2 * FU_ASTAGES + 2 * FU_SSTAGES);
-  const uint32_t bfull = bar2, bempty = bar2 + 8, wfull = bar2 + 16, wempty = bar2 + 24, dfull = bar2 + 32,
-                 dempty = bar2 + 40;
-  auto tfull = [&](uint32_t b) { return bar2 + 48 + 8u * b; };
-  auto tempty = [&](uint32_t b) { return bar2 + 48 + 8u * (FU_NT + b); };
-  const size_t off_bar = (size_t)p.n_slabs * FU_B_SLAB + FU_ASTAGES * A_SLAB + A_SLAB + FU_SSTAGES * FU_S_BYTES;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(smem + off_bar + FU_NBARS * 8);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  if (threadIdx.x == 0) {
-    for (int s = 0; s < FU_ASTAGES; ++s) { ptx::mbar_init(afull(s), 1); ptx::mbar_init(aempty(s), 1); }
-    for (int s = 0; s < FU_SSTAGES; ++s) { ptx::mbar_init(sfull(s), 1); ptx::mbar_init(sempty(s), 1); }
-    ptx::mbar_init(bfull, 1); ptx::mbar_init(bempty, 1);
-    ptx::mbar_init(wfull, 1); ptx::mbar_init(wempty, 1);
-    ptx::mbar_init(dfull, 1); ptx::mbar_init(dempty, 8);
-    for (int b = 0; b < FU_NT; ++b) { ptx::mbar_init(tfull(b), 1); ptx::mbar_init(tempty(b), 4); }
-    ptx::fence_barrier_init();
-  }
-  if (warp == 2) ptx::tmem_alloc(ptx::smem_u32(tmem_slot), 512);
-  ptx::tc_fence_before();
-  __syncthreads();
-  ptx::tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const int tiles_per_part = (p.n_vt + p.vsplit - 1) / p.vsplit;
-
-  if (warp == 0) {
-    // ---- blend operand + basis slabs
-    if (lane == 0) { ptx::prefetch_tmap(&tm_dirs); ptx::prefetch_tmap(&tm_feat); }
-    __syncwarp();
-    uint32_t stage = 0, phase = 0, uph = 0;
-    for (int u = blockIdx.x; u < p.n_units; u += gridDim.x) {
-      const int grp = u / p.vsplit, part = u % p.vsplit;
-      const int vt0 = part * tiles_per_part, vt1 = min(p.n_vt, vt0 + tiles_per_part);
-      ptx::mbar_wait(bempty, uph ^ 1);
-      if (ptx::elect_one()) {
-        ptx::mbar_arrive_expect_tx(bfull, (uint32_t)p.n_slabs * FU_B_SLAB);
-        for (int i = 0; i < p.n_slabs; ++i) ptx::tma_load_2d(b_base + i * FU_B_SLAB, &tm_feat, bfull, i * BK, grp * FU_NP);
-      }
-      uph ^= 1;
-      for (int vt = vt0; vt < vt1; ++vt)
-        for (int c = 0; c < 3; ++c)
-          for (int i = 0; i < p.n_slabs; ++i) {
-            ptx::mbar_wait(aempty(stage), phase ^ 1);
-            if (ptx::elect_one()) {
-              ptx::mbar_arrive_expect_tx(afull(stage), A_SLAB);
-              ptx::tma_load_2d(a_base + stage * A_SLAB, &tm_dirs, afull(stage), i * BK, c * p.V_pad + vt * TILE_V);
-            }
-            if (++stage == FU_ASTAGES) { stage = 0; phase ^= 1; }
-          }
-    }
-  } else if (warp == 3) {
-    // ---- skin weights (per tile) + transform chunks
-    if (lane == 0) { ptx::prefetch_tmap(&tm_w); ptx::prefetch_tmap(&tm_s); }
-    __syncwarp();
-    uint32_t stage = 0, phase = 0, wph = 0;
-    for (int u = blockIdx.x; u < p.n_units; u += gridDim.x) {
-      const int grp = u / p.vsplit, part = u % p.vsplit;
-      const int vt0 = part * tiles_per_part, vt1 = min(p.n_vt, vt0 + tiles_per_part);
-      for (int vt = vt0; vt < vt1; ++vt) {
-        ptx::mbar_wait(wempty, wph ^ 1);
-        if (ptx::elect_one()) {
-          ptx::mbar_arrive_expect_tx(wfull, A_SLAB);
-          ptx::tma_load_2d(w_base, &tm_w, wfull, 0, vt * TILE_V);
-        }
-        wph ^= 1;
-        for (int c = 0; c < FU_NCHUNK; ++c) {
-          ptx::mbar_wait(sempty(stage), phase ^ 1);
-          if (ptx::elect_one()) {
-            ptx::mbar_arrive_expect_tx(sfull(stage), FU_S_BYTES);
-            ptx::tma_load_2d(s_base + stage * FU_S_BYTES, &tm_s, sfull(stage), 0, (grp * FU_NP + c * FU_CP) * 12);
-          }
-          if (++stage == FU_SSTAGES) { stage = 0; phase ^= 1; }
-        }
-      }
-    }
-  } else if (warp == 1) {
-    // ---- MMA issuer
-    uint32_t astage = 0, aphase = 0, sstage = 0, sphase = 0, uph = 0, wph = 0, dph = 0, cc = 0;   // cc: chunks so far
-    const uint64_t adesc0 = ptx::umma_desc_sw128(a_base), bdesc0 = ptx::umma_desc_sw128(b_base);
-    const uint64_t wdesc0 = ptx::umma_desc_sw128(w_base);
-    for (int u = blockIdx.x; u < p.n_units; u += gridDim.x) {
-      const int part = u % p.vsplit;
-      const int vt0 = part * tiles_per_part, vt1 = min(p.n_vt, vt0 + tiles_per_part);
-      ptx::mbar_wait(bfull, uph);
-      uph ^= 1;
-      ptx::tc_fence_after();
-      for (int vt = vt0; vt < vt1; ++vt) {
-        ptx::mbar_wait(dempty, dph ^ 1);   // the previous tile's epilogue has read all of D
-        dph ^= 1;
-        ptx::tc_fence_after();
-#pragma unroll 1
-        for (int c = 0; c < 3; ++c) {
-          const uint32_t taddr = tmem_base + c * FU_NP;
-#pragma unroll
-          for (int i = 0; i < NSLABS; ++i) {
-            ptx::mbar_wait(afull(astage), aphase);
-            ptx::tc_fence_after();
-            const uint64_t adesc = adesc0 + (uint64_t)(astage * (A_SLAB >> 4));
-            if (ptx::elect_one()) {
-#pragma unroll
-              for (int j = 0; j < BK / 16; ++j) {
-                constexpr int SL = FU_B_SLAB >> 4;
-                const int g = i * (BK / 16) + j;   // compile-time after unrolling
-                if (g < HALF) {
-                  ptx::mma_f16_ss(taddr, adesc + 2 * j, bdesc0 + (uint64_t)((g >> 2) * SL + 2 * (g & 3)), FU_IDESC_BLEND,
-                                  g != 0 ? 1u : 0u);
-                  ptx::mma_f16_ss(taddr, adesc + 2 * j,
-                                  bdesc0 + (uint64_t)(((HALF + g) >> 2) * SL + 2 * ((HALF + g) & 3)), FU_IDESC_BLEND, 1u);
-                } else {
-                  ptx::mma_f16_ss(taddr, adesc + 2 * j,
-                                  bdesc0 + (uint64_t)(((g - HALF) >> 2) * SL + 2 * ((g - HALF) & 3)), FU_IDESC_BLEND, 1u);
-                }
-              }
-              ptx::mma_commit(aempty(astage));
-              if (c == 2 && i == NSLABS - 1) ptx::mma_commit(dfull);
-            }
-            if (++astage == FU_ASTAGES) { astage = 0; aphase ^= 1; }
-          }
-        }
-        ptx::mbar_wait(wfull, wph);
-        wph ^= 1;
-        ptx::tc_fence_after();
-        for (int c = 0; c < FU_NCHUNK; ++c, ++cc) {
-          const uint32_t buf = cc % FU_NT;
-          ptx::mbar_wait(tempty(buf), ((cc / FU_NT) & 1) ^ 1);
-          ptx::mbar_wait(sfull(sstage), sphase);
-          ptx::tc_fence_after();
-          const uint32_t taddr = tmem_base + 3 * FU_NP + buf * 64;
-          const uint64_t sdesc0 = ptx::umma_desc_sw128(s_base + sstage * FU_S_BYTES);
-          if (ptx::elect_one()) {
-#pragma unroll
-            for (int g = 0; g < JS; ++g) {   // w_hi x (A_hi + A_lo), then w_lo x A_hi
-              ptx::mma_f16_ss(taddr, wdesc0 + 2 * g, sdesc0 + 2 * g, FU_IDESC_SKIN, g ? 1u : 0u);
-              ptx::mma_f16_ss(taddr, wdesc0 + 2 * g, sdesc0 + 2 * (JS + g), FU_IDESC_SKIN, 1u);
-              ptx::mma_f16_ss(taddr, wdesc0 + 2 * (JS + g), sdesc0 + 2 * g, FU_IDESC_SKIN, 1u);
-            }
-            ptx::mma_commit(sempty(sstage));
-            ptx::mma_commit(tfull(buf));
-            if (c == FU_NCHUNK - 1) {
-              ptx::mma_commit(wempty);
-              if (vt == vt1 - 1) ptx::mma_commit(bempty);
-            }
-          }
-          if (++sstage == FU_SSTAGES) { sstage = 0; sphase ^= 1; }
-        }
-      }
-    }
-  } else if (warp >= 4) {
-    // ---- epilogue
-    const int q = warp & 3;
-    const int h = (warp - 4) >> 2;     // warp set = T buffer = chunk parity
-    const uint32_t lane_addr = (uint32_t)(q * 32) << 16;
-    const size_t pstride = (size_t)p.V * 3;
-    uint32_t dph = 0, cc0 = 0;         // cc0: chunk counter at the start of the tile (the MMA warp's cc)
-    for (int u = blockIdx.x; u < p.n_units; u += gridDim.x) {
-      const int grp = u / p.vsplit, part = u % p.vsplit;
-      const int vt0 = part * tiles_per_part, vt1 = min(p.n_vt, vt0 + tiles_per_part);
-      for (int vt = vt0; vt < vt1; ++vt) {
-        const int v0 = vt * TILE_V + q * 32;
-        const int v = v0 + lane;
-        const int n_floats = max(0, min(32, p.V - v0)) * 3;
-        float vt3[3] = {0.f, 0.f, 0.f};   // v_template rides in the GEMM (K slot S+P, feature 1)
-        if (p.v_template && v < p.V) { vt3[0] = p.v_template[v * 3]; vt3[1] = p.v_template[v * 3 + 1]; vt3[2] = p.v_template[v * 3 + 2]; }
-        ptx::mbar_wait(dfull, dph);
-        dph ^= 1;
-        ptx::tc_fence_after();
-#pragma unroll 1
-        for (int c = h; c < FU_NCHUNK; c += 2) {
-          const uint32_t cc = cc0 + c, buf = cc % FU_NT;
-          ptx::mbar_wait(tfull(buf), (cc / FU_NT) & 1);
-          ptx::tc_fence_after();
-          uint32_t t[64], dx[8], dy[8], dz[8];
-          const uint32_t d0 = tmem_base + lane_addr + c * FU_CP;
-          ptx::tmem_ld_32x64(tmem_base + lane_addr + 3 * FU_NP + buf * 64, t);
-          ptx::tmem_ld_32x8(d0, dx);
-          ptx::tmem_ld_32x8(d0 + FU_NP, dy);
-          ptx::tmem_ld_32x8(d0 + 2 * FU_NP, dz);
-          ptx::tmem_ld_wait();
-          ptx::tc_fence_before();
-          __syncwarp();
-          if (lane == 0) ptx::mbar_arrive(tempty(buf));
-          const int64_t b0 = (int64_t)grp * FU_NP + c * FU_CP;
-          int n_ok = FU_NP - c * FU_CP;                       // poses of this chunk inside the group ...
-          if (n_ok > FU_CP) n_ok = FU_CP;
-          if (b0 + n_ok > p.B) n_ok = (int)max((int64_t)0, p.B - b0);   // ... and inside the batch
-          // each lane stores its vertex's 12 bytes; the warp's 32 records are one contiguous 384-byte run
-          if (v < p.V) {
-            float* dst = p.verts + (size_t)b0 * pstride + (size_t)v * 3;
-#pragma unroll
-            for (int i = 0; i < FU_CP; ++i) {
-              if (i < n_ok) {
-                const float* T = reinterpret_cast<const float*>(t) + i * 12;
-                const float x = __uint_as_float(dx[i]) + vt3[0], y = __uint_as_float(dy[i]) + vt3[1],
-                            z = __uint_as_float(dz[i]) + vt3[2];
-                float* w = dst + (size_t)i * pstride;
-                w[0] = T[0] * x + T[1] * y + T[2] * z + T[9];
-                w[1] = T[3] * x + T[4] * y + T[5] * z + T[10];
-                w[2] = T[6] * x + T[7] * y + T[8] * z + T[11];
-              }
-            }
-          }
-        }
-        cc0 += FU_NCHUNK;
-        ptx::tc_fence_before();
-        __syncwarp();
-        if (lane == 0) ptx::mbar_arrive(dempty);
-      }
-    }
-  }
-  __syncthreads();
-  if (warp == 2) {
-    ptx::tc_fence_after();
-    ptx::tmem_dealloc(tmem_base, 512);
-  }
-}
-
 }  // namespace ltc
 
 int lbs_tc_prepare(dpb_lbs* h, const dpb_body_tensors* m) {
@@ -1087,54 +811,6 @@ int lbs_tc_skin_adjoint(dpb_lbs* h, const float* A, __half* skinop, const float*
   return DPB_OK;
 }
 
-bool lbs_tc_fused_fits(const dpb_lbs* h) {
-  if (!h->tc_ready || h->J >= h->jp || 2 * h->jp != ltc::BK) return false;   // one [hi | lo] slab incl. the transl slot
-  if (h->kext != 448) return false;   // the kernel is instantiated for SMPL's blend K (10 + 207 -> 224, hi | lo)
-  const int n_slabs = h->kext / ltc::BK;
-  const size_t smem = (size_t)n_slabs * ltc::FU_B_SLAB + (ltc::FU_ASTAGES + 1) * ltc::A_SLAB +
-                      ltc::FU_SSTAGES * ltc::FU_S_BYTES + ltc::FU_NBARS * 8 + 16 + 1024;
-  return smem <= 232448;
-}
-
-// verts[B,V,3] = skinned vertices, blend and skinning in one kernel (see lbs_fused_tc_kernel)
-int lbs_tc_fused(dpb_lbs* h, const float* betas, const float* feat, __half* featop, const float* A, const float* transl,
-                 __half* skinop, float* verts, int64_t B, cudaStream_t st) {
-  const int K2 = h->kext, Kp = K2 / 2, Jp = h->jp;
-  const int64_t B_pad = (B + ltc::PAD_POSES - 1) / ltc::PAD_POSES * ltc::PAD_POSES;
-  if (feat && A) {   // operands not already written by the pose kernel
-    const int64_t n = B_pad * Kp;
-    ltc::lbs_featop_kernel<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(betas, feat, h->S, h->P, h->P, Kp, featop, B, B_pad);
-    const int64_t n2 = B_pad * 12 * Jp;
-    ltc::lbs_skinop_kernel<<<(unsigned)((B_pad + 3) / 4), 128, 0, st>>>(A, transl, h->J, Jp, skinop, B, B_pad);
-    DPB_CUDA_CHECK(cudaGetLastError());
-  }
-  CUtensorMap tm_feat, tm_s;
-  int rc = make_tmap_2d(&tm_feat, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, featop, K2, (uint64_t)B_pad, ltc::BK, ltc::FU_NP, 2);
-  if (rc == DPB_OK)
-    rc = make_tmap_2d(&tm_s, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, skinop, 2 * Jp, (uint64_t)B_pad * 12, ltc::BK, 64, 2);
-  if (rc != DPB_OK) return rc;
-  ltc::FusedParams p{};
-  p.V = h->V;
-  p.V_pad = h->n_cols_pad;
-  p.n_vt = h->n_cols_pad / ltc::TILE_V;
-  p.vsplit = 2;
-  p.ksteps_half = Kp / 16;
-  p.n_slabs = K2 / ltc::BK;
-  p.jsteps = Jp / 16;
-  p.B = B;
-  p.n_units = (int)((B + ltc::FU_NP - 1) / ltc::FU_NP) * p.vsplit;
-  p.v_template = nullptr;   // folded into the GEMM
-  p.verts = verts;
-  const size_t smem = (size_t)p.n_slabs * ltc::FU_B_SLAB + (ltc::FU_ASTAGES + 1) * ltc::A_SLAB +
-                      ltc::FU_SSTAGES * ltc::FU_S_BYTES + ltc::FU_NBARS * 8 + 16 + 1024;
-  auto kern = ltc::lbs_fused_tc_kernel<14, 7, 2>;   // SMPL: K16 steps 224/16, slabs 448/64, joints 32/16
-  DPB_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-  const int grid = p.n_units < h->sm_count ? p.n_units : h->sm_count;
-  kern<<<grid, ltc::NUM_THREADS, smem, st>>>(p, h->tm_dirs, tm_feat, h->tm_wop, tm_s);
-  DPB_CUDA_CHECK(cudaGetLastError());
-  return DPB_OK;
-}
-
 // writes v_posed (template + shape blend + pose blend) into verts[B,V,3]
 int lbs_tc_blend(dpb_lbs* h, const LbsVariant& var, const float* betas, const float* feat, __half* featop, float* verts,
                  int64_t B, cudaStream_t st) {
@@ -1148,8 +824,7 @@ int lbs_tc_blend(dpb_lbs* h, const LbsVariant& var, const float* betas, const fl
   const int n_slabs = K2 / ltc::BK;
   const size_t bars = (2 * ltc::MAX_STAGES + 6) * 8 + 16 + 8 * ltc::XSTAGE * 4 + 1024;
   // 128-pose groups when the group's operand leaves room for >= 4 ring stages (SMPL), else 64 (SMPL-X)
-  int np = ((size_t)n_slabs * 128 * ltc::BK * 2 + 4 * ltc::A_SLAB + bars <= 232448) ? 128 : 64;
-  if (const char* e = getenv("DPB_LBS_NP")) np = atoi(e) == 64 ? 64 : np;   // timing experiments only
+  const int np = ((size_t)n_slabs * 128 * ltc::BK * 2 + 4 * ltc::A_SLAB + bars <= 232448) ? 128 : 64;
   CUtensorMap tm_feat;
   int rc = make_tmap_2d(&tm_feat, CU_TENSOR_MAP_DATA_TYPE_FLOAT16, featop, K2, (uint64_t)B_pad, ltc::BK, np, 2);
   if (rc != DPB_OK) return rc;
@@ -1173,8 +848,7 @@ int lbs_tc_blend(dpb_lbs* h, const LbsVariant& var, const float* betas, const fl
   // instantiations with compile-time K geometry for the two body models, run-time geometry otherwise
   void (*kern)(ltc::KParams, CUtensorMap, CUtensorMap) = nullptr;
   if (np == 128) kern = (K2 == 448) ? ltc::lbs_blend_tc_kernel<128, 14, 7> : ltc::lbs_blend_tc_kernel<128>;
-  else kern = (K2 == 1024) ? ltc::lbs_blend_tc_kernel<64, 32, 16>
-            : (K2 == 448) ? ltc::lbs_blend_tc_kernel<64, 14, 7> : ltc::lbs_blend_tc_kernel<64>;
+  else kern = (K2 == 1024) ? ltc::lbs_blend_tc_kernel<64, 32, 16> : ltc::lbs_blend_tc_kernel<64>;
   DPB_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   kern<<<grid, ltc::NUM_THREADS, smem, st>>>(p, var.tm_dirs, tm_feat);
   DPB_CUDA_CHECK(cudaGetLastError());

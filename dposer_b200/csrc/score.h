@@ -34,13 +34,8 @@ struct dpb_score {
   __half* act_h = nullptr;      // [slots*128, 1024] residual stream
   __half* act_t = nullptr;      // [slots*128, 1024] block intermediate
   CUtensorMap tm_act_h, tm_act_t;  // box {64, 128}
-  // small-batch engine (score_small.cu): the same operands with 64-row boxes (one column slice per CTA)
-  CUtensorMap tms_w[4], tms_post, tms_pre;
-  bool tcs_ready = false;
   float* pc_buf = nullptr;      // predictor-corrector mode: [2 * PC_MAX_STEPS] batch norm sums + one int barrier counter
   int tc_slots = 0;
-  size_t act_bytes = 0, l2_window = 0;   // activation scratch size; bytes of the persisting-L2 access-policy window (0 = off)
-  float l2_hit = 1.f;
   float* gn_tc = nullptr;       // [5][2][1024] gamma | beta as staged by the tcgen05 epilogue
   int* tc_flags = nullptr;      // [slots] hand-off flags of the sampler's segment schedule (score_tc.cu: SegIter)
   void* jvp_ops = nullptr;      // fp16 [hi | lo] weight operands of the tensor-core JVP (jvp_tc.cu), built on first use
@@ -81,8 +76,5 @@ struct TcJob {
 };
 int tc_launch(dpb_score* h, const TcJob& job, cudaStream_t st);
 bool tc_pc_possible(const dpb_score* h, int64_t B, int n_steps);
-int tcs_prepare(dpb_score* h);
-bool tcs_wanted(const dpb_score* h, const TcJob& job);
-int tcs_launch(dpb_score* h, const TcJob& job, cudaStream_t st);
 
 }  // namespace dpb

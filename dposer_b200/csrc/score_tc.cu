@@ -1165,35 +1165,12 @@ int tc_prepare(dpb_score* h, const dpb_score_weights* w) {
   // per-CTA activation scratch (one 128-row slot per SM)
   h->tc_slots = h->sm_count * tc::NSUB;
   const size_t rows = (size_t)h->tc_slots * tc::TILE_M;
-  // one allocation for both halves: a single L2 access-policy window covers the whole scratch
   DPB_CUDA_CHECK(cudaMalloc((void**)&h->act_h, 2 * rows * H * sizeof(__half)));
   h->act_t = h->act_h + rows * H;
   DPB_CUDA_CHECK(cudaMemset(h->act_h, 0, 2 * rows * H * sizeof(__half)));
-  {
-    // The scratch is written and re-read once per layer and never needed in HBM: ask for it to stay in L2
-    // (persisting carve-out + access-policy window on the launch).  profiles/r1_ncu_full_summary_final.md: without
-    // it ~68 % of every activation box was written back to DRAM (1.05 GB per 37 888 rows x 4 steps).
-    cudaDeviceProp prop;
-    DPB_CUDA_CHECK(cudaGetDeviceProperties(&prop, h->device));
-    h->act_bytes = 2 * rows * H * sizeof(__half);
-    h->l2_window = 0;
-    // MEASURED (profiles/r2_sampler_l2_policy.md): reserving the carve-out costs more than it saves -- 535 ms without
-    // it, 565 ms with carve-out + window, 694 ms with the carve-out alone -- so it is opt-in (DPB_TC_L2PERSIST=1 when the
-    // handle is created) and the default leaves L2 to the hardware policy plus evict_last hints on the scratch traffic.
-    const char* e = getenv("DPB_TC_L2PERSIST");
-    if (e && atoi(e) == 1 && prop.persistingL2CacheMaxSize > 0 && prop.accessPolicyMaxWindowSize > 0) {
-      size_t carve = (size_t)prop.persistingL2CacheMaxSize;
-      if (carve > h->act_bytes) carve = h->act_bytes;
-      if (cudaDeviceSetLimit(cudaLimitPersistingL2CacheSize, carve) == cudaSuccess) {
-        h->l2_window = h->act_bytes < (size_t)prop.accessPolicyMaxWindowSize ? h->act_bytes
-                                                                               : (size_t)prop.accessPolicyMaxWindowSize;
-        h->l2_hit = (float)((double)carve / (double)h->l2_window);
-        if (h->l2_hit > 1.f) h->l2_hit = 1.f;
-      } else {
-        cudaGetLastError();
-      }
-    }
-  }
+  // The scratch is written and re-read once per layer and never needed in HBM.  A persisting-L2 carve-out with an
+  // access-policy window on the launch measured slower (profiles/r2_sampler_l2_policy.md: 565 vs 535 ms), so L2 is
+  // left to the hardware policy plus evict_last hints on the scratch traffic.
   {  // gamma | beta of the five GroupNorms as the epilogue stages them (beta halved for the tanh-form SiLU)
     std::vector<float> gn((size_t)NL * 2 * H);
     DPB_CUDA_CHECK(cudaMemcpy(gn.data(), h->gn_packed, gn.size() * sizeof(float), cudaMemcpyDeviceToHost));
@@ -1228,15 +1205,12 @@ int tc_prepare(dpb_score* h, const dpb_score_weights* w) {
                                         tc::Width<DP>::SMEM_BYTES));
   DPB_CUDA_CHECK(cudaMalloc((void**)&h->pc_buf, (2 * PC_MAX_STEPS + 4) * sizeof(float)));
   h->tc_ready = true;
-  // the small-batch engine (score_small.cu) is built for the 63-D network only; 126-D handles always use the kernel above
-  return hd == DPB_POSE_DIM ? tcs_prepare(h) : DPB_OK;
+  return DPB_OK;
 }
 
 // the fused predictor-corrector mode needs every CTA to own one tile for the whole run (grid-wide norms per step)
 bool tc_pc_possible(const dpb_score* h, int64_t B, int n_steps) {
   if (!h->tc_ready || !h->pc_buf || n_steps > PC_MAX_STEPS) return false;
-  const char* e = getenv("DPB_TC_PC");                            // A/B timing: 0 forces the per-step launch sequence
-  if (e && atoi(e) == 0) return false;
   const int64_t n_tiles = (B + tc::TILE_M - 1) / tc::TILE_M;
   const int64_t max_grid = (h->tc_slots / tc::NSUB) / tc::CLUSTER * tc::CLUSTER;
   return (n_tiles + tc::CLUSTER - 1) / tc::CLUSTER * tc::CLUSTER <= max_grid;
@@ -1250,7 +1224,6 @@ void tc_release(dpb_score* h) {
 }
 
 int tc_launch(dpb_score* h, const TcJob& j, cudaStream_t st) {
-  if (!j.pc && tcs_wanted(h, j)) return tcs_launch(h, j, st);   // few row tiles: split the output features over 16 CTAs per tile
   tc::KParams p{};
   p.mode = j.mode;
   p.n_steps = j.pc ? 2 * j.n_steps : j.n_steps;
@@ -1293,19 +1266,6 @@ int tc_launch(dpb_score* h, const TcJob& j, cudaStream_t st) {
     cfg.blockDim = dim3(tc::NUM_THREADS);
     cfg.dynamicSmemBytes = h->pose_dp == DP128 ? tc::Width<DP128>::SMEM_BYTES : tc::Width<DP>::SMEM_BYTES;
     cfg.stream = st;
-    cudaLaunchAttribute attr[1];
-    int n_attr = 0;
-    if (h->l2_window > 0) {
-      attr[0].id = cudaLaunchAttributeAccessPolicyWindow;
-      attr[0].val.accessPolicyWindow.base_ptr = h->act_h;
-      attr[0].val.accessPolicyWindow.num_bytes = h->l2_window;
-      attr[0].val.accessPolicyWindow.hitRatio = h->l2_hit;
-      attr[0].val.accessPolicyWindow.hitProp = cudaAccessPropertyPersisting;
-      attr[0].val.accessPolicyWindow.missProp = cudaAccessPropertyStreaming;
-      n_attr = 1;
-    }
-    cfg.attrs = attr;
-    cfg.numAttrs = n_attr;
     if (h->pose_dp == DP128)
       DPB_CUDA_CHECK(cudaLaunchKernelEx(&cfg, tc::score_tc_kernel<DP128>, p, h->tm_act_h, h->tm_act_t, h->tm_pre,
                                         h->tm_w[0], h->tm_w[1], h->tm_w[2], h->tm_w[3], h->tm_post));

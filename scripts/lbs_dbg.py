@@ -1,12 +1,12 @@
 """Timing experiments on the fused LBS kernel: DPB_LBS_DEBUG masks in ONE process (run under `timeout`).
-usage: python scripts/lbs_dbg.py "0 1 3 5 7 ..." [fused]"""
+usage: python scripts/lbs_dbg.py "0 1 3 5 7 ..."
+"""
 import os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from dposer_b200 import synthetic
 from dposer_b200.body_model import BodyModel
 masks = [int(x) for x in (sys.argv[1] if len(sys.argv) > 1 else '0').split()]
-os.environ['DPB_LBS_FUSED'] = sys.argv[2] if len(sys.argv) > 2 else '3'
 B, mt = 65536, 'smpl'
 bm = BodyModel(synthetic.make_body_tensors(mt), batch_size=B, model_type=mt).cuda()
 inp = {k: v.cuda() for k, v in synthetic.lbs_inputs(B, mt).items()}

@@ -1,4 +1,4 @@
-"""A/B timing of the SMPL-X LBS forward (const-tail): CTA-pair fused kernel vs the two-kernel path."""
+"""Timing of the SMPL-X LBS forward (const tail: the CTA-pair fused kernel)."""
 import os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -20,4 +20,4 @@ with torch.no_grad():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(); bm(**inp); e1.record(); torch.cuda.synchronize()
         best = min(best, e0.elapsed_time(e1))
-print(f'{mt} B={B} fused={os.environ.get("DPB_LBS_FUSED","2")} pair={os.environ.get("DPB_LBS_PAIR","0")} staged={os.environ.get("DPB_LBS_STAGED","1")}: {best:.3f} ms  ({B/best*1e3/1e6:.2f} M poses/s)')
+print(f'{mt} B={B}: {best:.3f} ms  ({B/best*1e3/1e6:.2f} M poses/s)')

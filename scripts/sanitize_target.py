@@ -15,15 +15,11 @@ for mt, B in [('smpl', 200), ('smplx', 130)]:
     bm = BodyModel(synthetic.make_body_tensors(mt), batch_size=B, model_type=mt).cuda()
     inp = {k: v.cuda().requires_grad_(True) for k, v in synthetic.lbs_inputs(B, mt).items()}
     o = bm(**inp); (o.v.sum() + o.Jtr.sum()).backward(); torch.cuda.synchronize(); print('lbs ok', mt)
-# round 2: joints-only tensor-core path (compact sub-model), small-batch engine, score-net JVP, native fitting steps
+# round 2: joints-only tensor-core path (compact sub-model), score-net JVP, native fitting steps
 for mt, B in [('smplx', 96), ('smpl', 130)]:
     bm = BodyModel(synthetic.make_body_tensors(mt), batch_size=B, model_type=mt).cuda()
     inp = {k: v.cuda().requires_grad_(True) for k, v in synthetic.lbs_inputs(B, mt).items()}
     o = bm(need_verts=False, **inp); o.Jtr.sum().backward(); torch.cuda.synchronize(); print('lbs joints-only ok', mt)
-os.environ['DPB_TC_SMALL'] = '1'
-fn = sampling.get_sampling_fn(cfg, sde_lib.subVPSDE(0.1, 20., 3), (300, 63), lambda x: x, 1e-3, device='cuda')
-_, x = fn(model, z=torch.randn(300, 63)); torch.cuda.synchronize(); print('small engine ok', float(x.abs().mean()))
-os.environ['DPB_TC_SMALL'] = '0'
 from dposer_b200 import likelihood
 d, dv = likelihood.drift_and_div(model, sde_lib.subVPSDE(0.1, 20., 1000), torch.randn(70, 63).cuda(), 0.3,
                                  torch.randn(70, 63).cuda())

@@ -169,12 +169,10 @@ def test_lbs_backward_with_an_unused_output(which):
         assert (got - ref).abs().max() / scale < 2e-4, k
 
 
-@pytest.mark.parametrize('B', [97, 193, 1000])
-@pytest.mark.parametrize('staged', ['1', '0'])
-def test_lbs_pair_kernel_group_boundaries(B, staged, monkeypatch):
-    """CTA-pair fused kernel (lbs_fused2_kernel): pose counts one past / straddling 96-pose groups, both store paths
-    (staged full-line stores / direct stride-12 stores), SMPL and SMPL-X (const tail folded into the template)."""
-    monkeypatch.setenv('DPB_LBS_STAGED', staged)
+@pytest.mark.parametrize('B', [97, 129, 193, 255, 385, 1000])
+def test_lbs_pair_kernel_group_boundaries(B):
+    """CTA-pair fused kernels: SMPL runs lbs_fused3_kernel (128-pose groups), SMPL-X with the const tail folded into
+    the template runs lbs_fused2_kernel (96-pose groups).  Pose counts one past / one short of / straddling groups."""
     for mt in ('smpl', 'smplx'):
         m = synthetic.make_body_tensors(mt)
         inp = synthetic.lbs_inputs(B, mt, seed=17)

@@ -287,35 +287,3 @@ def test_likelihood_vs_reference_golden(gpu_model):
     assert max_rel(z, g['lik_z']) < 5e-3
     # device-side RK45 with scipy's controller: the step sequence follows the reference's to within a few evaluations
     assert abs(nfe - int(g['lik_nfe'])) <= 0.02 * int(g['lik_nfe']), (nfe, int(g['lik_nfe']))
-
-
-def test_small_batch_engine_matches_whole_tile_engine(gpu_model, monkeypatch):
-    """tcs::score_small_kernel (output features split over 16 CTAs per row tile, opt-in with DPB_TC_SMALL=1) against the
-    whole-tile tcgen05 kernel and the oracle goldens: 8-step sampler with replayed draws, completion (imputation) and a
-    plain forward at 500 rows."""
-    g = golden('sampler_golden.npz')
-    cfg = synthetic.default_config()
-    outs = {}
-    for small in ('1', '0'):
-        monkeypatch.setenv('DPB_TC_SMALL', small)
-        gpu_model.engine = L.ENGINE_TC
-        try:
-            B, N = 500, 8
-            sde = sde_lib.subVPSDE(0.1, 20., N)
-            fn = sampling.get_sampling_fn(cfg, sde, (B, 63), lambda x: x, 1e-3, device='cuda')
-            gen = torch.Generator().manual_seed(3)
-            z0 = torch.randn(B, 63, generator=gen)
-            noise = torch.randn(N, 1, B, 63, generator=gen).cuda()
-            traj, x = fn(gpu_model, z=z0, noise=noise)
-            _, mask, obs = synthetic.completion_inputs(n_partial=B, hypotheses=1)
-            nz3 = torch.randn(N, 3, B, 63, generator=gen).cuda()
-            import types
-            _, xc = fn(gpu_model, z=z0, observation=obs.cuda(), mask=mask.cuda(), noise=nz3,
-                       args=types.SimpleNamespace(task='completion'))
-            score = gpu_model(z0.cuda(), torch.full((B,), 499.5))
-            outs[small] = (x, traj[-1], xc, score)
-        finally:
-            gpu_model.engine = L.ENGINE_AUTO
-    for a, b in zip(outs['1'], outs['0']):
-        assert torch.isfinite(a).all()
-        assert max_rel(a, b.cpu().numpy()) < 1e-3
