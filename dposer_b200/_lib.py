@@ -50,9 +50,9 @@ EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create
            'dpb_lbs_backward', 'dpb_lbs_backward_scratch_bytes', 'dpb_lbs_backward_scratch_bytes_joints', 'dpb_apd_partial', 'dpb_mean_point_error', 'dpb_fit_loss',
            'dpb_motion_loss', 'dpb_camera_fit_loss', 'dpb_adam_step', 'dpb_affine_cols', 'dpb_axis_to_rot6d_cols',
            'dpb_axis_to_rot6d_cols_vjp', 'dpb_joint_map_gather',
-           'dpb_joint_map_scatter', 'dpb_masked_mse_grad', 'dpb_seq_smooth3', 'dpb_train_create', 'dpb_train_destroy',
+           'dpb_joint_map_scatter', 'dpb_masked_mse_grad', 'dpb_seq_smooth3', 'dpb_train_create', 'dpb_train_create_dim', 'dpb_train_destroy',
            'dpb_train_loss_grad', 'dpb_train_adam_scratch_bytes', 'dpb_train_grad_norm', 'dpb_train_adam', 'dpb_ema_update', 'dpb_train_set_seed_pointer', 'dpb_gemm_nt_workspace_bytes', 'dpb_gemm_nt', 'dpb_train_forward', 'dpb_train_backward', 'dpb_rows_axpby', 'dpb_weighted_sqdiff', 'dpb_rk45_stage', 'dpb_rk45_scratch_bytes', 'dpb_rk45_error',
-           'dpb_pf_ode_rhs', 'dpb_selfisect_create', 'dpb_selfisect_destroy', 'dpb_selfisect_workspace_bytes',
+           'dpb_pf_ode_rhs', 'dpb_pf_ode_rhs_dim', 'dpb_selfisect_create', 'dpb_selfisect_destroy', 'dpb_selfisect_workspace_bytes',
            'dpb_selfisect_run', 'dpb_procrustes']
 
 _lib = None
@@ -129,6 +129,7 @@ def load():
     lib.dpb_joint_map_gather.argtypes = [vp, C.c_int, vp, C.c_int, vp, i64, vp]
     lib.dpb_joint_map_scatter.argtypes = [vp, C.c_int, vp, C.c_int, vp, i64, vp]
     lib.dpb_train_create.argtypes = [C.POINTER(vp), i64, C.c_int]
+    lib.dpb_train_create_dim.argtypes = [C.POINTER(vp), i64, C.c_int, C.c_int]
     lib.dpb_train_destroy.argtypes = [vp]
     lib.dpb_train_loss_grad.argtypes = [vp, C.POINTER(ScoreWeights), C.POINTER(ScoreWeights), vp, vp, vp, vp, f32, u64, vp,
                                         vp, vp]
@@ -149,6 +150,7 @@ def load():
     lib.dpb_rk45_scratch_bytes.restype = sz
     lib.dpb_rk45_error.argtypes = [vp, vp, vp, i64, f64, f64, f64, vp, vp]
     lib.dpb_pf_ode_rhs.argtypes = [vp, vp, vp, vp, f32, f32, vp, i64, vp]
+    lib.dpb_pf_ode_rhs_dim.argtypes = [vp, vp, vp, vp, f32, f32, vp, i64, C.c_int, vp]
     lib.dpb_mean_point_error.argtypes = [vp, vp, i64, C.c_int, vp, C.c_int, vp, vp]
     lib.dpb_selfisect_create.argtypes = [C.POINTER(vp), _i32p, C.c_int, C.c_int, C.c_int]
     lib.dpb_selfisect_destroy.argtypes = [vp]

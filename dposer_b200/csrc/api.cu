@@ -274,23 +274,23 @@ extern "C" int dpb_sampler_run_pc(dpb_score_t* h, float* x_io, const dpb_step_ta
 }
 
 extern "C" size_t dpb_score_jvp_workspace_bytes(dpb_score_t* h, int64_t B) {
-  if (!h || B <= 0 || h->pose_dim != DPB_POSE_DIM) return 0;
-  const size_t simt = simt_forward_ws_bytes(2 * B), tc = score_jvp_tc_ws_bytes(B);
-  return (simt > tc ? simt : tc) + align_up((size_t)2 * B * DP * 4, 256) + 1024;
+  if (!h || B <= 0) return 0;
+  const int dp = h->pose_dp;
+  const size_t simt = simt_forward_ws_bytes(2 * B, dp), tc = score_jvp_tc_ws_bytes(B, dp);
+  return (simt > tc ? simt : tc) + align_up((size_t)2 * B * dp * 4, 256) + 1024;
 }
 
 extern "C" int dpb_score_jvp(dpb_score_t* h, const float* x, const float* v, const float* table, const int32_t* t_index,
                              const float* row_scale, float scale, float* out, float* jv, int64_t B, void* ws,
                              size_t ws_bytes, void* stream) {
   if (!h) return fail(DPB_EINVAL, "dpb_score_jvp: null handle");
-  if (h->pose_dim != DPB_POSE_DIM) return fail(DPB_EUNSUPPORTED, "dpb_score_jvp: the forward-mode derivative is built for 63-D (axis) "
-                                              "networks only, not for rot6d (126-D)");
   DeviceGuard guard(h->device);
   DPB_REQUIRE(x && v && table && out && jv, "dpb_score_jvp: x, v, table, out and jv are required");
   if (B <= 0) return DPB_OK;
   cudaStream_t st = (cudaStream_t)stream;
+  const int dp = h->pose_dp;
   WsCarver c(ws, ws_bytes);
-  float* raw = c.take<float>((size_t)2 * B * DP);
+  float* raw = c.take<float>((size_t)2 * B * dp);
   if (!c.ok() || ws == nullptr || ws_bytes < dpb_score_jvp_workspace_bytes(h, B))
     return fail(DPB_ENOMEM, "dpb_score_jvp: workspace too small");
   void* rest = static_cast<uint8_t*>(ws) + c.off;
@@ -298,9 +298,9 @@ extern "C" int dpb_score_jvp(dpb_score_t* h, const float* x, const float* v, con
   int rc = !t_index ? score_jvp_tc_raw(h, x, v, table, raw, B, rest, ws_bytes - c.off, st)
                     : simt_forward_jvp_raw(h, x, v, table, t_index, raw, B, rest, ws_bytes - c.off, st);
   if (rc != DPB_OK) return rc;
-  rc = launch_scale_out(raw, row_scale, scale, out, B, DP, st);
+  rc = launch_scale_out(raw, row_scale, scale, out, B, dp, st);
   if (rc != DPB_OK) return rc;
-  return launch_scale_out(raw + (size_t)B * DP, row_scale, scale, jv, B, DP, st);   // the scaling is linear: same factor
+  return launch_scale_out(raw + (size_t)B * dp, row_scale, scale, jv, B, dp, st);   // the scaling is linear: same factor
 }
 
 extern "C" int dpb_sampler_run(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, const float* obs,

@@ -70,7 +70,9 @@ __global__ void __launch_bounds__(256) error_final_kernel(const double* __restri
 }
 
 // right-hand side of the probability-flow ODE from the network outputs (likelihood.py:58-66 / sampling.py:505-509):
-// k[b*63 + c] = fx x - 0.5 g2 score ;  k[B*63 + b] = fx sum_c eps^2 - 0.5 g2 sum_c jv eps   (jv / eps null: drift only)
+// k[b*PD + c] = fx x - 0.5 g2 score ;  k[B*PD + b] = fx sum_c eps^2 - 0.5 g2 sum_c jv eps   (jv / eps null: drift only),
+// PD = the pose width (63 axis-angle, 126 rot6d)
+template <int PD>
 __global__ void __launch_bounds__(256) pf_rhs_kernel(const float* __restrict__ x, const float* __restrict__ score,
                                                      const float* __restrict__ jv, const float* __restrict__ eps, float fx,
                                                      float g2, float* __restrict__ kout, int64_t B) {
@@ -78,8 +80,8 @@ __global__ void __launch_bounds__(256) pf_rhs_kernel(const float* __restrict__ x
   const int lane = threadIdx.x & 31;
   if (b >= B) return;
   float d1 = 0.f, d2 = 0.f;
-  for (int c = lane; c < D; c += 32) {
-    const size_t i = (size_t)b * D + c;
+  for (int c = lane; c < PD; c += 32) {
+    const size_t i = (size_t)b * PD + c;
     kout[i] = fx * x[i] - 0.5f * g2 * score[i];
     if (jv) { const float e = eps[i]; d1 += e * e; d2 += jv[i] * e; }
   }
@@ -88,7 +90,7 @@ __global__ void __launch_bounds__(256) pf_rhs_kernel(const float* __restrict__ x
     d1 += __shfl_xor_sync(0xffffffffu, d1, o);
     d2 += __shfl_xor_sync(0xffffffffu, d2, o);
   }
-  if (lane == 0) kout[(size_t)B * D + b] = fx * d1 - 0.5f * g2 * d2;
+  if (lane == 0) kout[(size_t)B * PD + b] = fx * d1 - 0.5f * g2 * d2;
 }
 
 }  // namespace rk
@@ -119,11 +121,21 @@ extern "C" int dpb_rk45_error(const double* y, const double* y_new, const float*
   return DPB_OK;
 }
 
-extern "C" int dpb_pf_ode_rhs(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2,
-                              float* k_out, int64_t B, void* stream) {
+extern "C" int dpb_pf_ode_rhs_dim(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2,
+                                  float* k_out, int64_t B, int pose_dim, void* stream) {
+  if (pose_dim != DPB_POSE_DIM && pose_dim != DPB_POSE_DIM_ROT6D)
+    return fail(DPB_EUNSUPPORTED, "dpb_pf_ode_rhs_dim: pose_dim must be 63 (axis-angle) or 126 (rot6d)");
   DPB_REQUIRE(x && score && k_out && B > 0 && (!jv || eps), "dpb_pf_ode_rhs: bad argument");
   PtrDeviceGuard guard(x);
-  rk::pf_rhs_kernel<<<(unsigned)((B + 7) / 8), 256, 0, (cudaStream_t)stream>>>(x, score, jv, eps, fx, g2, k_out, B);
+  const unsigned grid = (unsigned)((B + 7) / 8);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (pose_dim == D126) rk::pf_rhs_kernel<D126><<<grid, 256, 0, st>>>(x, score, jv, eps, fx, g2, k_out, B);
+  else rk::pf_rhs_kernel<D><<<grid, 256, 0, st>>>(x, score, jv, eps, fx, g2, k_out, B);
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;
+}
+
+extern "C" int dpb_pf_ode_rhs(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2,
+                              float* k_out, int64_t B, void* stream) {
+  return dpb_pf_ode_rhs_dim(x, score, jv, eps, fx, g2, k_out, B, DPB_POSE_DIM, stream);
 }

@@ -299,23 +299,24 @@ int simt_forward_raw(dpb_score* h, const float* x, const float* table, const int
 
 // raw[0:B] = net(x) and raw[B:2B] = (d net / d x) v  (both before the sigma division), fp32 engine: every GEMM runs on
 // the stacked rows [primal ; tangent] (the tangent rows skip the bias), every GroupNorm + SiLU on its forward-mode twin.
-// ws: simt_forward_ws_bytes(2 B).  63-D handles only (dpb_score_jvp rejects 126-D).  Serves the Hutchinson divergence of lib/algorithms/advanced/likelihood.py:26-37:
+// ws: simt_forward_ws_bytes(2 B, DP).  Serves the Hutchinson divergence of lib/algorithms/advanced/likelihood.py:26-37:
 // eps . (J eps) is the scalar the reference gets from autograd's eps . (J^T eps).
 int simt_forward_jvp_raw(dpb_score* h, const float* x, const float* v, const float* table, const int32_t* t_index,
                          float* raw, int64_t B, void* ws, size_t ws_bytes, cudaStream_t st) {
   if (B <= 0) return DPB_OK;
   const int64_t B2 = 2 * B;
+  const int dp = h->pose_dp;
   WsCarver c(ws, ws_bytes);
-  float* xp = c.take<float>((size_t)B2 * DP);
+  float* xp = c.take<float>((size_t)B2 * dp);
   float* pre = c.take<float>((size_t)B2 * H);
   float* hbuf = c.take<float>((size_t)B2 * H);
   float* tbuf = c.take<float>((size_t)B2 * H);
   if (!c.ok() || ws == nullptr) return fail(DPB_ENOMEM, "score jvp: workspace too small");
   const int stride = NL * H;
   dim3 gemm_grid(H / BN, (unsigned)((B2 + BM - 1) / BM));
-  launch_pad_x(x, xp, B, DP, st);
-  launch_pad_x(v, xp + (size_t)B * DP, B, DP, st);
-  sgemm_bias_kernel<<<gemm_grid, 256, 0, st>>>(xp, h->pre_w, pre, B2, H, DP, table, t_index, stride, nullptr, B);
+  launch_pad_x(x, xp, B, dp, st);
+  launch_pad_x(v, xp + (size_t)B * dp, B, dp, st);
+  sgemm_bias_kernel<<<gemm_grid, 256, 0, st>>>(xp, h->pre_w, pre, B2, H, dp, table, t_index, stride, nullptr, B);
   gn_silu_jvp_kernel<<<(unsigned)B, 256, 0, st>>>(pre, h->gn_w[0], h->gn_b[0], nullptr, hbuf, B);
   for (int blk = 0; blk < 2; ++blk) {
     int l1 = 1 + 2 * blk, l2 = 2 + 2 * blk;
@@ -326,8 +327,8 @@ int simt_forward_jvp_raw(dpb_score* h, const float* x, const float* v, const flo
                                                  t_index, stride, nullptr, B);
     gn_silu_jvp_kernel<<<(unsigned)B, 256, 0, st>>>(pre, h->gn_w[l2], h->gn_b[l2], hbuf, hbuf, B);
   }
-  dim3 post_grid(DP / BN, (unsigned)((B2 + BM - 1) / BM));
-  sgemm_bias_kernel<<<post_grid, 256, 0, st>>>(hbuf, h->post_w, raw, B2, DP, H, nullptr, nullptr, 0, h->post_b, B);
+  dim3 post_grid(dp / BN, (unsigned)((B2 + BM - 1) / BM));
+  sgemm_bias_kernel<<<post_grid, 256, 0, st>>>(hbuf, h->post_w, raw, B2, dp, H, nullptr, nullptr, 0, h->post_b, B);
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;
 }
@@ -336,7 +337,7 @@ int simt_forward_jvp_raw(dpb_score* h, const float* x, const float* v, const flo
 // ------------------------------------------------------------------ the same JVP with every contraction on tcgen05
 // (gemm_tc.cu: fp16 [hi | lo] operands, three products, fp32 accumulation in TMEM -- ~1e-6 relative, so it stands in for
 // the fp32 SGEMM above).  Batch-uniform time only (one table row, the likelihood's case): the affine part of a layer is a
-// column bias applied to the primal rows.  The weight operands are built once per handle.
+// column bias applied to the primal rows.  The weight operands are built once per handle, at the handle's padded width.
 struct JvpOps {
   __half* pool = nullptr;
   Op16 Wpre, W[4], Wpost;
@@ -351,11 +352,11 @@ static Op16 carve_op16(WsCarver& ws, int64_t rows, int64_t kp) {
   return o;
 }
 
-static size_t jvp_weight_layout(JvpOps* o, void* base, size_t cap) {
+static size_t jvp_weight_layout(JvpOps* o, int dp, void* base, size_t cap) {
   WsCarver ws(base, cap);
-  o->Wpre = carve_op16(ws, H, DP);
+  o->Wpre = carve_op16(ws, H, dp);
   for (int l = 0; l < 4; ++l) o->W[l] = carve_op16(ws, H, H);
-  o->Wpost = carve_op16(ws, DP, H);
+  o->Wpost = carve_op16(ws, dp, H);
   return align_up(ws.off, 256);
 }
 
@@ -364,20 +365,20 @@ struct JvpWs {
   Op16 xp16, a16;
 };
 
-static size_t jvp_ws_layout(JvpWs* w, int64_t B2, void* base, size_t cap) {
+static size_t jvp_ws_layout(JvpWs* w, int64_t B2, int dp, void* base, size_t cap) {
   WsCarver ws(base, cap);
-  w->xp = ws.take<float>((size_t)B2 * DP);
+  w->xp = ws.take<float>((size_t)B2 * dp);
   w->pre = ws.take<float>((size_t)B2 * H);
   w->hbuf = ws.take<float>((size_t)B2 * H);
   w->tbuf = ws.take<float>((size_t)B2 * H);
-  w->xp16 = carve_op16(ws, B2, DP);
+  w->xp16 = carve_op16(ws, B2, dp);
   w->a16 = carve_op16(ws, B2, H);
   return align_up(ws.off, 256);
 }
 
-size_t score_jvp_tc_ws_bytes(int64_t B) {
+size_t score_jvp_tc_ws_bytes(int64_t B, int dp) {
   JvpWs w;
-  return jvp_ws_layout(&w, 2 * B, nullptr, ~(size_t)0) + 1024;
+  return jvp_ws_layout(&w, 2 * B, dp, nullptr, ~(size_t)0) + 1024;
 }
 
 void score_jvp_tc_release(dpb_score* h) {
@@ -392,28 +393,29 @@ int score_jvp_tc_raw(dpb_score* h, const float* x, const float* v, const float* 
                      size_t ws_bytes, cudaStream_t st) {
   if (B <= 0) return DPB_OK;
   int rc = DPB_OK;
+  const int dp = h->pose_dp;
   JvpOps* o = static_cast<JvpOps*>(h->jvp_ops);
   if (!o) {
     if ((rc = gemm_tc_init()) != DPB_OK) return rc;
     o = new JvpOps();
-    const size_t bytes = jvp_weight_layout(o, nullptr, ~(size_t)0);
+    const size_t bytes = jvp_weight_layout(o, dp, nullptr, ~(size_t)0);
     if (cudaMalloc((void**)&o->pool, bytes) != cudaSuccess) { delete o; return fail(DPB_ENOMEM, "score jvp: weight operands"); }
-    jvp_weight_layout(o, o->pool, bytes);
+    jvp_weight_layout(o, dp, o->pool, bytes);
     h->jvp_ops = o;
-    if ((rc = split16(h->pre_w, H, DP, DP, &o->Wpre, nullptr, st)) != DPB_OK) return rc;
+    if ((rc = split16(h->pre_w, H, dp, dp, &o->Wpre, nullptr, st)) != DPB_OK) return rc;
     for (int l = 0; l < 4; ++l)
       if ((rc = split16(h->blk_w[l], H, H, H, &o->W[l], nullptr, st)) != DPB_OK) return rc;
-    if ((rc = split16(h->post_w, DP, H, H, &o->Wpost, nullptr, st)) != DPB_OK) return rc;
+    if ((rc = split16(h->post_w, dp, H, H, &o->Wpost, nullptr, st)) != DPB_OK) return rc;
   }
   const int64_t B2 = 2 * B;
   JvpWs w;
-  if (ws == nullptr || jvp_ws_layout(&w, B2, ws, ws_bytes) > ws_bytes) return fail(DPB_ENOMEM, "score jvp: workspace too small");
+  if (ws == nullptr || jvp_ws_layout(&w, B2, dp, ws, ws_bytes) > ws_bytes) return fail(DPB_ENOMEM, "score jvp: workspace too small");
   const int M = (int)B2, Bi = (int)B;
-  launch_pad_x(x, w.xp, B, DP, st);
-  launch_pad_x(v, w.xp + (size_t)B * DP, B, DP, st);
+  launch_pad_x(x, w.xp, B, dp, st);
+  launch_pad_x(v, w.xp + (size_t)B * dp, B, dp, st);
 #define JTRY(expr) do { rc = (expr); if (rc != DPB_OK) return rc; } while (0)
-  JTRY(split16(w.xp, M, DP, DP, &w.xp16, nullptr, st));
-  JTRY(gemm_tc(w.xp16, o->Wpre, M, H, DP, w.pre, H, table, nullptr, nullptr, 0, st, Bi));
+  JTRY(split16(w.xp, M, dp, dp, &w.xp16, nullptr, st));
+  JTRY(gemm_tc(w.xp16, o->Wpre, M, H, dp, w.pre, H, table, nullptr, nullptr, 0, st, Bi));
   gn_silu_jvp_kernel<<<(unsigned)B, 256, 0, st>>>(w.pre, h->gn_w[0], h->gn_b[0], nullptr, w.hbuf, B);
   for (int blk = 0; blk < 2; ++blk) {
     const int l1 = 1 + 2 * blk, l2 = 2 + 2 * blk;
@@ -425,7 +427,7 @@ int score_jvp_tc_raw(dpb_score* h, const float* x, const float* v, const float* 
     gn_silu_jvp_kernel<<<(unsigned)B, 256, 0, st>>>(w.pre, h->gn_w[l2], h->gn_b[l2], w.hbuf, w.hbuf, B);
   }
   JTRY(split16(w.hbuf, M, H, H, &w.a16, nullptr, st));
-  JTRY(gemm_tc(w.a16, o->Wpost, M, DP, H, raw, DP, h->post_b, nullptr, nullptr, 0, st, Bi));
+  JTRY(gemm_tc(w.a16, o->Wpost, M, dp, H, raw, dp, h->post_b, nullptr, nullptr, 0, st, Bi));
 #undef JTRY
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;

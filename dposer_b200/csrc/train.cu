@@ -22,6 +22,7 @@
 struct dpb_train {
   int device = 0;
   int64_t B = 0, Bp = 0;
+  int pose_dim = 63, pose_dp = 64;        // network width D (63 axis-angle, 126 rot6d) and its padded width DP (64, 128)
   char* pool = nullptr;
   size_t pool_bytes = 0;
   float *xp, *z, *temb0, *q, *temb, *tproj, *u[5], *act[5], *res, *gres, *Gall, *gA, *gB, *gtemb, *gq, *t1, *t2;
@@ -38,30 +39,33 @@ namespace trn {
 
 constexpr int SS_BLOCKS = 512;
 
-// perturbed = mean_c x + std_c z (losses.py:112-115), z from Philox or given; sinusoidal embedding of the label (model.py:37-51)
+// perturbed = mean_c x + std_c z (losses.py:112-115), z from Philox or given; sinusoidal embedding of the label (model.py:37-51).
+// Thread t < PDP / 4 owns columns 4t..4t+3 and draws them with Philox counter t: at 126 threads 16..31 add columns 64..127.
+template <int PDP>
 __global__ void __launch_bounds__(256) prep_kernel(const float* __restrict__ batch, const float* __restrict__ rows,
                                                    const float* __restrict__ z_given, uint64_t seed,
                                                    const uint64_t* __restrict__ seed_dev,
                                                    const float* __restrict__ freqs, float* __restrict__ xp,
                                                    float* __restrict__ z, float* __restrict__ temb0, int64_t B) {
+  constexpr int PD = pose_dim_of(PDP);
   if (seed_dev) seed = *seed_dev;
   const int64_t b = blockIdx.x;
   const int t = threadIdx.x;
   const float label = rows[b], mc = rows[B + b], sc = rows[2 * B + b];
-  if (t < 16) {
+  if (t < PDP / 4) {
     float zz[4];
     if (z_given) {
 #pragma unroll
-      for (int i = 0; i < 4; ++i) zz[i] = (4 * t + i < D) ? z_given[b * D + 4 * t + i] : 0.f;
+      for (int i = 0; i < 4; ++i) zz[i] = (4 * t + i < PD) ? z_given[b * PD + 4 * t + i] : 0.f;
     } else {
       normal4(seed, (uint64_t)b, 0u, 0u, (uint32_t)t, zz);
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
       const int k = 4 * t + i;
-      const float zv = k < D ? zz[i] : 0.f;
-      z[b * DP + k] = zv;
-      xp[b * DP + k] = k < D ? mc * batch[b * D + k] + sc * zv : 0.f;
+      const float zv = k < PD ? zz[i] : 0.f;
+      z[b * PDP + k] = zv;
+      xp[b * PDP + k] = k < PD ? mc * batch[b * PD + k] + sc * zv : 0.f;
     }
   }
   const float arg = label * freqs[t];
@@ -201,21 +205,23 @@ __global__ void __launch_bounds__(1024) colsum3_kernel(const float* __restrict__
 }
 
 // e = res_c res + z_c z ; loss_row = row_w sum e^2 ; d loss / d res = 2 row_w res_c e / B   (losses.py:124-131)
+template <int PDP>
 __global__ void __launch_bounds__(256) loss_kernel(const float* __restrict__ res, const float* __restrict__ z,
                                                    const float* __restrict__ rows, float* __restrict__ gres,
                                                    float* __restrict__ loss_rows, int64_t B) {
   const int64_t b = (int64_t)blockIdx.x * 8 + (threadIdx.x >> 5);
   const int lane = threadIdx.x & 31;
   if (b >= B) return;
+  constexpr int PD = pose_dim_of(PDP);
   const float rc = rows[3 * B + b], zc = rows[4 * B + b], w = rows[5 * B + b];
   float acc = 0.f;
 #pragma unroll
-  for (int h2 = 0; h2 < 2; ++h2) {
+  for (int h2 = 0; h2 < PDP / 32; ++h2) {
     const int k = lane + 32 * h2;
     float e = 0.f;
-    if (k < D) e = rc * res[b * DP + k] + zc * z[b * DP + k];
+    if (k < PD) e = rc * res[b * PDP + k] + zc * z[b * PDP + k];
     acc += e * e;
-    gres[b * DP + k] = k < D ? 2.0f * w * rc * e / (float)B : 0.f;
+    gres[b * PDP + k] = k < PD ? 2.0f * w * rc * e / (float)B : 0.f;
   }
   for (int o = 16; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
   if (lane == 0) loss_rows[b] = w * acc;
@@ -288,7 +294,7 @@ static Op16 carve16(WsCarver& ws, int64_t rows, int64_t kp) {
 
 static size_t layout(dpb_train* h, void* base, size_t cap) {
   WsCarver ws(base, cap);
-  const int64_t B = h->B, Bp = h->Bp;
+  const int64_t B = h->B, Bp = h->Bp, DP = h->pose_dp;
   h->xp = ws.take<float>(B * DP); h->z = ws.take<float>(B * DP);
   h->temb0 = ws.take<float>(B * E); h->q = ws.take<float>(B * E); h->temb = ws.take<float>(B * E);
   h->tproj = ws.take<float>(B * NL * H);
@@ -322,7 +328,9 @@ static size_t layout(dpb_train* h, void* base, size_t cap) {
 
 using namespace dpb;
 
-extern "C" int dpb_train_create(dpb_train** out, int64_t batch, int device) {
+extern "C" int dpb_train_create_dim(dpb_train** out, int64_t batch, int pose_dim, int device) {
+  if (pose_dim != DPB_POSE_DIM && pose_dim != DPB_POSE_DIM_ROT6D)
+    return fail(DPB_EUNSUPPORTED, "dpb_train_create_dim: pose_dim must be 63 (axis-angle) or 126 (rot6d)");
   DPB_REQUIRE(out && batch > 0, "dpb_train_create: bad argument");
   DeviceGuard guard(device);
   int rc = gemm_tc_init();
@@ -330,6 +338,8 @@ extern "C" int dpb_train_create(dpb_train** out, int64_t batch, int device) {
   dpb_train* h = new dpb_train();
   h->device = device;
   h->B = batch;
+  h->pose_dim = pose_dim;
+  h->pose_dp = pose_dim == D126 ? DP128 : DP;
   h->Bp = (batch + 63) / 64 * 64;
   h->pool_bytes = trn::layout(h, nullptr, ~(size_t)0);
   cudaError_t e = cudaMalloc((void**)&h->pool, h->pool_bytes);
@@ -341,6 +351,10 @@ extern "C" int dpb_train_create(dpb_train** out, int64_t batch, int device) {
   cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
   *out = h;
   return DPB_OK;
+}
+
+extern "C" int dpb_train_create(dpb_train** out, int64_t batch, int device) {
+  return dpb_train_create_dim(out, batch, DPB_POSE_DIM, device);
 }
 
 extern "C" int dpb_train_set_seed_pointer(dpb_train* h, const uint64_t* seed_dev) {
@@ -363,19 +377,21 @@ extern "C" int dpb_train_destroy(dpb_train* h) {
 namespace dpb {
 namespace trn {
 
-// x [B,63] -> xp [B,64] (pad column zero); sinusoidal embedding of the per-row label
+// x [B,D] -> xp [B,DP] (pad columns zero); sinusoidal embedding of the per-row label
+template <int PDP>
 __global__ void __launch_bounds__(256) prep_given_kernel(const float* __restrict__ x, const float* __restrict__ labels,
                                                          const float* __restrict__ freqs, float* __restrict__ xp,
                                                          float* __restrict__ temb0, int64_t B) {
+  constexpr int PD = pose_dim_of(PDP);
   const int64_t b = blockIdx.x;
   const int t = threadIdx.x;
-  if (t < DP) xp[b * DP + t] = t < D ? x[b * D + t] : 0.f;
+  if (t < PDP) xp[b * PDP + t] = t < PD ? x[b * PD + t] : 0.f;
   const float arg = labels[b] * freqs[t];
   temb0[b * E + t] = sinf(arg);
   temb0[b * E + E / 2 + t] = cosf(arg);
 }
 
-// [B,63] <-> [B,64] copies of the network output / its cotangent
+// [B,D] <-> [B,DP] copies of the network output / its cotangent
 __global__ void pad_cols_kernel(const float* __restrict__ src, int ls, float* __restrict__ dst, int ld, int cols, int64_t B) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (i >= B * ld) return;
@@ -402,6 +418,7 @@ struct Ptrs {
 static int weight_operands(dpb_train* h, const dpb_train_tensors* P, bool back, cudaStream_t st) {
   int rc = DPB_OK;
   const Ptrs w(P);
+  const int D = h->pose_dim;
   TRY(split16(P->pre_w, H, D, D, &h->Wpre16, back ? &h->WpreT16 : nullptr, st));
   for (int l = 0; l < 4; ++l) TRY(split16(w.Wl[l], H, H, H, &h->W16[l], back ? &h->WT16[l] : nullptr, st));
   TRY(split16(P->post_w, D, H, H, &h->Wpost16, back ? &h->WpostT16 : nullptr, st));
@@ -419,7 +436,7 @@ static int forward(dpb_train* h, const dpb_train_tensors* P, const uint8_t* mask
   int rc = DPB_OK;
   const Ptrs w(P);
   const int64_t B = h->B;
-  const int Bi = (int)B;
+  const int Bi = (int)B, D = h->pose_dim, DP = h->pose_dp;
   const unsigned gw = (unsigned)((B * 32 + 7) / 8);
   TRY(split16(h->xp, Bi, DP, DP, &h->xp16, back ? &h->xpT16 : nullptr, st));
   TRY(split16(h->temb0, Bi, E, E, &h->temb0_16, back ? &h->temb0T16 : nullptr, st));
@@ -441,13 +458,13 @@ static int forward(dpb_train* h, const dpb_train_tensors* P, const uint8_t* mask
 }
 
 // h->gres (cotangent of res) -> every parameter gradient (overwritten, or added to with `acc`) and, if asked, the
-// cotangent of the network input g_x [B,63]
+// cotangent of the network input g_x [B,D]
 static int backward(dpb_train* h, const dpb_train_tensors* P, const dpb_train_tensors* G, const uint8_t* mask_given,
                     float drop_p, uint64_t seed, bool acc, float* g_x, cudaStream_t st) {
   int rc = DPB_OK;
   const Ptrs w(P);
   const int64_t B = h->B;
-  const int Bi = (int)B;
+  const int Bi = (int)B, D = h->pose_dim, DP = h->pose_dp;
   const unsigned gw = (unsigned)((B * 32 + 7) / 8);
   float* gWl[4] = {(float*)G->blk_w[0], (float*)G->blk_w[1], (float*)G->blk_w[2], (float*)G->blk_w[3]};
   float* gWt[5] = {(float*)G->pre_t_w, (float*)G->blk_t_w[0], (float*)G->blk_t_w[1], (float*)G->blk_t_w[2], (float*)G->blk_t_w[3]};
@@ -465,7 +482,7 @@ static int backward(dpb_train* h, const dpb_train_tensors* P, const dpb_train_te
   auto fork = [&]() { if (sd != st) { cudaEventRecord(h->ev_fork, st); cudaStreamWaitEvent(sd, h->ev_fork, 0); } };
   fork();
   TRY(gemm_tc(h->gresT16, h->XT16[4], D, H, Bi, (float*)G->post_w, H, nullptr, nullptr, addc((float*)G->post_w), H, sd));   // dW_post
-  colsum_kernel<<<2, cs, 0, st>>>(h->gres, B, D, DP, 1.0f, (float*)G->post_b, nullptr, ia);
+  colsum_kernel<<<DP / 32, cs, 0, st>>>(h->gres, B, D, DP, 1.0f, (float*)G->post_b, nullptr, ia);
   TRY(gemm_tc(h->gres16, h->WpostT16, Bi, H, DP, h->gA, H, nullptr, nullptr, nullptr, 0, st));                   // d h''
   // cotangent buffers: gA carries d h'' -> d h' -> d h (outputs of the even stages), gB the odd stages' outputs
   for (int s = NL - 1; s >= 0; --s) {
@@ -513,10 +530,14 @@ extern "C" int dpb_train_loss_grad(dpb_train* h, const dpb_train_tensors* P, con
   const int64_t B = h->B;
   int rc = trn::weight_operands(h, P, G != nullptr, st);
   if (rc != DPB_OK) return rc;
-  trn::prep_kernel<<<(unsigned)B, 256, 0, st>>>(batch, rows, z_given, seed, h->seed_dev, P->emb_freqs, h->xp, h->z, h->temb0, B);
+  const bool wide = h->pose_dp == DP128;
+  if (wide) trn::prep_kernel<DP128><<<(unsigned)B, 256, 0, st>>>(batch, rows, z_given, seed, h->seed_dev, P->emb_freqs, h->xp, h->z, h->temb0, B);
+  else trn::prep_kernel<DP><<<(unsigned)B, 256, 0, st>>>(batch, rows, z_given, seed, h->seed_dev, P->emb_freqs, h->xp, h->z, h->temb0, B);
   if ((rc = trn::forward(h, P, mask_given, drop_p, seed, G != nullptr, st)) != DPB_OK) return rc;
   float* lrows = loss_rows ? loss_rows : h->loss_rows;
-  trn::loss_kernel<<<(unsigned)((B + 7) / 8), 256, 0, st>>>(h->res, h->z, rows, h->gres, lrows, B);
+  const unsigned gl = (unsigned)((B + 7) / 8);
+  if (wide) trn::loss_kernel<DP128><<<gl, 256, 0, st>>>(h->res, h->z, rows, h->gres, lrows, B);
+  else trn::loss_kernel<DP><<<gl, 256, 0, st>>>(h->res, h->z, rows, h->gres, lrows, B);
   trn::colsum_kernel<<<1, dim3(32, 32), 0, st>>>(lrows, B, 1, 1, 1.0f / (float)B, loss, nullptr, 0);
   DPB_CUDA_CHECK(cudaGetLastError());
   if (!G) return DPB_OK;
@@ -536,7 +557,9 @@ extern "C" int dpb_train_forward(dpb_train* h, const dpb_train_tensors* P, const
   const int64_t B = h->B;
   int rc = trn::weight_operands(h, P, true, st);
   if (rc != DPB_OK) return rc;
-  trn::prep_given_kernel<<<(unsigned)B, 256, 0, st>>>(x, labels, P->emb_freqs, h->xp, h->temb0, B);
+  const int D = h->pose_dim, DP = h->pose_dp;
+  if (DP == DP128) trn::prep_given_kernel<DP128><<<(unsigned)B, 256, 0, st>>>(x, labels, P->emb_freqs, h->xp, h->temb0, B);
+  else trn::prep_given_kernel<dpb::DP><<<(unsigned)B, 256, 0, st>>>(x, labels, P->emb_freqs, h->xp, h->temb0, B);
   if ((rc = trn::forward(h, P, mask_given, drop_p, seed, true, st)) != DPB_OK) return rc;
   trn::pad_cols_kernel<<<(unsigned)((B * D + 255) / 256), 256, 0, st>>>(h->res, DP, res, D, D, B);
   DPB_CUDA_CHECK(cudaGetLastError());
@@ -550,6 +573,7 @@ extern "C" int dpb_train_backward(dpb_train* h, const dpb_train_tensors* P, cons
   DeviceGuard guard(h->device);
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t B = h->B;
+  const int D = h->pose_dim, DP = h->pose_dp;
   trn::pad_cols_kernel<<<(unsigned)((B * DP + 255) / 256), 256, 0, st>>>(g_res, D, h->gres, DP, D, B);
   int rc = trn::backward(h, P, G, mask_given, drop_p, seed, accumulate != 0, g_x, st);
   if (rc != DPB_OK) return rc;

@@ -24,8 +24,8 @@ int gemm_tc(const Op16& A, const Op16& B, int M, int N, int K, float* C, int64_t
 // fp32 [R, C] -> fp16 [hi | lo] in row form (operand rows = R) and / or column form (operand rows = C)
 int split16(const float* src, int R, int Cc, int64_t ld, const Op16* row, const Op16* col, cudaStream_t st);
 
-// score-net JVP on the same GEMM (jvp_tc.cu): raw [2B, 64] = post_dense of the stacked [primal ; tangent] rows
-size_t score_jvp_tc_ws_bytes(int64_t B);
+// score-net JVP on the same GEMM (score_simt.cu): raw [2B, DP] = post_dense of the stacked [primal ; tangent] rows
+size_t score_jvp_tc_ws_bytes(int64_t B, int dp);
 int score_jvp_tc_raw(dpb_score* h, const float* x, const float* v, const float* table, float* raw, int64_t B, void* ws,
                      size_t ws_bytes, cudaStream_t st);
 void score_jvp_tc_release(dpb_score* h);

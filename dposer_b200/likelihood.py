@@ -19,7 +19,10 @@ from . import utils as mutils
 
 
 def drift_and_div(model, sde, x, t, epsilon, ws=None):
-    """(drift [B,63], div [B]) of the probability-flow ODE at the batch-uniform time ``t`` (python float)."""
+    """(drift [B,D], div [B]) of the probability-flow ODE at the batch-uniform time ``t`` (python float); D = the network's
+    width (63 or 126)."""
+    model.check_width(x, 'x')
+    model.check_width(epsilon, 'epsilon', x.shape[0])
     L.require_cuda(x, 'x')
     B = x.shape[0]
     tt = torch.tensor([float(t)], dtype=torch.float32)
@@ -47,9 +50,10 @@ def get_likelihood_fn(sde, inverse_scaler, hutchinson_type='Rademacher', rtol=1e
     """likelihood.py:40-113.  ``likelihood_fn(model, data, epsilon=None)``: ``epsilon`` fixes the probe (parity tests)."""
 
     def likelihood_fn(model, data, epsilon=None):
-        if getattr(model, 'is_rot6d', False):
-            raise NotImplementedError('likelihood evaluation (score-network JVP) is built for the 63-D axis network, not '
-                                      'for rot6d (126-D) score networks')
+        model.check_width(data, 'data')
+        if epsilon is not None:
+            model.check_width(epsilon, 'epsilon', data.shape[0])
+        mutils.rot6d_needs_cuda(model, model.pre_dense.weight.is_cuda, 'likelihood evaluation')
         with torch.no_grad():
             L.require_cuda(data, 'data')
             data = data.to(torch.float32)

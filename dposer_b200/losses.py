@@ -24,8 +24,6 @@ from . import sde_lib
 from . import utils as mutils
 from .sde_lib import VESDE, VPSDE
 
-_DATA_DIM = L.POSE_DIM
-
 
 # ---------------------------------------------------------------------------------------------
 # native engine: one dpb_train handle per (model, batch size)
@@ -58,16 +56,14 @@ def _tensor_struct(model, pick):
 class _Engine:
     def __init__(self, model, B, device):
         from .model import embedding_freqs
-        if getattr(model, 'is_rot6d', False):
-            raise NotImplementedError('the training kernels are built for the 63-D axis network, not for rot6d (126-D) '
-                                      'score networks')
+        mutils.rot6d_needs_cuda(model, torch.device(device).type == 'cuda', 'training')
         if not model._geometry_ok:
-            raise NotImplementedError('the training kernels are built for the shipped geometry (63-D pose, hidden 1024, '
-                                      'embed 512, 2 blocks)')
-        self.B, self.device = int(B), device
+            raise NotImplementedError('the training kernels are built for the shipped geometry (63-D axis-angle or 126-D '
+                                      'rot6d pose, hidden 1024, embed 512, 2 blocks)')
+        self.B, self.device, self.D = int(B), device, int(model.pose_width)
         self.freqs = embedding_freqs(L.EMBED).to(device=device, dtype=torch.float32).contiguous()
         out = C.c_void_p()
-        L.check(L.load().dpb_train_create(C.byref(out), self.B, device.index or 0), 'dpb_train_create')
+        L.check(L.load().dpb_train_create_dim(C.byref(out), self.B, self.D, device.index or 0), 'dpb_train_create_dim')
         self.ptr = out
         self.loss = torch.zeros(1, device=device)
         self.loss_rows = torch.zeros(self.B, device=device)
@@ -82,7 +78,7 @@ class _Engine:
 
 def _engine(model, B, device):
     eng = getattr(model, '_train_engine', None)
-    if eng is None or eng.B != int(B) or eng.device != device:
+    if eng is None or eng.B != int(B) or eng.device != device or eng.D != model.pose_width:
         eng = _Engine(model, B, device)
         model._train_engine = eng
     return eng
@@ -91,12 +87,13 @@ def _engine(model, B, device):
 def native_loss(model, batch, rows, z=None, drop_mask=None, drop_p=0.0, seed=0, grads=True, clone=True, seed_dev=None):
     """One ``dpb_train_loss_grad`` call.  rows: host or device fp32 [6,B] (label, mean_c, std_c, res_c, z_c, row_w).
     Returns the loss as a [] device tensor (a fresh copy unless ``clone=False``); per-row losses stay in
-    ``model._train_engine.loss_rows``."""
+    ``model._train_engine.loss_rows``.  ``batch`` (and ``z``) are [B, D] with D the network's width (63 or 126)."""
+    model.check_width(batch, 'batch')
+    if z is not None:
+        model.check_width(z, 'z', batch.shape[0])
     L.require_cuda(batch, 'batch')
     dev = batch.device
     B = batch.shape[0]
-    if batch.shape[1] != _DATA_DIM:
-        raise NotImplementedError('the training kernels take the 63-D axis-angle representation')
     eng = _engine(model, B, dev)
     batch = batch.detach().to(torch.float32).contiguous()
     rows = rows.to(device=dev, dtype=torch.float32).contiguous()
@@ -244,6 +241,11 @@ def _draw_seed():
     return mutils.host_seed()
 
 
+def _reduction(model, reduce_mean):
+    """Row weight of the squared error: the mean over the network's D columns (1 / 63 or 1 / 126) or half the sum."""
+    return (1.0 / model.pose_width) if reduce_mean else 0.5
+
+
 def _run(model, batch, rows, train, z, drop_mask):
     p = float(model.config.model.dropout) if train else 0.0
     loss = native_loss(model, batch, rows, z=z, drop_mask=drop_mask if train else None, drop_p=p, seed=_draw_seed(),
@@ -257,9 +259,9 @@ def get_sde_loss_fn(sde, train, reduce_mean=False, continuous=True, likelihood_w
     if return_data:
         raise NotImplementedError('without autograd the estimate cannot carry gradients out of loss_fn: the auxiliary loss '
                                   'runs as a whole in get_step_fn(auxiliary_loss=True) / losses.auxiliary_loss_grad')
-    red = (1.0 / _DATA_DIM) if reduce_mean else 0.5
 
     def make_rows(model, B, t=None):
+        red = _reduction(model, reduce_mean)
         if t is None:
             t = torch.rand(B) * (sde.T - eps) + eps                  # losses.py:111 (CPU generator here)
         t = t.detach().to('cpu', torch.float32)
@@ -284,9 +286,9 @@ def get_smld_loss_fn(vesde, train, reduce_mean=False):
     """losses.py:140-161 (legacy NCSN objective; labels index the DESCENDING sigma array)."""
     assert isinstance(vesde, VESDE), "SMLD training only works for VESDEs."
     smld_sigma_array = torch.flip(vesde.discrete_sigmas, dims=(0,))
-    red = (1.0 / _DATA_DIM) if reduce_mean else 0.5
 
     def make_rows(model, B, labels=None):
+        red = _reduction(model, reduce_mean)
         if labels is None:
             labels = torch.randint(0, vesde.N, (B,))
         labels = labels.cpu()
@@ -305,9 +307,9 @@ def get_smld_loss_fn(vesde, train, reduce_mean=False):
 def get_ddpm_loss_fn(vpsde, train, reduce_mean=True):
     """losses.py:164-184 (legacy DDPM objective)."""
     assert isinstance(vpsde, VPSDE), "DDPM training only works for VPSDEs."
-    red = (1.0 / _DATA_DIM) if reduce_mean else 0.5
 
     def make_rows(model, B, labels=None):
+        red = _reduction(model, reduce_mean)
         if labels is None:
             labels = torch.randint(0, vpsde.N, (B,))
         labels = labels.cpu()
@@ -354,9 +356,13 @@ def auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_step
     ``drop_mask``: [denoise_steps, 5, B, 1024] keep-masks (parity mode); ``score_scale`` multiplies the score-matching term
     (tests switch it off to look at the body-model terms alone).  Returns a dict of [] device tensors."""
     from .misc import linear_interpolation
+    if getattr(model, 'is_rot6d', False):
+        raise NotImplementedError('the auxiliary v2v / j2j loss is built for the 63-D axis-angle network: a rot6d (126-D) '
+                                  'network would need a rot6d -> axis-angle map under the body model')
     L.require_cuda(batch, 'batch')
     lib = L.load()
     dev, B, N = batch.device, batch.shape[0], int(denoise_steps)
+    D = model.pose_width
     st = L.current_stream(dev)
     p_drop = float(model.config.model.dropout)
     engines = getattr(model, '_aux_engines', None)
@@ -392,7 +398,7 @@ def auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_step
     # ---- forward chain
     batch = batch.detach().to(torch.float32).contiguous()
     if z is None:
-        z = torch.empty(B, _DATA_DIM, device=dev)
+        z = torch.empty(B, D, device=dev)
         L.check(lib.dpb_normal_fill(L.ptr(z), B, C.c_uint64(_draw_seed()), C.c_uint64(0), 0, st))
     else:
         z = up(z)
@@ -401,14 +407,14 @@ def auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_step
     masks = [None] * N if drop_mask is None else [drop_mask[i].to(device=dev, dtype=torch.uint8).contiguous() for i in range(N)]
     res0 = None
     for i in range(N):
-        res = torch.empty(B, _DATA_DIM, device=dev)
+        res = torch.empty(B, D, device=dev)
         L.check(lib.dpb_train_forward(engines[i].ptr, C.byref(P), L.ptr(x), L.ptr(labels[i]), L.ptr(masks[i]), p_drop,
                                       C.c_uint64(seeds[i]), L.ptr(res), st))
         if i == 0:
             res0 = res
         x = _rows_axpby(c1s[i], x, c2s[i], res)
     # ---- score-matching term on the first evaluation: (score std + z)^2 = rc^2 (res - (-z / rc))^2, rc = m std
-    red = (1.0 / _DATA_DIM) if reduce_mean else 0.5
+    red = _reduction(model, reduce_mean)
     rc = m0 * std0
     target = _rows_axpby(up(-1.0 / rc), z)
     score_loss, g_res_score = _weighted_sqdiff(target, res0, up(red * rc * rc), float(score_scale) / B)
@@ -427,7 +433,7 @@ def auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_step
     # ---- chain backwards: the first call overwrites the gradients, the others add
     for i in reversed(range(N)):
         g_res = _rows_axpby(c2s[i], g_x, ones, g_res_score) if i == 0 else _rows_axpby(c2s[i], g_x)
-        g_in = torch.empty(B, _DATA_DIM, device=dev) if i > 0 else None
+        g_in = torch.empty(B, D, device=dev) if i > 0 else None
         L.check(lib.dpb_train_backward(engines[i].ptr, C.byref(P), C.byref(G), L.ptr(g_res), L.ptr(masks[i]), p_drop,
                                        C.c_uint64(seeds[i]), 0 if i == N - 1 else 1, L.ptr(g_in), st))
         if i > 0:
@@ -446,7 +452,7 @@ class _GraphedStep:
         self.eng = _engine(model, B, dev)
         self.buf = torch.zeros(8 + 6 * B, device=dev)            # [step_size, inv_sqrt_bc2, omd, -, seed lo, seed hi, -, -, rows]
         self.host = torch.zeros(8 + 6 * B)
-        self.batch = torch.zeros(B, _DATA_DIM, device=dev)
+        self.batch = torch.zeros(B, model.pose_width, device=dev)
         rows, hyper = self.buf[8:].view(6, B), self.buf[:3]
         seed_dev = C.c_void_p(self.buf.data_ptr() + 16)
         p = float(model.config.model.dropout)
@@ -513,6 +519,7 @@ def get_step_fn(sde, train, optimize_fn=None, reduce_mean=False, continuous=True
         model = state['model']
         if train and graph and not data_parallel and not auxiliary_loss and 'z' not in draws and 'drop_mask' not in draws:
             optimizer, ema, B = state['optimizer'], state['ema'], batch.shape[0]
+            model.check_width(batch, 'batch')
             L.require_cuda(batch, 'batch')
             g = graphs.get(B)
             if g is None:

@@ -103,14 +103,18 @@ def solve_rk45(backend, t0, t_bound, rtol=1e-3, atol=1e-6, max_attempts=1000000)
 
 
 class PFOdeBackend(Backend):
-    """Probability-flow ODE of the score model on the GPU: state [x (B*63) | logp (B)] (``with_div``) or x alone, in fp64;
-    a function evaluation is the score net (+ its JVP along ``epsilon``) and ``dpb_pf_ode_rhs``."""
+    """Probability-flow ODE of the score model on the GPU: state [x (B*D) | logp (B)] (``with_div``) or x alone, in fp64,
+    with D the network's width (63 or 126); a function evaluation is the score net (+ its JVP along ``epsilon``) and
+    ``dpb_pf_ode_rhs_dim``."""
 
     def __init__(self, model, sde, x0, epsilon=None):
+        model.check_width(x0, 'x')
+        if epsilon is not None:
+            model.check_width(epsilon, 'epsilon', x0.shape[0])
         L.require_cuda(x0, 'x')
         self.model, self.sde, self.dev = model, sde, x0.device
-        self.B = x0.shape[0]
-        self.nx = self.B * L.POSE_DIM
+        self.B, self.D = x0.shape[0], int(model.pose_width)
+        self.nx = self.B * self.D
         self.with_div = epsilon is not None
         self.n = self.nx + (self.B if self.with_div else 0)
         self.eps = None if epsilon is None else epsilon.to(device=self.dev, dtype=torch.float32).contiguous()
@@ -118,7 +122,7 @@ class PFOdeBackend(Backend):
         self.y[:self.nx] = x0.reshape(-1).double()
         self.y_new = torch.zeros_like(self.y)
         self.k = torch.zeros(7, self.n, dtype=torch.float32, device=self.dev)
-        self.xs = torch.empty(self.B, L.POSE_DIM, dtype=torch.float32, device=self.dev)
+        self.xs = torch.empty(self.B, self.D, dtype=torch.float32, device=self.dev)
         self.score = torch.empty_like(self.xs)
         self.jv = torch.empty_like(self.xs)
         self.lib = L.load()
@@ -127,7 +131,7 @@ class PFOdeBackend(Backend):
         nws = int(self.lib.dpb_score_jvp_workspace_bytes(self.h.ptr, self.B)) if self.with_div else 0
         self.ws = torch.empty(nws, dtype=torch.uint8, device=self.dev) if nws else None
 
-    # ---- one function evaluation: xs (fp32 [B,63]) at time t -> k[i]
+    # ---- one function evaluation: xs (fp32 [B,D]) at time t -> k[i]
     def _f(self, t, i):
         tt = torch.tensor([float(t)], dtype=torch.float32)
         coef, label = mutils.em_coefficients(self.sde, self.model, tt, probability_flow=True, continuous=True)
@@ -139,11 +143,12 @@ class PFOdeBackend(Backend):
             table = self.model.time_table(label)
             L.check(self.lib.dpb_score_jvp(self.h.ptr, L.ptr(self.xs), L.ptr(self.eps), L.ptr(table[0]), None, None, m,
                                            L.ptr(self.score), L.ptr(self.jv), self.B, L.ptr(self.ws), self.ws.numel(), st))
-            L.check(self.lib.dpb_pf_ode_rhs(L.ptr(self.xs), L.ptr(self.score), L.ptr(self.jv), L.ptr(self.eps), fx, g2,
-                                            L.ptr(self.k[i]), self.B, st))
+            L.check(self.lib.dpb_pf_ode_rhs_dim(L.ptr(self.xs), L.ptr(self.score), L.ptr(self.jv), L.ptr(self.eps), fx, g2,
+                                                L.ptr(self.k[i]), self.B, self.D, st))
         else:
             score = self.model.raw_forward(self.xs, label, torch.tensor([m]))
-            L.check(self.lib.dpb_pf_ode_rhs(L.ptr(self.xs), L.ptr(score), None, None, fx, g2, L.ptr(self.k[i]), self.B, st))
+            L.check(self.lib.dpb_pf_ode_rhs_dim(L.ptr(self.xs), L.ptr(score), None, None, fx, g2, L.ptr(self.k[i]), self.B,
+                                                self.D, st))
 
     def _stage(self, s, h, y_out):
         L.check(self.lib.dpb_rk45_stage(L.ptr(self.y), L.ptr(self.k), self.n, float(h), s, L.ptr(y_out), L.ptr(self.xs),

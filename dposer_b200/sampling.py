@@ -166,9 +166,11 @@ def get_ode_sampler(sde, shape, inverse_scaler, denoise=False, rtol=1e-5, atol=1
         return sde.reverse(score_fn, probability_flow=True).sde(x, t)[0]
 
     def ode_sampler(model, z=None):
-        if method == 'RK45' and device.type == 'cuda' and getattr(model, 'is_rot6d', False):
-            raise NotImplementedError('the device RK45 probability-flow ODE is built for the 63-D axis network, not for '
-                                      'rot6d (126-D) score networks')
+        if len(shape) != 2 or shape[1] != model.pose_width:
+            raise ValueError(f'sampler shape {tuple(shape)} does not match the {model.pose_width}-D score network')
+        if z is not None:
+            model.check_width(z, 'z')
+        mutils.rot6d_needs_cuda(model, model.pre_dense.weight.is_cuda, 'the probability-flow ODE sampler')
         with torch.no_grad():
             x = (sde.prior_sampling(shape) if z is None else z).to(device)
             if method == 'RK45' and device.type == 'cuda':

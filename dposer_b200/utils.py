@@ -173,3 +173,10 @@ def prior_scalars(sde, model, t, continuous=True):
 def host_seed():
     """A 63-bit seed drawn from torch's global CPU generator (so torch.manual_seed controls the kernels' Philox)."""
     return int(torch.randint(0, 2 ** 62, (1,), dtype=torch.int64).item())
+
+
+def rot6d_needs_cuda(model, on_cuda, what):
+    """A 126-D (rot6d) network runs ``what`` on the GPU only: refuse it, naming rot6d, before any library call."""
+    if getattr(model, 'is_rot6d', False) and not on_cuda:
+        raise NotImplementedError(f'{what} of rot6d (126-D) score networks runs on CUDA only: there is no CPU '
+                                  'implementation (move the network to a CUDA device)')

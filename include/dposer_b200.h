@@ -90,8 +90,7 @@ typedef struct {
 /* a 63-D (axis-angle, ScoreModelFC(config, 21, 3)) network */
 int dpb_score_create(dpb_score_t** h, const dpb_score_weights* w, int device);
 /* pose_dim = 63 (axis-angle) or 126 (rot6d, ScoreModelFC(config, 21, 6)); any other value: DPB_EUNSUPPORTED.
- * Every entry point that takes the handle reads D = pose_dim from it; "[B,D]" below means that width.
- * Not built for D = 126: dpb_score_jvp (DPB_EUNSUPPORTED). */
+ * Every entry point that takes the handle reads D = pose_dim from it; "[B,D]" below means that width. */
 int dpb_score_create_dim(dpb_score_t** h, const dpb_score_weights* w, int pose_dim, int device);
 /* D of the handle (63 or 126), or DPB_EINVAL for a null handle */
 int dpb_score_pose_dim(dpb_score_t* h);
@@ -115,8 +114,9 @@ int dpb_score_forward(dpb_score_t* h, const float* x, const float* table, const 
                       const float* row_scale, float scale, float* out, int64_t B, int flags,
                       void* ws, size_t ws_bytes, void* stream);
 
-/* Forward-mode derivative of dpb_score_forward (fp32 engine), 63-D handles only: out [B,63] as dpb_score_forward,
- * jv [B,63] = (d out / d x) v for a direction v [B,63], with the same row_scale / scale applied to both.  Replaces the autograd
+/* Forward-mode derivative of dpb_score_forward: out [B,D] as dpb_score_forward, jv [B,D] = (d out / d x) v for a
+ * direction v [B,D], with the same row_scale / scale applied to both (t_index NULL: split-fp16 tcgen05 GEMMs; per-row
+ * t_index: the fp32 SGEMM path).  Replaces the autograd
  * call of the Hutchinson-Skilling trace estimator in lib/algorithms/advanced/likelihood.py:26-37: the scalar
  * eps . (J eps) it needs is what the reference computes as eps . (J^T eps).  ws: dpb_score_jvp_workspace_bytes. */
 size_t dpb_score_jvp_workspace_bytes(dpb_score_t* h, int64_t B);
@@ -356,7 +356,11 @@ size_t dpb_rk45_scratch_bytes(void);
 int dpb_rk45_error(const double* y, const double* y_new, const float* k, int64_t n, double h, double rtol, double atol,
                    void* scratch, void* stream);
 /* k_out[b,c] = fx x - 0.5 g2 score (drift of the reverse ODE, sde_lib.py:98-106 with probability_flow) and, with jv / eps,
- * k_out[B*63 + b] = fx sum_c eps^2 - 0.5 g2 sum_c jv eps (Hutchinson divergence, likelihood.py:26-37) */
+ * k_out[B*D + b] = fx sum_c eps^2 - 0.5 g2 sum_c jv eps (Hutchinson divergence, likelihood.py:26-37); x, score, jv, eps
+ * [B,D] with D = pose_dim (63 or 126; any other value: DPB_EUNSUPPORTED, checked before the arguments) */
+int dpb_pf_ode_rhs_dim(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2,
+                       float* k_out, int64_t B, int pose_dim, void* stream);
+/* the pose_dim = 63 case of dpb_pf_ode_rhs_dim */
 int dpb_pf_ode_rhs(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2, float* k_out,
                    int64_t B, void* stream);
 
@@ -370,16 +374,20 @@ typedef struct dpb_train dpb_train_t;
  * emb_freqs (parameters only) = DEVICE [256]. */
 typedef dpb_score_weights dpb_train_tensors;
 
-/* scratch for steps of exactly `batch` rows (activations, cotangents, fp16 operand copies) */
+/* scratch for steps of exactly `batch` rows (activations, cotangents, fp16 operand copies) of a network of width
+ * pose_dim = 63 (axis-angle) or 126 (rot6d); any other value: DPB_EUNSUPPORTED, before any device is touched.  "[B,D]"
+ * below means that width. */
+int dpb_train_create_dim(dpb_train_t** h, int64_t batch, int pose_dim, int device);
+/* the pose_dim = 63 case of dpb_train_create_dim */
 int dpb_train_create(dpb_train_t** h, int64_t batch, int device);
 int dpb_train_destroy(dpb_train_t* h);
 /* loss = mean_b row_w[b] sum_k (res_c[b] res[b,k] + z_c[b] z[b,k])^2 on perturbed = mean_c x + std_c z, where res is the
  * network's post_dense output at the per-row label (losses.py:108-131; the sigma / std divisions and the reduce_mean /
  * likelihood-weighting factors are folded into the row scalars by the host).
  *   params    DEVICE parameter pointers;  grads  DEVICE gradient pointers (every one overwritten) or NULL = loss only
- *   batch     DEVICE fp32 [B,63] clean (normalised) poses
+ *   batch     DEVICE fp32 [B,D] clean (normalised) poses
  *   rows      DEVICE fp32 [6,B]: label (= 999 t), mean_c, std_c, res_c, z_c, row_w
- *   z_given   DEVICE fp32 [B,63] Gaussian draws (parity mode) or NULL: Philox4x32-10 keyed by (seed, row)
+ *   z_given   DEVICE fp32 [B,D] Gaussian draws (parity mode) or NULL: Philox4x32-10 keyed by (seed, row, column quad)
  *   mask_given DEVICE uint8 [5,B,1024] dropout keep-masks in layer order (parity mode) or NULL: Philox
  *   drop_p    dropout probability (0 = eval mode)
  *   loss      DEVICE fp32 [1];  loss_rows DEVICE fp32 [B] or NULL */
@@ -389,9 +397,9 @@ int dpb_train_loss_grad(dpb_train_t* h, const dpb_train_tensors* params, const d
 /* The two halves of dpb_train_loss_grad on their own, for losses that chain several network evaluations under the
  * optimiser (the auxiliary loss: multi_step_denoise of losses.py:91-106 feeding the body model, :244-258).  One handle holds
  * the activations of ONE evaluation: forward stores them, backward consumes them (same mask / drop_p / seed).
- *   x DEVICE [B,63] network input, labels DEVICE [B] (= 999 t), res DEVICE [B,63] post_dense output (before the sigma division)
- *   g_res DEVICE [B,63] cotangent of res; accumulate != 0 adds to the gradients instead of overwriting them;
- *   g_x DEVICE [B,63] cotangent of x, or NULL */
+ *   x DEVICE [B,D] network input, labels DEVICE [B] (= 999 t), res DEVICE [B,D] post_dense output (before the sigma division)
+ *   g_res DEVICE [B,D] cotangent of res; accumulate != 0 adds to the gradients instead of overwriting them;
+ *   g_x DEVICE [B,D] cotangent of x, or NULL */
 int dpb_train_forward(dpb_train_t* h, const dpb_train_tensors* params, const float* x, const float* labels,
                       const uint8_t* mask_given, float drop_p, uint64_t seed, float* res, void* stream);
 int dpb_train_backward(dpb_train_t* h, const dpb_train_tensors* params, const dpb_train_tensors* grads, const float* g_res,
