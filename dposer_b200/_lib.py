@@ -49,7 +49,7 @@ EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create
            'dpb_lbs_destroy', 'dpb_lbs_set_const_tail', 'dpb_lbs_num_joints_out', 'dpb_lbs_workspace_bytes', 'dpb_lbs_forward',
            'dpb_lbs_backward', 'dpb_lbs_backward_scratch_bytes', 'dpb_lbs_backward_scratch_bytes_joints', 'dpb_apd_partial', 'dpb_mean_point_error', 'dpb_fit_loss',
            'dpb_motion_loss', 'dpb_camera_fit_loss', 'dpb_adam_step', 'dpb_affine_cols', 'dpb_axis_to_rot6d_cols',
-           'dpb_axis_to_rot6d_cols_vjp', 'dpb_joint_map_gather',
+           'dpb_axis_to_rot6d_cols_vjp', 'dpb_rot6d_to_axis_cols', 'dpb_rot6d_to_axis_cols_vjp', 'dpb_joint_map_gather',
            'dpb_joint_map_scatter', 'dpb_masked_mse_grad', 'dpb_seq_smooth3', 'dpb_train_create', 'dpb_train_create_dim', 'dpb_train_destroy',
            'dpb_train_loss_grad', 'dpb_train_adam_scratch_bytes', 'dpb_train_grad_norm', 'dpb_train_adam', 'dpb_ema_update', 'dpb_train_set_seed_pointer', 'dpb_gemm_nt_workspace_bytes', 'dpb_gemm_nt', 'dpb_train_forward', 'dpb_train_backward', 'dpb_rows_axpby', 'dpb_weighted_sqdiff', 'dpb_rk45_stage', 'dpb_rk45_scratch_bytes', 'dpb_rk45_error',
            'dpb_pf_ode_rhs', 'dpb_pf_ode_rhs_dim', 'dpb_selfisect_create', 'dpb_selfisect_destroy', 'dpb_selfisect_workspace_bytes',
@@ -126,6 +126,8 @@ def load():
     lib.dpb_affine_cols.argtypes = [vp, i64, vp, vp, vp, i64, i64, C.c_int, C.c_int, f32, vp]
     lib.dpb_axis_to_rot6d_cols.argtypes = [vp, i64, vp, vp, vp, i64, i64, C.c_int, vp]
     lib.dpb_axis_to_rot6d_cols_vjp.argtypes = [vp, i64, vp, vp, i64, vp, i64, i64, C.c_int, vp]
+    lib.dpb_rot6d_to_axis_cols.argtypes = [vp, i64, vp, vp, vp, i64, i64, C.c_int, vp]
+    lib.dpb_rot6d_to_axis_cols_vjp.argtypes = [vp, i64, vp, vp, vp, i64, vp, i64, i64, C.c_int, vp]
     lib.dpb_joint_map_gather.argtypes = [vp, C.c_int, vp, C.c_int, vp, i64, vp]
     lib.dpb_joint_map_scatter.argtypes = [vp, C.c_int, vp, C.c_int, vp, i64, vp]
     lib.dpb_train_create.argtypes = [C.POINTER(vp), i64, C.c_int]

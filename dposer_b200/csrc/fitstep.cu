@@ -10,7 +10,10 @@
 //   affine_cols_kernel                             Posenormalizer z-score (lib/dataset/AMASS.py:187-259)
 //   axis_to_rot6d kernels                          Posenormalizer.offline_normalize(from_axis=True) of a rot6d prior
 //       (run/smplify.py:109-115, lib/utils/transforms.py:237-255) and its vector-Jacobian product
+//   rot6d_to_axis kernels                          Posenormalizer.offline_denormalize(to_axis=True) of a rot6d network's
+//       output (lib/utils/transforms.py:197-234) and its vector-Jacobian product: the auxiliary training loss at 126-D
 //   joint_map kernels                             lib/body_model/smpl.py:70 joints[:, joint_map] and its adjoint
+#include <cfloat>
 #include <cmath>
 
 #include "common.cuh"
@@ -259,6 +262,147 @@ __global__ void __launch_bounds__(256) axis_to_rot6d_vjp_kernel(const float* __r
   o[2] = s * a2 + k.A * w2 + k.B * Ga2;
 }
 
+// ---- normalised rot6d -> axis-angle, one thread per (row, joint): transforms.rot6d_to_axis_angle(x * std + mean) --
+// Gram-Schmidt of the columns a1 = (u0, u2, u4), a2 = (u1, u3, u5), Shepperd's quaternion (pivot: the largest of
+// trace / R00 / R11 / R22, first on ties like argmax), then 2 atan2(|v|, w) v / |v| (2 v below |v| = 1e-12).
+// The frame is evaluated as b1 = a1 / |a1|, b3 = (a1 x a2) / |a1 x a2|, b2 = b3 x b1 -- the same frame as
+// b2 = normalize(a2 - (b1.a2) b1), b3 = b1 x b2 -- in fp64 from u = fma(x, std, mean), then rounded to fp32; the
+// quaternion and the angle follow in fp32.  When a1 and a2 are nearly parallel, the frame is ill-conditioned: an fp32
+// Gram-Schmidt (and an fp32 u alone) errs by eps / sin(a1, a2).  On Gaussian 6-vectors (what an untrained network
+// emits) the torch function in fp32 is up to 2.3e-5 rad off float64 on ~0.1 % of joints.  In fp64 the frame is exact
+// to fp32 rounding at any angle between the columns.
+// Degenerate joints (|a1| or |e| = |a1 x a2| / |a1| below the 1e-12 clamp of F.normalize), non-finite inputs and
+// non-finite results give 0 in the three outputs (and in the six cotangents of the VJP).
+struct Rot6dLog {
+  float b1[3], b2[3], b3[3];
+  float n1, ne, p;      // |a1|, |e|, b1 . a2
+  float phi[3];         // the axis-angle vector
+  float ang, w, n;      // its angle 2 atan2(n, w), the quaternion's scalar part and |v|
+  bool ok;
+};
+
+__device__ __forceinline__ Rot6dLog rot6d_log(const float* __restrict__ x, const float* __restrict__ mean,
+                                              const float* __restrict__ sd) {
+  Rot6dLog o;
+  double a1[3], a2[3];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    a1[k] = fma((double)x[2 * k], (double)sd[2 * k], (double)mean[2 * k]);
+    a2[k] = fma((double)x[2 * k + 1], (double)sd[2 * k + 1], (double)mean[2 * k + 1]);
+  }
+  const double c[3] = {a1[1] * a2[2] - a1[2] * a2[1], a1[2] * a2[0] - a1[0] * a2[2], a1[0] * a2[1] - a1[1] * a2[0]};
+  const double n1 = sqrt(a1[0] * a1[0] + a1[1] * a1[1] + a1[2] * a1[2]);
+  const double nc = sqrt(c[0] * c[0] + c[1] * c[1] + c[2] * c[2]);
+  const double ne = nc / n1;
+  // also false for NaN; the bound on |a1| and |e| keeps 1 / (|a1| |e|) of the VJP finite in fp32
+  o.ok = n1 >= 1e-12 && ne >= 1e-12 && n1 <= FLT_MAX && ne <= FLT_MAX;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    o.b1[k] = (float)(a1[k] / n1);
+    o.b3[k] = (float)(c[k] / nc);
+  }
+  o.n1 = (float)n1;
+  o.ne = (float)ne;
+  o.p = (float)((a1[0] * a2[0] + a1[1] * a2[1] + a1[2] * a2[2]) / n1);
+  o.b2[0] = o.b3[1] * o.b1[2] - o.b3[2] * o.b1[1];
+  o.b2[1] = o.b3[2] * o.b1[0] - o.b3[0] * o.b1[2];
+  o.b2[2] = o.b3[0] * o.b1[1] - o.b3[1] * o.b1[0];
+  // R = [b1 b2 b3] (columns); the quaternion in the torch function's order of operations
+  const float r00 = o.b1[0], r11 = o.b2[1], r22 = o.b3[2];
+  const float d21 = o.b2[2] - o.b3[1], d02 = o.b3[0] - o.b1[2], d10 = o.b1[1] - o.b2[0];
+  const float s01 = o.b2[0] + o.b1[1], s02 = o.b3[0] + o.b1[2], s12 = o.b3[1] + o.b2[2];
+  const float tr = r00 + r11 + r22;
+  int piv = 0;
+  float best = tr;
+  if (r00 > best) { piv = 1; best = r00; }
+  if (r11 > best) { piv = 2; best = r11; }
+  if (r22 > best) piv = 3;
+  float q[4];
+  if (piv == 0) {
+    const float s = sqrtf(fmaxf(1.f + r00 + r11 + r22, 1e-30f)) * 2.f;
+    q[0] = s / 4.f; q[1] = d21 / s; q[2] = d02 / s; q[3] = d10 / s;
+  } else if (piv == 1) {
+    const float s = sqrtf(fmaxf(1.f + r00 - r11 - r22, 1e-30f)) * 2.f;
+    q[0] = d21 / s; q[1] = s / 4.f; q[2] = s01 / s; q[3] = s02 / s;
+  } else if (piv == 2) {
+    const float s = sqrtf(fmaxf(1.f - r00 + r11 - r22, 1e-30f)) * 2.f;
+    q[0] = d02 / s; q[1] = s01 / s; q[2] = s / 4.f; q[3] = s12 / s;
+  } else {
+    const float s = sqrtf(fmaxf(1.f - r00 - r11 + r22, 1e-30f)) * 2.f;
+    q[0] = d10 / s; q[1] = s02 / s; q[2] = s12 / s; q[3] = s / 4.f;
+  }
+  if (q[0] < 0.f) {
+#pragma unroll
+    for (int k = 0; k < 4; ++k) q[k] = -q[k];
+  }
+  o.w = q[0];
+  o.n = sqrtf(q[1] * q[1] + q[2] * q[2] + q[3] * q[3]);
+  o.ang = 2.f * atan2f(o.n, q[0]);
+  const float f = o.n < 1e-12f ? 2.f : o.ang / fmaxf(o.n, 1e-12f);
+#pragma unroll
+  for (int k = 0; k < 3; ++k) o.phi[k] = q[k + 1] * f;
+  o.ok = o.ok && isfinite(o.phi[0]) && isfinite(o.phi[1]) && isfinite(o.phi[2]);
+  return o;
+}
+
+__global__ void __launch_bounds__(256) rot6d_to_axis_kernel(const float* __restrict__ x, int64_t ldx,
+                                                             const float* __restrict__ mean, const float* __restrict__ sd,
+                                                             float* __restrict__ out, int64_t ldo, int64_t rows, int nj) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows * nj) return;
+  const int64_t r = i / nj;
+  const int j = (int)(i % nj);
+  const Rot6dLog L = rot6d_log(x + r * ldx + 6 * j, mean + 6 * j, sd + 6 * j);
+  float* o = out + r * ldo + 3 * j;
+#pragma unroll
+  for (int k = 0; k < 3; ++k) o[k] = L.ok ? L.phi[k] : 0.f;
+}
+
+// With g the cotangent of phi, theta = |phi|, the right-perturbation log-map Jacobian gives the cotangent of the
+// frame rotation delta (dR = R [delta]x):
+//   gd = J_r^-T g = g - phi x g / 2 + c (phi (phi.g) - theta^2 g),   c = 1/theta^2 - (1 + cos t) / (2 t sin t)
+//      = 1/theta^2 - w / (2 theta n)  (from the quaternion: no cancellation of sin against 1 + cos up to pi),
+// and delta = (b3.db2, -b3.db1, b2.db1) with db1 = (I - b1 b1^T) da1 / |a1|, b3.db2 = b3.(da2 - (b1.a2) db1) / |e|:
+//   g_a1 = (gd_z b2 - gd_y b3) / |a1| - gd_x (b1.a2) / (|a1| |e|) b3,   g_a2 = gd_x b3 / |e|,   g_x = g_u * std.
+// Below theta = 0.5, c = 1/12 + theta^2/720 + theta^4/30240 (first dropped term theta^6/1209600, 1.5e-7 of c at 0.5);
+// above, the closed form's error in c theta^2 -- the only way c enters gd -- is a few fp32 ulps of 1, independent of theta.
+__global__ void __launch_bounds__(256) rot6d_to_axis_vjp_kernel(const float* __restrict__ x, int64_t ldx,
+                                                                 const float* __restrict__ mean,
+                                                                 const float* __restrict__ sd, const float* __restrict__ g,
+                                                                 int64_t ldg, float* __restrict__ g_x, int64_t ldgx,
+                                                                 int64_t rows, int nj) {
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= rows * nj) return;
+  const int64_t r = i / nj;
+  const int j = (int)(i % nj);
+  const Rot6dLog L = rot6d_log(x + r * ldx + 6 * j, mean + 6 * j, sd + 6 * j);
+  const float* gr = g + r * ldg + 3 * j;
+  const float g0 = gr[0], g1 = gr[1], g2 = gr[2];
+  const float* f = L.phi;
+  const float t2 = L.ang * L.ang;
+  const float c = L.ang < 0.5f ? 1.f / 12 + t2 * (1.f / 720 + t2 * (1.f / 30240))
+                               : 1.f / t2 - L.w / (2.f * L.ang * L.n);
+  const float fg = f[0] * g0 + f[1] * g1 + f[2] * g2;
+  const float gd0 = g0 - 0.5f * (f[1] * g2 - f[2] * g1) + c * (f[0] * fg - t2 * g0);
+  const float gd1 = g1 - 0.5f * (f[2] * g0 - f[0] * g2) + c * (f[1] * fg - t2 * g1);
+  const float gd2 = g2 - 0.5f * (f[0] * g1 - f[1] * g0) + c * (f[2] * fg - t2 * g2);
+  const float i1 = 1.f / L.n1, ie = 1.f / L.ne;
+  const float k3 = -(gd1 + gd0 * L.p * ie) * i1;     // coefficient of b3 in g_a1
+  const float k2 = gd2 * i1, ka2 = gd0 * ie;
+  float gu[6];
+#pragma unroll
+  for (int k = 0; k < 3; ++k) {
+    gu[2 * k] = k2 * L.b2[k] + k3 * L.b3[k];
+    gu[2 * k + 1] = ka2 * L.b3[k];
+  }
+  bool ok = L.ok;
+#pragma unroll
+  for (int k = 0; k < 6; ++k) ok = ok && isfinite(gu[k]);
+  float* o = g_x + r * ldgx + 6 * j;
+#pragma unroll
+  for (int k = 0; k < 6; ++k) o[k] = ok ? gu[k] * sd[6 * j + k] : 0.f;
+}
+
 // cotangent of mean((x*m - o*m)^2) (nn.MSELoss 'mean' on masked tensors, run/completion.py:197): 2 m^2 (x - o) / n
 __global__ void masked_mse_grad_kernel(const float* __restrict__ x, const float* __restrict__ o,
                                        const float* __restrict__ m, float* __restrict__ g, int64_t n) {
@@ -392,6 +536,36 @@ extern "C" int dpb_axis_to_rot6d_cols_vjp(const float* x, int64_t ldx, const flo
   const int64_t n = rows * n_joints;
   axis_to_rot6d_vjp_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, ldx, sd, g, ldg, g_x, ldgx,
                                                                                           rows, n_joints);
+  DPB_CUDA_CHECK(cudaGetLastError());
+  return DPB_OK;
+}
+
+extern "C" int dpb_rot6d_to_axis_cols(const float* x, int64_t ldx, const float* mean, const float* sd, float* out,
+                                      int64_t ldo, int64_t rows, int n_joints, void* stream) {
+  DPB_REQUIRE(x && mean && sd && out && n_joints > 0 && rows >= 0, "dpb_rot6d_to_axis_cols: bad argument");
+  DPB_REQUIRE(ldx >= 6 * (int64_t)n_joints && ldo >= 3 * (int64_t)n_joints,
+              "dpb_rot6d_to_axis_cols: row strides must cover 6 * n_joints inputs and 3 * n_joints outputs");
+  if (rows == 0) return DPB_OK;
+  PtrDeviceGuard guard(x);
+  const int64_t n = rows * n_joints;
+  rot6d_to_axis_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, ldx, mean, sd, out, ldo, rows,
+                                                                                      n_joints);
+  DPB_CUDA_CHECK(cudaGetLastError());
+  return DPB_OK;
+}
+
+extern "C" int dpb_rot6d_to_axis_cols_vjp(const float* x, int64_t ldx, const float* mean, const float* sd, const float* g,
+                                          int64_t ldg, float* g_x, int64_t ldgx, int64_t rows, int n_joints,
+                                          void* stream) {
+  DPB_REQUIRE(x && mean && sd && g && g_x && n_joints > 0 && rows >= 0, "dpb_rot6d_to_axis_cols_vjp: bad argument");
+  DPB_REQUIRE(ldx >= 6 * (int64_t)n_joints && ldg >= 3 * (int64_t)n_joints && ldgx >= 6 * (int64_t)n_joints,
+              "dpb_rot6d_to_axis_cols_vjp: row strides must cover 6 * n_joints inputs / cotangents and 3 * n_joints "
+              "gradients");
+  if (rows == 0) return DPB_OK;
+  PtrDeviceGuard guard(x);
+  const int64_t n = rows * n_joints;
+  rot6d_to_axis_vjp_kernel<<<(unsigned)((n + 255) / 256), 256, 0, (cudaStream_t)stream>>>(x, ldx, mean, sd, g, ldg, g_x,
+                                                                                          ldgx, rows, n_joints);
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;
 }

@@ -12,7 +12,8 @@ What differs from the reference, by construction:
     passed in (``t=``, ``z=``, ``drop_mask=``) -- that is how the parity tests replay the reference's draws;
   * the auxiliary v2v / j2j loss ("not recommended" in the reference's config) runs as a whole inside ``step_fn``
     (:func:`auxiliary_loss_grad`): the DDIM chain keeps one native engine per network evaluation and is walked backwards
-    by hand; only ``denormalize`` + the body model (a native autograd function) go through torch autograd.
+    by hand; only ``denormalize`` + the body model (a native autograd function) go through torch autograd.  For a rot6d
+    (126-D) network the map to the axis-angle body pose and its Jacobian are kernels (``steps.rot6d_to_axis_cols``).
 """
 import ctypes as C
 
@@ -21,6 +22,7 @@ import torch
 
 from . import _lib as L
 from . import sde_lib
+from . import steps
 from . import utils as mutils
 from .sde_lib import VESDE, VPSDE
 
@@ -347,18 +349,41 @@ def _weighted_sqdiff(p, q, w, scale, want_grad=True):
     return loss, grad
 
 
+def _rot6d_affine(denormalize):
+    """(mean, std) of the rot6d normaliser whose bound ``offline_denormalize`` is ``denormalize``: the form in which the
+    estimate of a rot6d network reaches the body model natively (an arbitrary callable cannot run as a kernel)."""
+    from .misc import Posenormalizer
+    norm = getattr(denormalize, '__self__', None)
+    if not (isinstance(norm, Posenormalizer) and norm.rot_rep == 'rot6d' and
+            getattr(denormalize, '__func__', None) is Posenormalizer.offline_denormalize):
+        raise NotImplementedError("the auxiliary loss of a rot6d (126-D) network maps its estimate to the axis-angle body "
+                                  "pose natively: denormalize must be the offline_denormalize of a "
+                                  f"Posenormalizer(rot_rep='rot6d'), got {denormalize!r}")
+    return norm.column_affine()
+
+
+def _rot6d_pose(x, mean, std):
+    """[B, 63] axis-angle body pose of the normalised rot6d rows x [B, 126]."""
+    out = torch.empty(x.shape[0], x.shape[1] // 2, device=x.device)
+    steps.rot6d_to_axis_cols(x, 0, mean, std, out)
+    return out
+
+
 def auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_steps=5, reduce_mean=False, continuous=True,
                         eps=1e-5, t=None, z=None, drop_mask=None, score_scale=1.0):
     """Loss of get_step_fn(auxiliary_loss=True) (losses.py:244-258) and every parameter gradient, without autograd through
     the network: ``denoise_steps`` network evaluations of multi_step_denoise (each on its own native engine, activations
     kept), the estimate through ``denormalize`` + ``body_model`` (torch autograd over the native LBS function), weighted
     v2v / j2j terms, then the chain backwards -- every evaluation's backward adds into the same flat gradient buffers.
+    A rot6d (126-D) network needs ``denormalize`` = the ``offline_denormalize`` of a ``Posenormalizer(rot_rep='rot6d')``:
+    its (mean, std) feed the native rot6d -> axis-angle map (``offline_denormalize(x, to_axis=True)``), whose
+    vector-Jacobian product hands the body model's cotangent back to the chain; autograd then starts at the axis pose.
     ``drop_mask``: [denoise_steps, 5, B, 1024] keep-masks (parity mode); ``score_scale`` multiplies the score-matching term
     (tests switch it off to look at the body-model terms alone).  Returns a dict of [] device tensors."""
     from .misc import linear_interpolation
-    if getattr(model, 'is_rot6d', False):
-        raise NotImplementedError('the auxiliary v2v / j2j loss is built for the 63-D axis-angle network: a rot6d (126-D) '
-                                  'network would need a rot6d -> axis-angle map under the body model')
+    mutils.rot6d_needs_cuda(model, next(model.parameters()).is_cuda, 'the auxiliary loss')
+    affine = _rot6d_affine(denormalize) if getattr(model, 'is_rot6d', False) else None
+    model.check_width(batch, 'batch')
     L.require_cuda(batch, 'batch')
     lib = L.load()
     dev, B, N = batch.device, batch.shape[0], int(denoise_steps)
@@ -395,11 +420,13 @@ def auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_step
         c1s.append(up(c1))
         c2s.append(up(-(s_b - c1 * s_c) * cf[:, 5] * s_c))          # x' = c1 x + (s_b - c1 s_c) noise, noise = -m res s_c
     ones = torch.ones(B, device=dev)
+    if affine is not None:
+        affine = [up(v) for v in affine]
     # ---- forward chain
     batch = batch.detach().to(torch.float32).contiguous()
     if z is None:
         z = torch.empty(B, D, device=dev)
-        L.check(lib.dpb_normal_fill(L.ptr(z), B, C.c_uint64(_draw_seed()), C.c_uint64(0), 0, st))
+        L.check(lib.dpb_normal_fill_dim(L.ptr(z), B, C.c_uint64(_draw_seed()), C.c_uint64(0), 0, D, st))
     else:
         z = up(z)
     x = _rows_axpby(up(mean_c), batch, up(std0), z)                                    # perturbed data, losses.py:113-115
@@ -421,15 +448,22 @@ def auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_step
     # ---- body-model terms on the estimate (torch autograd over denormalize + the native LBS function)
     wdev = up(weight)
     with torch.no_grad():                      # the target first: the body model keeps ONE saved forward state per module
-        gt = body_model(pose_body=denormalize(batch))
+        gt = body_model(pose_body=denormalize(batch) if affine is None else _rot6d_pose(batch, *affine))
         gt_v, gt_j = gt.v.clone(), gt.Jtr.clone()
     with torch.enable_grad():
-        leaf = x.detach().requires_grad_(True)
-        pred = body_model(pose_body=denormalize(leaf))
+        if affine is None:
+            leaf = x.detach().requires_grad_(True)
+            pose = denormalize(leaf)
+        else:                                  # rot6d: autograd starts at the axis pose, the map's VJP is a kernel
+            leaf = pose = _rot6d_pose(x, *affine).requires_grad_(True)
+        pred = body_model(pose_body=pose)
         loss_v2v, g_v = _weighted_sqdiff(gt_v, pred.v.detach().contiguous(), wdev, 1.0 / (B * pred.v.shape[1]))
         loss_j2j, g_j = _weighted_sqdiff(gt_j, pred.Jtr.detach().contiguous(), wdev, 1.0 / (B * pred.Jtr.shape[1]))
         torch.autograd.backward([pred.v, pred.Jtr], [g_v.view_as(pred.v), g_j.view_as(pred.Jtr)])
     g_x = leaf.grad.contiguous()
+    if affine is not None:
+        g_pose, g_x = g_x, torch.empty(B, D, device=dev)
+        steps.rot6d_to_axis_cols_vjp(x, 0, *affine, g_pose, g_x)
     # ---- chain backwards: the first call overwrites the gradients, the others add
     for i in reversed(range(N)):
         g_res = _rows_axpby(c2s[i], g_x, ones, g_res_score) if i == 0 else _rows_axpby(c2s[i], g_x)
@@ -497,8 +531,10 @@ def get_step_fn(sde, train, optimize_fn=None, reduce_mean=False, continuous=True
     from . import dist as D
     if auxiliary_loss:
         assert denormalize is not None and body_model is not None
-        if rot_rep != 'axis':
-            raise NotImplementedError("the auxiliary loss is built for rot_rep='axis' (the 63-D network input)")
+        if rot_rep not in ('axis', 'rot6d'):
+            raise ValueError(f"rot_rep must be 'axis' or 'rot6d', got {rot_rep!r}")
+        if rot_rep == 'rot6d':
+            _rot6d_affine(denormalize)
         if not continuous or likelihood_weighting:
             raise NotImplementedError('the auxiliary loss goes with the continuous, unweighted SDE loss')
     if continuous:
@@ -531,6 +567,10 @@ def get_step_fn(sde, train, optimize_fn=None, reduce_mean=False, continuous=True
             state['step'] += 1
             model.mark_updated()
         elif train and auxiliary_loss:
+            mutils.rot6d_needs_cuda(model, next(model.parameters()).is_cuda, 'the auxiliary loss')
+            want = L.POSE_DIM_ROT6D if rot_rep == 'rot6d' else L.POSE_DIM
+            if model.pose_width != want:
+                raise ValueError(f'rot_rep={rot_rep!r} needs a {want}-D score network, got a {model.pose_width}-D one')
             optimizer = state['optimizer']
             ld = auxiliary_loss_grad(model, sde, batch, denormalize, body_model, denoise_steps=denoise_steps,
                                      reduce_mean=reduce_mean, **draws)

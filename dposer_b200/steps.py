@@ -115,12 +115,13 @@ def affine_cols(x, off, ld, mean, std, out, inverse=False, out_off=0, out_ld=Non
                                      float(squash), L.current_stream(out.device)))
 
 
-def _rot6d_operands(x, off, rows, nj, cols):
-    """Checks of the two rot6d calls, all before any library call: ``x`` [rows, ld] holds 3 * nj axis-angle columns
-    from ``off``; ``cols`` lists (name, tensor, width): a [rows, width] matrix, or for width None the 6 * nj per-column
-    statistics.  Shapes first (ValueError), then devices (RuntimeError for a CPU tensor)."""
-    if x.dim() != 2 or nj < 1 or x.shape[0] != rows or off < 0 or off + 3 * nj > x.shape[1]:
-        raise ValueError(f'x: expected {rows} rows holding {3 * nj} axis-angle columns from column {off}, '
+def _rot6d_operands(x, off, rows, nj, per_joint, cols):
+    """Checks of the rot6d calls, all before any library call: ``x`` [rows, ld] holds ``per_joint`` * nj input columns
+    (3: axis-angle, 6: rot6d) from ``off``; ``cols`` lists (name, tensor, width): a [rows, width] matrix, or for width
+    None the 6 * nj per-column statistics.  Shapes first (ValueError), then devices (RuntimeError for a CPU tensor)."""
+    what = 'axis-angle' if per_joint == 3 else 'rot6d'
+    if x.dim() != 2 or nj < 1 or x.shape[0] != rows or off < 0 or off + per_joint * nj > x.shape[1]:
+        raise ValueError(f'x: expected {rows} rows holding {per_joint * nj} {what} columns from column {off}, '
                          f'got {list(x.shape)}')
     for name, t, width in cols:
         if (t.numel() != 6 * nj) if width is None else (list(t.shape) != [rows, width]):
@@ -141,7 +142,7 @@ def axis_to_rot6d_cols(x, off, mean, std, out):
     nj = out.shape[-1] // 6
     if out.dim() != 2 or out.shape[1] != 6 * nj:
         raise ValueError(f'out: expected 6 columns per joint, got {list(out.shape)}')
-    _rot6d_operands(x, off, out.shape[0], nj, [('out', out, 6 * nj), ('mean', mean, None), ('std', std, None)])
+    _rot6d_operands(x, off, out.shape[0], nj, 3, [('out', out, 6 * nj), ('mean', mean, None), ('std', std, None)])
     L.check(L.load().dpb_axis_to_rot6d_cols(_p(x, off), x.shape[1], L.ptr(mean), L.ptr(std), L.ptr(out), out.shape[1],
                                             x.shape[0], nj, L.current_stream(x.device)))
 
@@ -152,9 +153,32 @@ def axis_to_rot6d_cols_vjp(x, off, std, g, g_x):
     nj = g.shape[-1] // 6
     if g.dim() != 2 or g.shape[1] != 6 * nj:
         raise ValueError(f'g: expected 6 columns per joint, got {list(g.shape)}')
-    _rot6d_operands(x, off, g.shape[0], nj, [('g', g, 6 * nj), ('g_x', g_x, 3 * nj), ('std', std, None)])
+    _rot6d_operands(x, off, g.shape[0], nj, 3, [('g', g, 6 * nj), ('g_x', g_x, 3 * nj), ('std', std, None)])
     L.check(L.load().dpb_axis_to_rot6d_cols_vjp(_p(x, off), x.shape[1], L.ptr(std), L.ptr(g), g.shape[1], L.ptr(g_x),
                                                 g_x.shape[1], x.shape[0], nj, L.current_stream(x.device)))
+
+
+def rot6d_to_axis_cols(x, off, mean, std, out):
+    """out[r, 3j:3j+3] = rot6d_to_axis_angle(x[r, off+6j : off+6j+6] * std[6j:6j+6] + mean[6j:6j+6]) for the
+    out.shape[1] / 3 joints (dpb_rot6d_to_axis_cols): the body pose of a rot6d network's normalised output."""
+    nj = out.shape[-1] // 3
+    if out.dim() != 2 or out.shape[1] != 3 * nj:
+        raise ValueError(f'out: expected 3 columns per joint, got {list(out.shape)}')
+    _rot6d_operands(x, off, out.shape[0], nj, 6, [('out', out, 3 * nj), ('mean', mean, None), ('std', std, None)])
+    L.check(L.load().dpb_rot6d_to_axis_cols(_p(x, off), x.shape[1], L.ptr(mean), L.ptr(std), L.ptr(out), out.shape[1],
+                                            x.shape[0], nj, L.current_stream(x.device)))
+
+
+def rot6d_to_axis_cols_vjp(x, off, mean, std, g, g_x):
+    """g_x [rows, 6 n] = the cotangent of x[:, off:off+6n] given g [rows, 3 n], the cotangent of rot6d_to_axis_cols'
+    output (dpb_rot6d_to_axis_cols_vjp)."""
+    nj = g.shape[-1] // 3
+    if g.dim() != 2 or g.shape[1] != 3 * nj:
+        raise ValueError(f'g: expected 3 columns per joint, got {list(g.shape)}')
+    _rot6d_operands(x, off, g.shape[0], nj, 6, [('g', g, 3 * nj), ('g_x', g_x, 6 * nj), ('mean', mean, None),
+                                                ('std', std, None)])
+    L.check(L.load().dpb_rot6d_to_axis_cols_vjp(_p(x, off), x.shape[1], L.ptr(mean), L.ptr(std), L.ptr(g), g.shape[1],
+                                                L.ptr(g_x), g_x.shape[1], x.shape[0], nj, L.current_stream(x.device)))
 
 
 def motion_loss(lbs, target, seq_len, n_data, w_temp, w_data, seq_terms=None):

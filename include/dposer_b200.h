@@ -330,6 +330,21 @@ int dpb_axis_to_rot6d_cols(const float* x, int64_t ldx, const float* mean, const
  * from x (nothing is saved by the forward); NaN in a joint's 3 entries when its input is non-finite. */
 int dpb_axis_to_rot6d_cols_vjp(const float* x, int64_t ldx, const float* std, const float* g, int64_t ldg, float* g_x,
                                int64_t ldgx, int64_t rows, int n_joints, void* stream);
+/* The other way, the body pose of a rot6d (126-D) network's normalised output:
+ * Posenormalizer.offline_denormalize(x, to_axis=True) (lib/utils/transforms.py:197-234), on strided views.  For joint j
+ * of row r, u = x[r*ldx + 6j .. 6j+5] * std[6j..] + mean[6j..] and
+ *   out[r*ldo + 3j .. 3j+2] = rot6d_to_axis_angle(u):
+ * Gram-Schmidt of the columns a1 = (u0, u2, u4), a2 = (u1, u3, u5) into R = [b1 b2 b3], Shepperd's quaternion (pivot:
+ * the largest of trace / R00 / R11 / R22), then 2 atan2(|v|, w) v / |v| (2 v for |v| < 1e-12); the angle is in [0, pi].
+ * mean / std [6 n_joints] as in dpb_axis_to_rot6d_cols.  Degenerate joints -- |a1| or |a2 - (b1.a2) b1| below 1e-12
+ * (F.normalize's clamp) -- non-finite inputs and non-finite results give 0 in the joint's 3 outputs. */
+int dpb_rot6d_to_axis_cols(const float* x, int64_t ldx, const float* mean, const float* std, float* out, int64_t ldo,
+                           int64_t rows, int n_joints, void* stream);
+/* Its vector-Jacobian product: g_x[r*ldgx + 6j + k] = sum_i g[r*ldg + 3j+i] d out_i / d x_k, recomputed from x (nothing
+ * is saved by the forward); 0 in a joint's 6 entries wherever the forward gives 0 by the rule above, or the result is
+ * not finite. */
+int dpb_rot6d_to_axis_cols_vjp(const float* x, int64_t ldx, const float* mean, const float* std, const float* g,
+                               int64_t ldg, float* g_x, int64_t ldgx, int64_t rows, int n_joints, void* stream);
 /* out[r,c] = w0 x[r-1,c] + w1 x[r,c] + w2 x[r+1,c] inside each sequence of seq_len rows, zero-padded at its ends
  * (gaussian_smoothing(window_size=3), lib/utils/misc.py:84-95, per sequence as in run/motion_denoising.py:281-285);
  * keep_ends != 0 copies the first and last row of every sequence instead.  out must not alias x. */
