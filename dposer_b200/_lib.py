@@ -41,18 +41,18 @@ class BodyTensors(C.Structure):
                 ('n_lmk', C.c_int), ('lmk_faces', _i32p), ('lmk_bary', _f32p)]
 
 
-EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create', 'dpb_score_create_dim',
+EXPORTS = ['dpb_version', 'dpb_last_error', 'dpb_device_info', 'dpb_score_create_dim',
            'dpb_score_pose_dim', 'dpb_normal_fill_dim', 'dpb_langevin_norms_dim', 'dpb_langevin_update_dim', 'dpb_score_destroy',
            'dpb_score_time_table', 'dpb_score_workspace_bytes', 'dpb_score_forward', 'dpb_score_jvp',
            'dpb_score_jvp_workspace_bytes', 'dpb_sampler_run_pc', 'dpb_sampler_pc_workspace_bytes', 'dpb_sampler_run',
-           'dpb_langevin_norms', 'dpb_langevin_update', 'dpb_normal_fill', 'dpb_prior_loss', 'dpb_lbs_create',
+           'dpb_prior_loss', 'dpb_lbs_create',
            'dpb_lbs_destroy', 'dpb_lbs_set_const_tail', 'dpb_lbs_num_joints_out', 'dpb_lbs_workspace_bytes', 'dpb_lbs_forward',
            'dpb_lbs_backward', 'dpb_lbs_backward_scratch_bytes', 'dpb_lbs_backward_scratch_bytes_joints', 'dpb_apd_partial', 'dpb_mean_point_error', 'dpb_fit_loss',
            'dpb_motion_loss', 'dpb_camera_fit_loss', 'dpb_adam_step', 'dpb_affine_cols', 'dpb_axis_to_rot6d_cols',
            'dpb_axis_to_rot6d_cols_vjp', 'dpb_rot6d_to_axis_cols', 'dpb_rot6d_to_axis_cols_vjp', 'dpb_joint_map_gather',
-           'dpb_joint_map_scatter', 'dpb_masked_mse_grad', 'dpb_seq_smooth3', 'dpb_train_create', 'dpb_train_create_dim', 'dpb_train_destroy',
+           'dpb_joint_map_scatter', 'dpb_masked_mse_grad', 'dpb_seq_smooth3', 'dpb_train_create_dim', 'dpb_train_destroy',
            'dpb_train_loss_grad', 'dpb_train_adam_scratch_bytes', 'dpb_train_grad_norm', 'dpb_train_adam', 'dpb_ema_update', 'dpb_train_set_seed_pointer', 'dpb_gemm_nt_workspace_bytes', 'dpb_gemm_nt', 'dpb_train_forward', 'dpb_train_backward', 'dpb_rows_axpby', 'dpb_weighted_sqdiff', 'dpb_rk45_stage', 'dpb_rk45_scratch_bytes', 'dpb_rk45_error',
-           'dpb_pf_ode_rhs', 'dpb_pf_ode_rhs_dim', 'dpb_selfisect_create', 'dpb_selfisect_destroy', 'dpb_selfisect_workspace_bytes',
+           'dpb_pf_ode_rhs_dim', 'dpb_selfisect_create', 'dpb_selfisect_destroy', 'dpb_selfisect_workspace_bytes',
            'dpb_selfisect_run', 'dpb_procrustes']
 
 _lib = None
@@ -77,7 +77,6 @@ def load():
     lib.dpb_version.restype = C.c_int
     lib.dpb_last_error.restype = C.c_char_p
     lib.dpb_device_info.argtypes = [C.c_int, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]
-    lib.dpb_score_create.argtypes = [C.POINTER(vp), C.POINTER(ScoreWeights), C.c_int]
     lib.dpb_score_create_dim.argtypes = [C.POINTER(vp), C.POINTER(ScoreWeights), C.c_int, C.c_int]
     lib.dpb_score_pose_dim.argtypes = [vp]
     lib.dpb_score_destroy.argtypes = [vp]
@@ -87,9 +86,6 @@ def load():
     lib.dpb_score_forward.argtypes = [vp, vp, vp, vp, vp, f32, vp, i64, C.c_int, vp, sz, vp]
     lib.dpb_sampler_run.argtypes = [vp, vp, C.POINTER(StepTables), vp, vp, vp, u64, u64, vp, vp, i64, C.c_int, vp,
                                     sz, vp]
-    lib.dpb_langevin_norms.argtypes = [vp, vp, vp, i64, vp]
-    lib.dpb_langevin_update.argtypes = [vp, vp, vp, vp, vp, f32, f32, i64, vp]
-    lib.dpb_normal_fill.argtypes = [vp, i64, u64, u64, C.c_int, vp]
     lib.dpb_langevin_norms_dim.argtypes = [vp, vp, vp, i64, C.c_int, vp]
     lib.dpb_langevin_update_dim.argtypes = [vp, vp, vp, vp, vp, f32, f32, i64, C.c_int, vp]
     lib.dpb_normal_fill_dim.argtypes = [vp, i64, u64, u64, C.c_int, C.c_int, vp]
@@ -130,7 +126,6 @@ def load():
     lib.dpb_rot6d_to_axis_cols_vjp.argtypes = [vp, i64, vp, vp, vp, i64, vp, i64, i64, C.c_int, vp]
     lib.dpb_joint_map_gather.argtypes = [vp, C.c_int, vp, C.c_int, vp, i64, vp]
     lib.dpb_joint_map_scatter.argtypes = [vp, C.c_int, vp, C.c_int, vp, i64, vp]
-    lib.dpb_train_create.argtypes = [C.POINTER(vp), i64, C.c_int]
     lib.dpb_train_create_dim.argtypes = [C.POINTER(vp), i64, C.c_int, C.c_int]
     lib.dpb_train_destroy.argtypes = [vp]
     lib.dpb_train_loss_grad.argtypes = [vp, C.POINTER(ScoreWeights), C.POINTER(ScoreWeights), vp, vp, vp, vp, f32, u64, vp,
@@ -151,7 +146,6 @@ def load():
     lib.dpb_rk45_stage.argtypes = [vp, vp, i64, f64, C.c_int, vp, vp, i64, vp]
     lib.dpb_rk45_scratch_bytes.restype = sz
     lib.dpb_rk45_error.argtypes = [vp, vp, vp, i64, f64, f64, f64, vp, vp]
-    lib.dpb_pf_ode_rhs.argtypes = [vp, vp, vp, vp, f32, f32, vp, i64, vp]
     lib.dpb_pf_ode_rhs_dim.argtypes = [vp, vp, vp, vp, f32, f32, vp, i64, C.c_int, vp]
     lib.dpb_mean_point_error.argtypes = [vp, vp, i64, C.c_int, vp, C.c_int, vp, vp]
     lib.dpb_selfisect_create.argtypes = [C.POINTER(vp), _i32p, C.c_int, C.c_int, C.c_int]

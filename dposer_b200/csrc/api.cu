@@ -63,17 +63,17 @@ static int up_f32(float** dst, const float* src, size_t n) {
 extern "C" int dpb_score_create_dim(dpb_score_t** out, const dpb_score_weights* w, int pose_dim, int device) {
   if (pose_dim != DPB_POSE_DIM && pose_dim != DPB_POSE_DIM_ROT6D)
     return fail(DPB_EUNSUPPORTED, "dpb_score_create_dim: pose_dim must be 63 (axis-angle) or 126 (rot6d)");
-  if (!out || !w) return fail(DPB_EINVAL, "dpb_score_create: null argument");
+  if (!out || !w) return fail(DPB_EINVAL, "dpb_score_create_dim: null argument");
   const void* req[] = {w->pre_w, w->pre_b, w->pre_t_w, w->pre_t_b, w->pre_gn_w, w->pre_gn_b, w->temb_w, w->temb_b,
                        w->post_w, w->post_b, w->emb_freqs};
-  for (const void* p : req) DPB_REQUIRE(p, "dpb_score_create: missing weight pointer");
+  for (const void* p : req) DPB_REQUIRE(p, "dpb_score_create_dim: missing weight pointer");
   for (int i = 0; i < 4; ++i)
     DPB_REQUIRE(w->blk_w[i] && w->blk_b[i] && w->blk_t_w[i] && w->blk_t_b[i] && w->blk_gn_w[i] && w->blk_gn_b[i],
-                "dpb_score_create: missing block weight pointer");
+                "dpb_score_create_dim: missing block weight pointer");
   int sm = 0, maj = 0, mnr = 0;
   int rc = dpb_device_info(device, &sm, &maj, &mnr);
   if (rc != DPB_OK) return rc;
-  if (maj != 10) return fail(DPB_ECUDA, "dpb_score_create: device is not sm_100 (B200) class");
+  if (maj != 10) return fail(DPB_ECUDA, "dpb_score_create_dim: device is not sm_100 (B200) class");
   DeviceGuard guard(device);
   dpb_score* h = new dpb_score();
   h->device = device;
@@ -116,10 +116,6 @@ extern "C" int dpb_score_create_dim(dpb_score_t** out, const dpb_score_weights* 
   }
   *out = h;
   return DPB_OK;
-}
-
-extern "C" int dpb_score_create(dpb_score_t** out, const dpb_score_weights* w, int device) {
-  return dpb_score_create_dim(out, w, DPB_POSE_DIM, device);
 }
 
 extern "C" int dpb_score_pose_dim(dpb_score_t* h) {

@@ -125,7 +125,7 @@ extern "C" int dpb_pf_ode_rhs_dim(const float* x, const float* score, const floa
                                   float* k_out, int64_t B, int pose_dim, void* stream) {
   if (pose_dim != DPB_POSE_DIM && pose_dim != DPB_POSE_DIM_ROT6D)
     return fail(DPB_EUNSUPPORTED, "dpb_pf_ode_rhs_dim: pose_dim must be 63 (axis-angle) or 126 (rot6d)");
-  DPB_REQUIRE(x && score && k_out && B > 0 && (!jv || eps), "dpb_pf_ode_rhs: bad argument");
+  DPB_REQUIRE(x && score && k_out && B > 0 && (!jv || eps), "dpb_pf_ode_rhs_dim: bad argument");
   PtrDeviceGuard guard(x);
   const unsigned grid = (unsigned)((B + 7) / 8);
   cudaStream_t st = (cudaStream_t)stream;
@@ -133,9 +133,4 @@ extern "C" int dpb_pf_ode_rhs_dim(const float* x, const float* score, const floa
   else rk::pf_rhs_kernel<D><<<grid, 256, 0, st>>>(x, score, jv, eps, fx, g2, k_out, B);
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;
-}
-
-extern "C" int dpb_pf_ode_rhs(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2,
-                              float* k_out, int64_t B, void* stream) {
-  return dpb_pf_ode_rhs_dim(x, score, jv, eps, fx, g2, k_out, B, DPB_POSE_DIM, stream);
 }

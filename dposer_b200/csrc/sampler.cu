@@ -291,7 +291,7 @@ extern "C" int dpb_langevin_norms_dim(const float* grad, const float* noise, flo
                                       void* stream) {
   const int dp = dpb::dp_of_dim(pose_dim);
   if (!dp) return dpb::fail(DPB_EUNSUPPORTED, "dpb_langevin_norms_dim: pose_dim must be 63 or 126");
-  if (!grad || !noise || !sums || B <= 0) return dpb::fail(DPB_EINVAL, "dpb_langevin_norms: bad argument");
+  if (!grad || !noise || !sums || B <= 0) return dpb::fail(DPB_EINVAL, "dpb_langevin_norms_dim: bad argument");
   dpb::PtrDeviceGuard guard(grad);
   DPB_BY_WIDTH(dp, (dpb::langevin_norms_kernel<W><<<dpb::blocks_for(B, 8), 256, 0, (cudaStream_t)stream>>>(grad, noise,
                                                                                                           sums, B)));
@@ -299,16 +299,12 @@ extern "C" int dpb_langevin_norms_dim(const float* grad, const float* noise, flo
   return DPB_OK;
 }
 
-extern "C" int dpb_langevin_norms(const float* grad, const float* noise, float* sums, int64_t B, void* stream) {
-  return dpb_langevin_norms_dim(grad, noise, sums, B, DPB_POSE_DIM, stream);
-}
-
 extern "C" int dpb_langevin_update_dim(float* x_io, float* x_mean, const float* grad, const float* noise,
                                        const float* sums, float snr, float alpha, int64_t B, int pose_dim,
                                        void* stream) {
   const int dp = dpb::dp_of_dim(pose_dim);
   if (!dp) return dpb::fail(DPB_EUNSUPPORTED, "dpb_langevin_update_dim: pose_dim must be 63 or 126");
-  if (!x_io || !grad || !noise || !sums || B <= 0) return dpb::fail(DPB_EINVAL, "dpb_langevin_update: bad argument");
+  if (!x_io || !grad || !noise || !sums || B <= 0) return dpb::fail(DPB_EINVAL, "dpb_langevin_update_dim: bad argument");
   dpb::PtrDeviceGuard guard(x_io);
   DPB_BY_WIDTH(dp, (dpb::langevin_update_kernel<W><<<dpb::blocks_for(B * pose_dim, 256), 256, 0, (cudaStream_t)stream>>>(
                        x_io, x_mean, grad, noise, sums, snr, alpha, B)));
@@ -316,23 +312,14 @@ extern "C" int dpb_langevin_update_dim(float* x_io, float* x_mean, const float* 
   return DPB_OK;
 }
 
-extern "C" int dpb_langevin_update(float* x_io, float* x_mean, const float* grad, const float* noise,
-                                   const float* sums, float snr, float alpha, int64_t B, void* stream) {
-  return dpb_langevin_update_dim(x_io, x_mean, grad, noise, sums, snr, alpha, B, DPB_POSE_DIM, stream);
-}
-
 extern "C" int dpb_normal_fill_dim(float* out, int64_t B, uint64_t seed, uint64_t step, int slot, int pose_dim,
                                    void* stream) {
   const int dp = dpb::dp_of_dim(pose_dim);
   if (!dp) return dpb::fail(DPB_EUNSUPPORTED, "dpb_normal_fill_dim: pose_dim must be 63 or 126");
-  if (!out || B <= 0) return dpb::fail(DPB_EINVAL, "dpb_normal_fill: bad argument");
+  if (!out || B <= 0) return dpb::fail(DPB_EINVAL, "dpb_normal_fill_dim: bad argument");
   dpb::PtrDeviceGuard guard(out);
   DPB_BY_WIDTH(dp, (dpb::normal_fill_kernel<W><<<dpb::blocks_for(B * (W / 4), 256), 256, 0, (cudaStream_t)stream>>>(
                        out, B, seed, (uint32_t)step, (uint32_t)slot)));
   DPB_CUDA_CHECK(cudaGetLastError());
   return DPB_OK;
-}
-
-extern "C" int dpb_normal_fill(float* out, int64_t B, uint64_t seed, uint64_t step, int slot, void* stream) {
-  return dpb_normal_fill_dim(out, B, seed, step, slot, DPB_POSE_DIM, stream);
 }

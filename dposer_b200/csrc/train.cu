@@ -331,7 +331,7 @@ using namespace dpb;
 extern "C" int dpb_train_create_dim(dpb_train** out, int64_t batch, int pose_dim, int device) {
   if (pose_dim != DPB_POSE_DIM && pose_dim != DPB_POSE_DIM_ROT6D)
     return fail(DPB_EUNSUPPORTED, "dpb_train_create_dim: pose_dim must be 63 (axis-angle) or 126 (rot6d)");
-  DPB_REQUIRE(out && batch > 0, "dpb_train_create: bad argument");
+  DPB_REQUIRE(out && batch > 0, "dpb_train_create_dim: bad argument");
   DeviceGuard guard(device);
   int rc = gemm_tc_init();
   if (rc != DPB_OK) return rc;
@@ -343,7 +343,7 @@ extern "C" int dpb_train_create_dim(dpb_train** out, int64_t batch, int pose_dim
   h->Bp = (batch + 63) / 64 * 64;
   h->pool_bytes = trn::layout(h, nullptr, ~(size_t)0);
   cudaError_t e = cudaMalloc((void**)&h->pool, h->pool_bytes);
-  if (e != cudaSuccess) { delete h; return fail(DPB_ENOMEM, std::string("dpb_train_create: ") + cudaGetErrorString(e)); }
+  if (e != cudaSuccess) { delete h; return fail(DPB_ENOMEM, std::string("dpb_train_create_dim: ") + cudaGetErrorString(e)); }
   cudaMemset(h->pool, 0, h->pool_bytes);                  // operand pads (k >= K, rows >= valid) stay zero for good
   trn::layout(h, h->pool, h->pool_bytes);
   cudaStreamCreateWithFlags(&h->side, cudaStreamNonBlocking);
@@ -351,10 +351,6 @@ extern "C" int dpb_train_create_dim(dpb_train** out, int64_t batch, int pose_dim
   cudaEventCreateWithFlags(&h->ev_join, cudaEventDisableTiming);
   *out = h;
   return DPB_OK;
-}
-
-extern "C" int dpb_train_create(dpb_train** out, int64_t batch, int device) {
-  return dpb_train_create_dim(out, batch, DPB_POSE_DIM, device);
 }
 
 extern "C" int dpb_train_set_seed_pointer(dpb_train* h, const uint64_t* seed_dev) {

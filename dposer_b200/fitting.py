@@ -13,27 +13,22 @@ the native kernels by hand (``steps.py``): normalise -> prior loss + closed-form
 kernels (value + cotangents) -> LBS backward -> fused Adam.  With ``graphs=True`` every step index is captured once
 into a CUDA graph and replayed for every further batch of independent problems that reuses the buffers.
 
-The prior's input follows the score network's width, chosen once when the buffers are set up:
-
-* 63-D (axis-angle) network: x0 = (pose - mean_poses) / std_poses, and Adam scales the prior's gradient by 1 / std.
-* 126-D (rot6d) network: x0 = normalize(axis_angle_to_rot6d(pose)) with the normaliser's active rule
-  (``Posenormalizer.column_affine``), and the prior's gradient returns to the axis-angle pose through the Jacobian of
-  that map (``steps.axis_to_rot6d_cols`` / ``axis_to_rot6d_cols_vjp``).  This is what ``prior.DPoser.forward`` (and
-  the reference's SMPLify prior, run/smplify.py:109-115) computes.  This project applies the same input to the
-  motion-denoising prior: the reference's motion loop normalises without ``from_axis`` (run/motion_denoising.py:238),
-  so it cannot take a rot6d network at all.
+The prior's input follows the score network's width (``steps.PriorInput``, built once with the buffers): a 63-D
+(axis-angle) network takes the z-scored pose, a 126-D (rot6d) network normalize(axis_angle_to_rot6d(pose)), which is
+what ``prior.DPoser.forward`` (and the reference's SMPLify prior, run/smplify.py:109-115) computes.  This project applies
+the same input to the motion-denoising prior: the reference's motion loop normalises without ``from_axis``
+(run/motion_denoising.py:238), so it cannot take a rot6d network at all.
 
 The normaliser must match the network: a rot6d network with an axis normaliser, or the reverse, raises ValueError; a
 rot6d network with a normaliser that has no ``rot_rep`` (no rot6d statistics) raises NotImplementedError.
 """
-import math
-
 import numpy as np
 import torch
 
 from . import _lib as L
 from . import steps as S
 from . import utils as mutils
+from .misc import quan_t
 from .prior import MotionPrior
 
 # constants.JOINT_IDS of ['OP Neck', 'OP RHip', 'OP LHip', 'Right Hip', 'Left Hip'] (run/smplify.py:136-137)
@@ -55,17 +50,6 @@ def _prior_input(model, normalizer, who):
         raise ValueError(f'{who}: a {model.pose_width}-D score network needs a Posenormalizer(rot_rep={want!r}), '
                          f'got rot_rep={rep!r}')
     return rot6d
-
-
-def _quan_t(strategy, N, total, step, trun, sample_time, offset):
-    """run/motion_denoising.py:240-247 / run/smplify.py:153-166 / run/completion.py:183-191."""
-    if strategy == '1':
-        return int(torch.randint(N, [1]))
-    if strategy == '2':
-        return int(sample_time)
-    if strategy == '3':
-        return N - math.floor(torch.tensor(total - step - 1) * (N / (trun * total))) - offset
-    raise NotImplementedError('unsupported time sampling strategy')
 
 
 class MotionDenoise(MotionPrior):
@@ -107,17 +91,10 @@ class MotionDenoise(MotionPrior):
         core = self.body_model.core
         rows = self.batch_size
         f = lambda *s: torch.zeros(*s, dtype=torch.float32, device=dev)   # noqa: E731
-        pw = self.model.pose_width
-        b = dict(dev=dev, full_pose=f(rows, core.J * 3), shape=f(rows, core.S), x0=f(rows, pw), target=f(rows, 22, 3),
-                 z=f(rows, pw), lbs=S.LbsStep(core, rows, dev, need_verts=True),
-                 prior=S.PriorStep(self.model, self.sde, self.continuous, rows, dev), graphs=None, sched_key=None, seed=0)
-        if self.rot6d:
-            mean, std = self.Normalizer.column_affine()
-            b['g_axis'] = f(rows, 63)                   # the prior's gradient w.r.t. the axis-angle body pose
-        else:
-            mean, std = self.Normalizer.mean_poses, self.Normalizer.std_poses
-        b['mean'], b['std'] = mean.to(dev).float().contiguous(), std.to(dev).float().contiguous()
-        b['inv_std'] = None if self.rot6d else (1.0 / b['std']).contiguous()
+        b = dict(dev=dev, full_pose=f(rows, core.J * 3), shape=f(rows, core.S), target=f(rows, 22, 3),
+                 z=f(rows, self.model.pose_width), lbs=S.LbsStep(core, rows, dev, need_verts=True),
+                 prior=S.PriorStep(self.model, self.sde, self.continuous, rows, dev),
+                 prior_input=S.PriorInput(self.model, self.Normalizer, rows, dev), graphs=None, sched_key=None, seed=0)
         b['opt'] = S.Adam(b['full_pose'], 3, 63, 0.03)
         self._bufs = b
         return b
@@ -133,7 +110,7 @@ class MotionDenoise(MotionPrior):
         if getattr(bm, 'model_type', 'smplx') != 'smplx':
             raise NotImplementedError('MotionDenoise runs on the SMPL-X body model, as the reference does')
         b = self._buffers(dev)
-        lbs, pri = b['lbs'], b['prior']
+        lbs, pri, pin = b['lbs'], b['prior'], b['prior_input']
         rows, L_, J3 = self.batch_size, self.seq_len, b['full_pose'].shape[1]
         with torch.no_grad():
             smpl_gt = bm(betas=self.betas, pose_body=gt_poses) if gt_poses is not None else None
@@ -153,7 +130,7 @@ class MotionDenoise(MotionPrior):
         for it in range(iterations):
             for i in range(steps_per_iter):
                 step = it * steps_per_iter + i
-                qt = _quan_t(time_strategy, self.sde.N, total_steps, step, sample_trun, sample_time, 2)
+                qt = quan_t(time_strategy, self.sde.N, total_steps, step, sample_trun, sample_time, 2)
                 sched.append((it, float(timesteps[qt])))
         # the schedule's tables, the optimiser state and the captured step graphs live with the buffers: a further batch
         # of sequences with the same (deterministic) schedule replays the graphs of the first one
@@ -169,23 +146,18 @@ class MotionDenoise(MotionPrior):
 
         def one_step(k):
             it = sched[k][0]
-            if self.rot6d:
-                S.axis_to_rot6d_cols(b['full_pose'], 3, b['mean'], b['std'], b['x0'])
-            else:
-                S.affine_cols(b['full_pose'], 3, J3, b['mean'], b['std'], b['x0'])      # Posenormalizer (:238)
+            x0 = pin(b['full_pose'])                                                    # Posenormalizer (:238)
             z = None
             if z_list is not None:
                 b['z'].copy_(z_list[k].to(dev))
                 z = b['z']
-            g_prior = pri(b['x0'], k, False, float(self.batch_size_divisor), z=z, seed=seed, step=k)   # DPoser_loss (:251)
-            if self.rot6d:
-                S.axis_to_rot6d_cols_vjp(b['full_pose'], 3, b['std'], g_prior, b['g_axis'])
-                g_prior = b['g_axis']
+            g = pri(x0, k, False, float(self.batch_size_divisor), z=z, seed=seed, step=k)   # DPoser_loss (:251)
+            g_prior, col_scale = pin.adam_grad(b['full_pose'], g)
             lbs.forward(b['shape'], b['full_pose'], None)                               # body model (:255)
             S.motion_loss(lbs, b['target'], L_, 22, wd['temp'](1.0, it), wd['data'](1.0, it))   # :256-262
             lbs.backward(b['shape'], b['full_pose'], use_verts=True)
             opt.step(lbs.g_pose, 3, J3, 1.0, g2=g_prior, off2=0, ld2=63, s2=wd['dposer'](1.0, it),
-                     col_scale2=b['inv_std'])                                           # Adam (:266-268)
+                     col_scale2=col_scale)                                              # Adam (:266-268)
 
         for k in range(total_steps):
             sg.run(k, lambda k=k: one_step(k))
@@ -238,8 +210,8 @@ class SMPLify:
             pose_prior.batch_size = 1                       # reference runs B=1: prior = sum / 1 per image
 
     def sample_discrete_time(self, iteration):
-        return _quan_t(self.time_strategy, self.sde_N, self.stages * self.num_iters, iteration, self.sample_trun,
-                       self.sample_time, 5)
+        return quan_t(self.time_strategy, self.sde_N, self.stages * self.num_iters, iteration, self.sample_trun,
+                      self.sample_time, 5)
 
     def __call__(self, init_pose, init_betas, init_cam_t, camera_center, keypoints_2d, z_list=None, graphs=False):
         """run/smplify.py:168-281.  ``z_list`` (parity mode): the prior's Gaussian draw of every body step (+ the final
@@ -268,8 +240,7 @@ class SMPLify:
         jmap = smpl.joint_map.to(device=dev, dtype=torch.int32).contiguous()
         K = jmap.numel()
         j49, g49, loss_b = f(B, K, 3), f(B, K, 3), f(B)
-        pw = self.pose_prior.model.pose_width if self.pose_prior is not None else 63
-        g_cam, g_fit_pose, g_fit_betas, x0 = f(B, 3), f(B, J3), f(B, S_), f(B, pw)
+        g_cam, g_fit_pose, g_fit_betas = f(B, 3), f(B, J3), f(B, S_)
         conf = joints_conf.contiguous().float()
 
         def forward_joints(no_save=False):
@@ -304,15 +275,11 @@ class SMPLify:
             pri = S.PriorStep(pp.model, pp.sde, pp.continuous, B, dev)
             qts = [self.sample_discrete_time(k) for k in range(total)] + [self.sample_discrete_time(self.num_iters - 1)]
             pri.schedule([float(pp.timesteps[int(q)]) for q in qts])
-            mean, std = pp.Normalizer.column_affine() if self.rot6d else (pp.Normalizer.mean_poses,
-                                                                          pp.Normalizer.std_poses)
-            mean, std = mean.to(dev).float().contiguous(), std.to(dev).float().contiguous()
-            inv_std = None if self.rot6d else (1.0 / std).contiguous()
-            g_axis = f(B, 63) if self.rot6d else None   # the prior's gradient w.r.t. the axis-angle body pose
+            pin = S.PriorInput(pp.model, pp.Normalizer, B, dev)
+            zbuf = f(B, pp.model.pose_width)
         opt_b, opt_s = S.Adam(full_pose, 3, 63, self.step_size), S.Adam(shape, 0, 10, self.step_size)
         opt_g2 = S.Adam(full_pose, 0, 3, self.step_size)
         seed = mutils.host_seed() if z_list is None else 0
-        zbuf = f(B, pw)
         stage_weights = [dict(zip(self.loss_weights.keys(), vals)) for vals in zip(*self.loss_weights.values())]
 
         def body_step(k, w):
@@ -323,22 +290,17 @@ class SMPLify:
                                      float(w['angle_prior_weight']), float(w['shape_prior_weight']), L.ptr(loss_b), None,
                                      L.ptr(g49), L.ptr(g_fit_pose), L.ptr(g_fit_betas), B, st()))
             backward_joints(False)
-            g2 = None
+            g2, col_scale = None, None
             if pp is not None:
-                if self.rot6d:
-                    S.axis_to_rot6d_cols(full_pose, 3, mean, std, x0)         # offline_normalize(from_axis=True)
-                else:
-                    S.affine_cols(full_pose, 3, J3, mean, std, x0)
+                x0 = pin(full_pose)
                 z = None
                 if z_list is not None:
                     zbuf.copy_(z_list[k].to(dev))
                     z = zbuf
-                g2 = pri(x0, k, True, 1.0, z=z, seed=seed, step=k)          # DPoser.forward: weighted, sum / 1 per image
-                if self.rot6d:
-                    S.axis_to_rot6d_cols_vjp(full_pose, 3, std, g2, g_axis)
-                    g2 = g_axis
+                g = pri(x0, k, True, 1.0, z=z, seed=seed, step=k)           # DPoser.forward: weighted, sum / 1 per image
+                g2, col_scale = pin.adam_grad(full_pose, g)
             opt_b.step(lbs.g_pose, 3, J3, 1.0, g2=g2, off2=0, ld2=63, s2=float(w['pose_prior_weight']) ** 2,
-                       col_scale2=inv_std if pp is not None else None, g3=g_fit_pose, off3=0, ld3=J3, s3=1.0)
+                       col_scale2=col_scale, g3=g_fit_pose, off3=0, ld3=J3, s3=1.0)
             opt_s.step(lbs.g_shape, 0, S_, 1.0, g3=g_fit_betas, off3=0, ld3=S_, s3=1.0)
             opt_g2.step(lbs.g_pose, 0, J3)
 

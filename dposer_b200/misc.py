@@ -1,5 +1,6 @@
 """Small host-side helpers of the hot path (reference lib/utils/misc.py, lib/body_model/utils.py,
 lib/dataset/AMASS.py:187-259, lib/dataset/EvaSampler.py).  Pure tensor bookkeeping -- device agnostic."""
+import math
 import os
 
 import numpy as np
@@ -139,8 +140,19 @@ def shard_range(total, num_replicas, rank):
     return start, (base + 1 if rank < mod else base)
 
 
+def quan_t(strategy, N, total, step, trun, sample_time, offset):
+    """Discrete time index of step ``step`` of ``total`` under a task loop's time strategy (run/completion.py:183-191,
+    run/motion_denoising.py:240-247, run/smplify.py:153-166): '1' a uniform draw, '2' ``sample_time``, '3' the
+    truncated linear schedule."""
+    if strategy == '1':
+        return int(torch.randint(N, [1]))
+    if strategy == '2':
+        return int(sample_time)
+    if strategy == '3':
+        return N - math.floor(torch.tensor(total - step - 1) * (N / (trun * total))) - offset
+    raise NotImplementedError('unsupported time sampling strategy')
+
+
 def quan_t_schedule(N, total_steps, trun, offset):
-    """Time strategy '3' (run/completion.py:189-190, run/motion_denoising.py:245, run/smplify.py:153-166)."""
-    import math
-    return [N - math.floor(torch.tensor(total_steps - s - 1) * (N / (trun * total_steps))) - offset
-            for s in range(total_steps)]
+    """Every step's time index under strategy '3' (``quan_t``)."""
+    return [quan_t('3', N, total_steps, s, trun, None, offset) for s in range(total_steps)]

@@ -7,14 +7,12 @@ and its closed-form gradient (x0_hat is detached in the reference, so no backwar
 the network exists).  The returned loss is an autograd scalar whose backward scales the
 kernel-produced gradient.
 """
-import math
-
 import torch
 import torch.nn as nn
 
 from . import _lib as L
 from . import utils as mutils
-from .misc import linear_interpolation
+from .misc import linear_interpolation, quan_t
 
 N_POSES = 21
 
@@ -177,17 +175,8 @@ class DPoserComp(_PriorBase):
         sched = []
         for it in range(iterations):
             for i in range(steps_per_iter):
-                step = it * steps_per_iter + i
-                if time_strategy == '1':
-                    quan_t = int(torch.randint(self.sde.N, [1]))
-                elif time_strategy == '2':
-                    quan_t = int(sample_time)
-                elif time_strategy == '3':
-                    quan_t = self.sde.N - math.floor(
-                        torch.tensor(total_steps - step - 1) * (self.sde.N / (sample_trun * total_steps))) - 2
-                else:
-                    raise NotImplementedError('unsupported time sampling strategy')
-                sched.append((it, quan_t, float(timesteps[quan_t])))
+                qt = quan_t(time_strategy, self.sde.N, total_steps, it * steps_per_iter + i, sample_trun, sample_time, 2)
+                sched.append((it, qt, float(timesteps[qt])))
         pri = S.PriorStep(self.model, self.sde, self.continuous, rows, dev)
         pri.schedule([t for _, _, t in sched])
         g_data = torch.empty_like(x)

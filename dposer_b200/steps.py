@@ -71,6 +71,38 @@ class PriorStep:
         return self.grad
 
 
+class PriorInput:
+    """How the fitting chains feed the prior from the axis-angle body pose, fixed by the score network's width:
+
+    * 63-D (axis-angle): x0 = (pose - mean_poses) / std_poses, and Adam scales the prior's gradient by 1 / std.
+    * 126-D (rot6d): x0 = normalize(axis_angle_to_rot6d(pose)) under ``Posenormalizer.column_affine()``, and the prior's
+      gradient returns to the axis-angle pose through the VJP of that map."""
+
+    def __init__(self, model, normalizer, rows, device):
+        self.rot6d = model.pose_width == L.POSE_DIM_ROT6D
+        mean, std = normalizer.column_affine() if self.rot6d else (normalizer.mean_poses, normalizer.std_poses)
+        self.mean, self.std = mean.to(device).float().contiguous(), std.to(device).float().contiguous()
+        self.inv_std = None if self.rot6d else (1.0 / self.std).contiguous()
+        # the prior's gradient w.r.t. the axis-angle body pose
+        self.g_axis = torch.zeros(rows, 63, dtype=torch.float32, device=device) if self.rot6d else None
+        self.x0 = torch.zeros(rows, model.pose_width, dtype=torch.float32, device=device)
+
+    def __call__(self, full_pose):
+        """The prior's input from the body pose full_pose[:, 3:66], in ``self.x0``."""
+        if self.rot6d:
+            axis_to_rot6d_cols(full_pose, 3, self.mean, self.std, self.x0)       # offline_normalize(from_axis=True)
+        else:
+            affine_cols(full_pose, 3, full_pose.shape[1], self.mean, self.std, self.x0)
+        return self.x0
+
+    def adam_grad(self, full_pose, g):
+        """``(g2, col_scale2)`` of ``Adam.step`` on the body pose from g, the prior's gradient w.r.t. x0."""
+        if not self.rot6d:
+            return g, self.inv_std
+        axis_to_rot6d_cols_vjp(full_pose, 3, self.std, g, self.g_axis)
+        return self.g_axis, None
+
+
 class LbsStep:
     """LBS forward + backward on preallocated buffers (the autograd-free twin of body_model._LbsFn)."""
 

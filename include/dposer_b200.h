@@ -39,8 +39,8 @@ extern "C" {
 #define DPB_ENOMEM (-3)       /* workspace too small or allocation failure */
 #define DPB_EUNSUPPORTED (-4) /* feature not available (maps to NotImplementedError) */
 
-/* network geometry (configs/subvp/amass_scorefc_continuous.py:36-45 + defaults).  DPB_POSE_DIM is the axis-angle
- * width; a score handle may instead be created for the rot6d width DPB_POSE_DIM_ROT6D (dpb_score_create_dim). */
+/* network geometry (configs/subvp/amass_scorefc_continuous.py:36-45 + defaults).  A score handle is created for the
+ * axis-angle width DPB_POSE_DIM or the rot6d width DPB_POSE_DIM_ROT6D (dpb_score_create_dim). */
 #define DPB_POSE_DIM 63
 #define DPB_POSE_DIM_ROT6D 126
 #define DPB_HIDDEN 1024
@@ -87,10 +87,9 @@ typedef struct {
   const float* emb_freqs;    /* [256] exp(-k ln(1e4)/255) evaluated by the host in fp32 (model.py:41-43) */
 } dpb_score_weights;
 
-/* a 63-D (axis-angle, ScoreModelFC(config, 21, 3)) network */
-int dpb_score_create(dpb_score_t** h, const dpb_score_weights* w, int device);
-/* pose_dim = 63 (axis-angle) or 126 (rot6d, ScoreModelFC(config, 21, 6)); any other value: DPB_EUNSUPPORTED.
- * Every entry point that takes the handle reads D = pose_dim from it; "[B,D]" below means that width. */
+/* pose_dim = 63 (axis-angle, ScoreModelFC(config, 21, 3)) or 126 (rot6d, ScoreModelFC(config, 21, 6)); any other
+ * value: DPB_EUNSUPPORTED.  Every entry point that takes the handle reads D = pose_dim from it; "[B,D]" below means
+ * that width. */
 int dpb_score_create_dim(dpb_score_t** h, const dpb_score_weights* w, int pose_dim, int device);
 /* D of the handle (63 or 126), or DPB_EINVAL for a null handle */
 int dpb_score_pose_dim(dpb_score_t* h);
@@ -154,14 +153,11 @@ int dpb_sampler_run(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, con
                     float* traj, float* x_mean, int64_t B, int flags, void* ws, size_t ws_bytes,
                     void* stream);
 
-/* Langevin corrector pieces (sampling.py:282-302): batch sums of row norms, then the update.
+/* Langevin corrector pieces (sampling.py:282-302) on rows of pose_dim (63 or 126) columns: batch sums of row norms,
+ * then the update.
  * sums DEVICE fp32[2] must be zeroed by the caller; norms: sums[0]+=sum_b||grad_b||, sums[1]+=sum_b||noise_b||.
  * update: step = (snr*(sums[1]/Bglobal)/(sums[0]/Bglobal))^2 * 2*alpha ; x_mean = x + step*grad ;
  *         x = x_mean + sqrt(2 step)*noise. */
-int dpb_langevin_norms(const float* grad, const float* noise, float* sums, int64_t B, void* stream);
-int dpb_langevin_update(float* x_io, float* x_mean, const float* grad, const float* noise,
-                        const float* sums, float snr, float alpha, int64_t B, void* stream);
-/* the same on rows of pose_dim (63 or 126) columns; the two above mean pose_dim = 63 */
 int dpb_langevin_norms_dim(const float* grad, const float* noise, float* sums, int64_t B, int pose_dim, void* stream);
 int dpb_langevin_update_dim(float* x_io, float* x_mean, const float* grad, const float* noise, const float* sums,
                             float snr, float alpha, int64_t B, int pose_dim, void* stream);
@@ -180,9 +176,7 @@ int dpb_sampler_run_pc(dpb_score_t* h, float* x_io, const dpb_step_tables* tbl, 
 /* fills out [B, pose_dim] with N(0,1) draws of the library's Philox stream.  Draw (row, column c) of (step, slot) is
  * Box-Muller output c % 4 of the Philox4x32-10 block with key = seed and counter = (row lo, row hi, step,
  * slot * DP/4 + c/4), DP = 64 for pose_dim 63 and 128 for 126: every (slot, column) of a row has its own counter.
- * Slots: 0 imputation before the score, 1 predictor, 2 imputation after the predictor, 3 prior-loss z, 4 Langevin.
- * dpb_normal_fill means pose_dim = 63. */
-int dpb_normal_fill(float* out, int64_t B, uint64_t seed, uint64_t step, int slot, void* stream);
+ * Slots: 0 imputation before the score, 1 predictor, 2 imputation after the predictor, 3 prior-loss z, 4 Langevin. */
 int dpb_normal_fill_dim(float* out, int64_t B, uint64_t seed, uint64_t step, int slot, int pose_dim, void* stream);
 
 /* ------------------------------------------------------------------------------------------
@@ -375,9 +369,6 @@ int dpb_rk45_error(const double* y, const double* y_new, const float* k, int64_t
  * [B,D] with D = pose_dim (63 or 126; any other value: DPB_EUNSUPPORTED, checked before the arguments) */
 int dpb_pf_ode_rhs_dim(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2,
                        float* k_out, int64_t B, int pose_dim, void* stream);
-/* the pose_dim = 63 case of dpb_pf_ode_rhs_dim */
-int dpb_pf_ode_rhs(const float* x, const float* score, const float* jv, const float* eps, float fx, float g2, float* k_out,
-                   int64_t B, void* stream);
 
 /* ------------------------------------------------------------------------------------------
  * Training step of the score network (replaces loss_fn + loss.backward() + optimize_fn + ema.update of
@@ -393,8 +384,6 @@ typedef dpb_score_weights dpb_train_tensors;
  * pose_dim = 63 (axis-angle) or 126 (rot6d); any other value: DPB_EUNSUPPORTED, before any device is touched.  "[B,D]"
  * below means that width. */
 int dpb_train_create_dim(dpb_train_t** h, int64_t batch, int pose_dim, int device);
-/* the pose_dim = 63 case of dpb_train_create_dim */
-int dpb_train_create(dpb_train_t** h, int64_t batch, int device);
 int dpb_train_destroy(dpb_train_t* h);
 /* loss = mean_b row_w[b] sum_k (res_c[b] res[b,k] + z_c[b] z[b,k])^2 on perturbed = mean_c x + std_c z, where res is the
  * network's post_dense output at the per-row label (losses.py:108-131; the sigma / std divisions and the reduce_mean /

@@ -219,7 +219,8 @@ def test_philox_126_columns_are_independent_normals():
     # the documented counter word slot * DP/4 + column/4: slot 1 of the 63-D layout (words 16..31) is slot 0, columns
     # 64.., of the 126-D layout -- the 63-D stream keeps its addressing (columns 0..61 of it; the 126-D row ends at 125)
     z63 = torch.empty(B, 63, device='cuda')
-    L.check(L.load().dpb_normal_fill(L.ptr(z63), B, C.c_uint64(123), C.c_uint64(7), 1, L.current_stream(z63.device)))
+    L.check(L.load().dpb_normal_fill_dim(L.ptr(z63), B, C.c_uint64(123), C.c_uint64(7), 1, 63,
+                                         L.current_stream(z63.device)))
     assert torch.equal(z63[:, :62], zs[0, :, 64:126])
 
 

@@ -77,11 +77,13 @@ def test_inkernel_philox_noise_is_standard_normal_and_engine_independent(gpu_mod
     import ctypes as C
     B = 4096
     z = torch.empty(B, 63, device='cuda')
-    L.check(L.load().dpb_normal_fill(L.ptr(z), B, C.c_uint64(123), C.c_uint64(7), 1, L.current_stream(z.device)))
+    L.check(L.load().dpb_normal_fill_dim(L.ptr(z), B, C.c_uint64(123), C.c_uint64(7), 1, 63,
+                                         L.current_stream(z.device)))
     assert abs(float(z.mean())) < 0.01 and abs(float(z.std()) - 1) < 0.01
     assert abs(float((z ** 4).mean()) - 3.0) < 0.1                      # kurtosis of N(0,1)
     z2 = torch.empty_like(z)
-    L.check(L.load().dpb_normal_fill(L.ptr(z2), B, C.c_uint64(123), C.c_uint64(8), 1, L.current_stream(z.device)))
+    L.check(L.load().dpb_normal_fill_dim(L.ptr(z2), B, C.c_uint64(123), C.c_uint64(8), 1, 63,
+                                         L.current_stream(z.device)))
     assert abs(float((z * z2).mean())) < 0.01                           # steps are independent
     # same seed -> same samples on both engines (they share the Philox addressing)
     cfg = synthetic.default_config()
